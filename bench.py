@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (hand-written sm_100a CUDA)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: oracle port on the host cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
 
 Workload at every N: BASELINE.json configs[1] per GPU -- MinAtar Space-Invaders shaped transitions
 (10x10x6), DQN + double-Q + PER, 1M-capacity shard, batch 256, 3-step returns.  One "step" is one
@@ -210,6 +211,36 @@ def build_ours(rank, world, device, capacity, fill, seed):
     buf.buffer._sampler.update_priority(torch.arange(fill, device=device), prio, sorted=True)
     torch.cuda.synchronize()
     return cfg, agent, buf, trace, ingest_s
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def step_outputs(step, prefix=""):
+    """What the last LearnerStep iteration computed, on the host: its loss and TD errors, the batch it sampled and
+    gathered, the parameters after its optimizer step and every priority leaf after its write-back.  Integer and fp64
+    arrays come back as float64, the rest as float32."""
+    import torch
+    torch.cuda.synchronize()
+    b = step.batch
+    out = {"loss": step.agent._static_total_loss, "td": step.td, "index": step.idx[:step.B_pad],
+           "weight": step.weight[:step.B_pad], "observation": b["observation"],
+           "next_observation": b["next"]["observation"], "reward": b["next"]["reward"], "gamma": b["gamma"],
+           "nonterminal": b["nonterminal"], "action": b["action"], "params": step.agent.optimizer.arena,
+           "priorities": step.tree.leaves()}
+    wide = (torch.int64, torch.int32, torch.float64)
+    return {prefix + k: v.detach().cpu().numpy().astype(np.float64 if v.dtype in wide else np.float32)
+            for k, v in out.items()}
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy for every array (--dump-outputs)."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("outputs to dump take %d bytes, more than %d" % (total, DUMP_MAX_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def time_kernel(fn, reps, torch):
@@ -849,7 +880,7 @@ def cpu_baseline(steps, fill, budget_s=25.0, batch=BATCH, warmup=3):
         one()
     t0 = time.perf_counter()
     n = 0
-    while n < steps and time.perf_counter() - t0 < budget_s:
+    while n < steps and (budget_s is None or time.perf_counter() - t0 < budget_s):
         one()
         n += 1
     dt = time.perf_counter() - t0
@@ -950,6 +981,8 @@ def run_ours(args):
     gpu_launches = (lp * args.steps) if lp is not None else (_lib.launch_count() - launches0)
     value = BATCH * world * args.steps / sec
     del pool
+    dump = args.dump_outputs is not None and rank == 0
+    outputs = step_outputs(step) if dump else None
 
     # ---------------- end-to-end through the public API with host buffers ----------------------
     # synthetic host inputs are generated BEFORE the timed region; the timed loop copies them through pinned
@@ -996,6 +1029,9 @@ def run_ours(args):
     e2e = {"value": BATCH * world * e2e_steps / e2e_sec, "unit": "transitions/s", "h2d_bytes_per_step": int(h2d),
            "d2h_bytes_per_step": 4, "updates_per_s": e2e_steps / e2e_sec,
            "host_wall_s": round(wall, 4), "loss": float(loss_host)}
+    if dump:
+        outputs.update(step_outputs(step, prefix="e2e_"))
+        dump_outputs(args.dump_outputs, outputs)
 
     sharded = cfg4 = None
     if world > 1 and not args.quick:
@@ -1085,15 +1121,15 @@ def run_reference(args):
     if rank != 0:
         return
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
-    # like for like with our arm at N GPUs: the global batch (256 per GPU) on the host, a 1M-filled buffer, and at
-    # least 200 timed iterations after 20 warm-ups (20 cold iterations overstated the ratio in round 1)
-    steps = max(args.steps, 200)
+    # like for like with our arm at N GPUs: the global batch (256 per GPU) on the host and a 1M-filled buffer.  Exactly
+    # --steps timed iterations; short cold runs overstate the GPU/CPU ratio, so compare at a few hundred steps
+    steps, warmup = args.steps, max(3, args.warmup)
     fill = int(os.environ.get("PB_REF_FILL", CAPACITY))      # tests shrink the fill; the driver's run uses the full 1M
-    cpu = cpu_baseline(steps=steps, fill=fill, budget_s=150.0, batch=BATCH * world, warmup=max(20, args.warmup))
+    cpu = cpu_baseline(steps=steps, fill=fill, budget_s=None, batch=BATCH * world, warmup=warmup)
     line = {
         "impl": "reference",
         "metric": METRIC,
-        "value": cpu["value"], "unit": "transitions/s", "n_gpus": args.gpus, "steps": steps, "warmup": max(20, args.warmup),
+        "value": cpu["value"], "unit": "transitions/s", "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
         "steps_requested": args.steps, "warmup_requested": args.warmup,
         "ms_per_step": cpu["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic", "learner_updates_per_s": cpu["updates_per_s"],
@@ -1118,7 +1154,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="skip extras and the CPU baseline (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, TD errors, batch, parameters, priorities; "
+                         "e2e_* for the end-to-end leg) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU arm's step; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -19,6 +19,7 @@ What is frozen:
   per_tree.npz       ORACLE-generated (parity unpinned: torchrl is absent) -- freezes the restated
                      tree/sampler arithmetic so the C oracle and the CUDA path cannot drift apart
 """
+import io
 import os
 import sys
 import types
@@ -29,6 +30,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 GOLD = os.path.join(ROOT, "tests", "golden")
+MAX_FILE_BYTES = 1 << 20          # no file in the repository is larger: bigger fixtures are stored in parts
 REF = "/root/reference"
 
 
@@ -99,6 +101,18 @@ def make_batch(rng, B, obs_shape, n_actions, binary_obs):
         "gamma": np.where(rng.random((B, 1)) < 0.7, 0.99 ** 3, 0.99 ** 2).astype(np.float32),
         "action": rng.integers(0, n_actions, (B, 1)).astype(np.int64),
     }
+
+
+def save_parts(name, out, groups):
+    """GOLD/<name>.npz; when that would exceed MAX_FILE_BYTES, the keys "<group>.*" of each group go to
+    GOLD/<name>.<group>.npz instead (tests/helpers.py load_golden merges the parts back)."""
+    whole = io.BytesIO()
+    np.savez_compressed(whole, **out)
+    if whole.tell() > MAX_FILE_BYTES:
+        for g in groups:
+            part = {k: out.pop(k) for k in list(out) if k.startswith(g + ".")}
+            np.savez_compressed(os.path.join(GOLD, "%s.%s.npz" % (name, g)), **part)
+    np.savez_compressed(os.path.join(GOLD, name + ".npz"), **out)
 
 
 def to_torch_batch(b):
@@ -185,7 +199,7 @@ def gen_agent_case(name, overrides, obs_shape, n_actions, B):
         if q is not None:
             out["act.q"] = q.numpy()
         out["act.action"] = act.numpy()
-    np.savez_compressed(os.path.join(GOLD, name + ".npz"), **out)
+    save_parts(name, out, ("grad_clipped", "param_after"))
     print("wrote", name, "params", sum(v.size for k, v in out.items() if k.startswith("param.")))
 
 

@@ -1,5 +1,6 @@
 """Shared test plumbing: golden fixtures, config reconstruction, script replay."""
 import ast
+import glob
 import os
 
 import numpy as np
@@ -9,7 +10,11 @@ GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    return dict(np.load(os.path.join(GOLD, name + ".npz"), allow_pickle=False))
+    """golden/<name>.npz merged with its parts golden/<name>.<group>.npz (a fixture over 1 MB is stored split)."""
+    out = {}
+    for path in [os.path.join(GOLD, name + ".npz")] + sorted(glob.glob(os.path.join(GOLD, name + ".*.npz"))):
+        out.update(np.load(path, allow_pickle=False))
+    return out
 
 
 def cfg_from_fixture(fx, device):
