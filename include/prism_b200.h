@@ -519,9 +519,6 @@ int pb_peer_adam(const pb_peer_group *g, long long n, float *param, float *exp_a
  * the channel-1 epoch (the parity of the double-buffered gradient arena); reduced[rank] receives the summed gradient.
  * partial_scratch: 4096 floats, the last 4 zero between calls. */
 long long pb_peer_allreduce_adam_max_n(void);
-/* HOST: number of ranks from which pb_peer_allreduce_adam runs two-phase (0 = never, the default; PB_PEER_TWO_PHASE in
- * the environment); set >= 0 changes it, returns the value in force. */
-int pb_peer_two_phase_min(int set);
 int pb_peer_allreduce_adam(const pb_peer_group *g, long long n, float *param, float *exp_avg, float *exp_avg_sq,
                            long long *step_count, float lr, float beta1, float beta2, float adam_eps, float max_grad_norm,
                            float *partial_scratch, float *norm_out, void *stream);

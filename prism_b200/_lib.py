@@ -136,7 +136,6 @@ SIGNATURES = {
     "pb_peer_pull_sum": [_PEER, _LL, _P, _P, C.POINTER(C.c_int), _P],
     "pb_peer_adam": [_PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
     "pb_peer_allreduce_adam_max_n": [],
-    "pb_peer_two_phase_min": [_I],
     "pb_peer_allreduce_adam": [_PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
     "pb_peer_state_put": [_PEER, _P, _P],
     "pb_peer_trace": [_I, _P, _I],

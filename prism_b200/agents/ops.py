@@ -192,7 +192,6 @@ def loss_combine(dist_loss, q_loss, per_weights):
     return _LossCombine.apply(dist_loss, q_loss, per_weights)
 
 
-PARALLEL_BACKWARD = __import__('os').environ.get('PB_PARALLEL_BACKWARD', '1') != '0'
 # LearnerStep.enable_trace() points this at its timeline-mark function (measurement runs only); None otherwise
 TRACE_MARK = None
 
@@ -203,22 +202,13 @@ def trace_mark(name):
 _SIDE_STREAMS = {}
 
 
-SERIAL_GRAPH = __import__('os').environ.get('PB_SERIAL_GRAPH', '0') == '1'   # tuning switch: no parallel branches at all
-
-
 def fork_stream(device, key="bwd"):
-    """A cached side stream (a parallel branch under CUDA-graph capture); the current stream when PB_SERIAL_GRAPH=1."""
+    """A cached side stream (a parallel branch under CUDA-graph capture)."""
     device = torch.device(device)
-    if SERIAL_GRAPH:
-        return torch.cuda.current_stream(device)
     s = _SIDE_STREAMS.get((device, key))
     if s is None:
         s = _SIDE_STREAMS[(device, key)] = torch.cuda.Stream(device=device)
     return s
-
-
-def _side_stream(device):
-    return fork_stream(device, "bwd")
 
 
 # Weight-gradient branches and their joins.  A layer's dW (and db) feed nothing but the optimizer, so inside the captured
@@ -291,7 +281,7 @@ class _Linear(torch.autograd.Function):
             db = torch.empty(K, N, dtype=torch.float32, device=dy.device) if ctx.has_bias else None
         # the two gradient GEMMs are independent and each is too small to fill the chip: the weight gradient goes to a
         # second stream (a parallel branch under CUDA-graph capture) and is joined before the function returns
-        side = _side_stream(dy.device) if (want_dx and want_dw and PARALLEL_BACKWARD) else None
+        side = fork_stream(dy.device) if (want_dx and want_dw) else None
         if want_dw:
             if side is not None:
                 cur = torch.cuda.current_stream(dy.device)
@@ -441,12 +431,12 @@ class _NarrowLinear(torch.autograd.Function):
         if want_dw or want_db:
             partials = torch.empty(K * lib.pb_narrow_linear_bwd_blocks(M) * (N * J + N), dtype=torch.float32, device=dy.device)
         # inside the learner step graph the dW / db reduction goes to the weight-gradient branch (see _JOINS)
-        split = partials is not None and want_dx and _JOINS["mode"] and PARALLEL_BACKWARD and not SERIAL_GRAPH
+        split = partials is not None and want_dx and _JOINS["mode"]
         _lib.check(lib.pb_narrow_linear_bwd(K, M, N, J, xc.data_ptr(), 0 if ctx.shared else M * J, wc.data_ptr(), dy.data_ptr(),
                                             _lib.ptr(dx), None if split else _lib.ptr(dw), None if split else _lib.ptr(db),
                                             _lib.ptr(partials), _stream(dy)), "pb_narrow_linear_bwd")
         if split:
-            side = _side_stream(dy.device)
+            side = fork_stream(dy.device)
             side.wait_stream(torch.cuda.current_stream(dy.device))
             with torch.cuda.stream(side):
                 _lib.check(lib.pb_narrow_linear_bwd_reduce(K, M, N, J, partials.data_ptr(), _lib.ptr(dw), _lib.ptr(db),
@@ -467,13 +457,12 @@ def _narrow_eligible(x, weight):
             and _lib.load().pb_narrow_linear_supported(x.shape[-2], N, J) == 1)
 
 
-TENSOR_CORE_LINEAR = True      # module switch for A/B timing
 TC_MIN_ROWS = 256              # an M = 128 tile needs rows to fill it
-TC_MIN_FLOPS = float(__import__('os').environ.get('PB_TC_MIN_FLOPS', 2.0e8))           # below this a layer is launch-bound and stays on the fused SIMT kernel / library
+TC_MIN_FLOPS = 2.0e8           # below this a layer is launch-bound and stays on the fused SIMT kernel / library
 
 
 def _tc_eligible(x, M, Kh, N, J):
-    return (TENSOR_CORE_LINEAR and x.is_cuda and (J % 4) == 0 and (N % 4) == 0 and M >= TC_MIN_ROWS
+    return (x.is_cuda and (J % 4) == 0 and (N % 4) == 0 and M >= TC_MIN_ROWS
             and 2.0 * M * Kh * N * J >= TC_MIN_FLOPS)
 
 

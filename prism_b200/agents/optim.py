@@ -82,8 +82,6 @@ class FlatAdam(object):
         self.grad_scale = 1.0           # 1/world_size under data parallelism
         self.allreduce = None           # callable(flat_grad) inserted between gather and Adam (library collective)
         self.peer = None                # PeerGroup: gradient exchange fused with clip + Adam over peer memory
-        self.peer_state = None          # 64-byte shard state block that rides on the exchange's handshake (LearnerStep)
-        self.peer_after_exchange = None  # callable run right after the handshake (LearnerStep: prefetch of the next batch)
 
     def _fused_max_n(self):
         m = getattr(self, "_fused_max", None)
@@ -138,7 +136,7 @@ class FlatAdam(object):
                                                       self.peer.grad_stride, None, None, None, stream),
                        "pb_pack_grads_parity")
             mark("opt:packed")
-            self.peer.allreduce_adam(self, state=self.peer_state, mark=mark, after_exchange=self.peer_after_exchange)
+            self.peer.allreduce_adam(self, mark=mark)
             return
         if self.allreduce is None and FUSED_STEP and len(self.params) <= 64 and self.numel <= self._fused_max_n():
             # small arena: gather + norm + clip + Adam in ONE launch (the gradient stays in registers)

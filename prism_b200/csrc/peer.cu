@@ -16,7 +16,6 @@
 //     published partial sums in rank order (bit-identical on every rank) and updates the local parameter replica.
 // pb_peer_barrier is a 1-block epoch barrier (flags in peer memory, monotonically increasing: graph-replay safe).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -258,6 +257,7 @@ __global__ void __launch_bounds__(256) peer_adam_kernel(pb_peer_group g, long lo
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int FA_THREADS = 256;
 constexpr int FA_U = 8;                                               // 128-bit elements per thread held in registers
+constexpr int FA_MAX_PEERS = PB_PEER_MAX - 1;                         // other ranks a thread pulls from
 
 __device__ __forceinline__ unsigned ld_acquire_gpu_u32(const unsigned *p)
 {
@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
                                                                          float beta1, float beta2, float adam_eps,
                                                                          float max_grad_norm, float *__restrict__ partials,
                                                                          unsigned int *__restrict__ counters,
-                                                                         float *__restrict__ norm_out, int two_phase)
+                                                                         float *__restrict__ norm_out)
 {
     __shared__ double red[FA_THREADS / 32];
     __shared__ float s_coef;
@@ -313,8 +313,7 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
     if (threadIdx.x == 0) ptrace(tr, 1);                              // handshake done
     const long long po = (long long)((e - 1) & 1ull) * g.grad_stride;  // the half packed for this exchange
     float4 sum[FA_U];
-    if (!two_phase) {
-    // ---- ONE-SHOT: pull + sum every rank's whole arena in rank order, kept in registers
+    // ---- pull + sum every rank's whole arena in rank order, kept in registers
     double acc = 0.0;
 #pragma unroll
     for (int k = 0; k < FA_U; ++k) {
@@ -322,6 +321,8 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
         sum[k] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (i < n4) {
             float4 s4 = ld_peer_f4(g.grad[0] + po + (i << 2));
+            // fully unrolled, the kernel fits 80 registers: 3 resident CTAs per SM, which sizes the grid (fa_max_blocks)
+#pragma unroll FA_MAX_PEERS
             for (int p = 1; p < g.world; ++p) {
                 const float4 v = ld_peer_f4(g.grad[p] + po + (i << 2));
                 s4.x += v.x; s4.y += v.y; s4.z += v.z; s4.w += v.w;
@@ -363,72 +364,6 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
         if (blockIdx.x == 0 && norm_out) { norm_out[0] = total_norm; norm_out[1] = coef; }
     }
     __syncthreads();
-    } else {
-    // ---- TWO-PHASE (8 ranks: pulling 7 whole arenas costs more than a second flag round).  Phase 1: this rank sums
-    // ITS slice of every rank's arena (rank order) and PUSHES the result into every rank's reduced buffer; its
-    // sum of squares goes to every rank's norm slots; then this rank's channel-3 flag is raised everywhere.
-    const long long S4 = (n4 + g.world - 1) / g.world;
-    const long long lo4 = (long long)g.rank * S4, hi4 = lo4 + S4 < n4 ? lo4 + S4 : n4;
-    double acc = 0.0;
-    for (long long j = lo4 + i0; j < hi4; j += stride) {
-        float4 s4 = ld_peer_f4(g.grad[0] + po + (j << 2));
-        for (int p = 1; p < g.world; ++p) {
-            const float4 v = ld_peer_f4(g.grad[p] + po + (j << 2));
-            s4.x += v.x; s4.y += v.y; s4.z += v.z; s4.w += v.w;
-        }
-        for (int p = 0; p < g.world; ++p) *reinterpret_cast<float4 *>(g.reduced[p] + (j << 2)) = s4;
-        acc += (double)(s4.x * s4.x + s4.y * s4.y) + (double)(s4.z * s4.z + s4.w * s4.w);
-    }
-    acc = warp_sum(acc);
-    if (lane == 0) red[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        ptrace(tr, 2);                                                // slice reduced + pushed
-        double t = 0.0;
-        for (int k = 0; k < FA_THREADS / 32; ++k) t += red[k];
-        partials[blockIdx.x] = (float)t;
-        // ONE system-scope fence per CTA: the barrier above ordered every thread's pushes before it (cumulativity);
-        // a fence per thread measured +12 us
-        __threadfence_system();
-        atomicAdd(&counters[0], 1u);
-    }
-    if (blockIdx.x == 0 && threadIdx.x < 32) {
-        // CTA 0 publishes the slice once every CTA of this grid has pushed its part
-        if (lane == 0) while (ld_acquire_gpu_u32(&counters[0]) < gridDim.x) { }
-        __syncwarp();
-        double a2 = 0.0;
-        for (int k = lane; k < (int)gridDim.x; k += 32) a2 += (double)__ldcg(partials + k);
-        a2 = warp_sum(a2);
-        if (lane < g.world) g.norm_parts[lane][g.rank] = a2;
-        __threadfence_system();
-        __syncwarp();
-        if (lane < g.world) st_release_sys(g.flags[lane] + 3 * PB_PEER_MAX + g.rank, e);
-    }
-    // ---- phase 2: every rank's slice has landed in the local reduced buffer
-    if (threadIdx.x < 32 && lane < g.world) {
-        const unsigned long long *mine = g.flags[g.rank] + 3 * PB_PEER_MAX + lane;
-        if (!wait_flag_sys(mine, e, g.timeout_ns) && g.status) atomicOr(g.status, 1u << 3);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        ptrace(tr, 3);                                                // all slices here
-        double sq = 0.0;
-        for (int r = 0; r < g.world; ++r) sq += ld_peer_f64(g.norm_parts[g.rank] + r);      // rank order: identical everywhere
-        const float total_norm = (float)sqrt(sq);
-        float coef = max_grad_norm / (total_norm + 1e-6f);            // clip_grad_norm_
-        coef = coef > 1.0f ? 1.0f : coef;
-        if (!(max_grad_norm > 0.0f)) coef = 1.0f;
-        s_coef = coef;
-        if (blockIdx.x == 0 && norm_out) { norm_out[0] = total_norm; norm_out[1] = coef; }
-    }
-#pragma unroll
-    for (int k = 0; k < FA_U; ++k) {
-        const long long i = i0 + k * stride;
-        sum[k] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (i < n4) sum[k] = ld_peer_f4(g.reduced[g.rank] + (i << 2));
-    }
-    __syncthreads();
-    }
     const float coef = s_coef;
     auto upd = [&](float &p, float gg, float &m, float &v) {          // same arithmetic as adam_clip_kernel
         gg *= coef;
@@ -446,7 +381,7 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
             const float4 gr = sum[k];
             upd(p.x, gr.x, m.x, v.x); upd(p.y, gr.y, m.y, v.y); upd(p.z, gr.z, m.z, v.z); upd(p.w, gr.w, m.w, v.w);
             p4[i] = p; m4[i] = m; v4[i] = v;
-            if (!two_phase) r4[i] = gr;                               // the summed gradient (diagnostics, tests)
+            r4[i] = gr;                                               // the summed gradient (diagnostics, tests)
         }
     }
     // ---- the last CTA out closes the exchange: counters back to zero, epoch and step count advanced
@@ -621,19 +556,6 @@ static int fa_max_blocks()
     return c;
 }
 
-int pb_peer_two_phase_min(int set)
-{
-    static std::atomic<int> two_min{-1};
-    if (set >= 0) two_min.store(set);
-    int v = two_min.load();
-    if (v < 0) {
-        const char *e = getenv("PB_PEER_TWO_PHASE");
-        v = e ? atoi(e) : 0;
-        two_min.store(v);
-    }
-    return v;
-}
-
 long long pb_peer_allreduce_adam_max_n(void) { return (long long)fa_max_blocks() * FA_THREADS * FA_U * 4; }
 
 int pb_peer_allreduce_adam(const pb_peer_group *g, long long n, float *param, float *exp_avg, float *exp_avg_sq,
@@ -654,17 +576,8 @@ int pb_peer_allreduce_adam(const pb_peer_group *g, long long n, float *param, fl
     if (nb > cap) nb = cap;
     if (nb < 1) nb = 1;
     unsigned int *counters = reinterpret_cast<unsigned int *>(partial_scratch + 4092);    // zero between calls
-    // two-phase (reduce-scatter by pull, all-gather by push) from pb_peer_two_phase_min() ranks on.  OFF by default:
-    // measured at 8 GPUs it equals the one-shot schedule (129.8 vs 128.7 us per step: what the step pays from 4 to 8
-    // ranks is waiting for the slowest of 8, not NVLink volume) and at 2 GPUs it costs a second flag round (+12 us).
-    const int two_min = pb_peer_two_phase_min(-1);
-    int two_phase = (two_min > 0 && g->world >= two_min) ? 1 : 0;
-    if (two_phase) {
-        for (int p = 0; p < g->world; ++p)
-            if (!g->reduced[p] || !g->norm_parts[p]) two_phase = 0;
-    }
     PB_LAUNCH_PDL(peer_allreduce_adam_kernel, (unsigned)nb, FA_THREADS, 0, stream, *g, n, param, exp_avg, exp_avg_sq, step_count,
-              lr, beta1, beta2, adam_eps, max_grad_norm, partial_scratch, counters, norm_out, two_phase);
+              lr, beta1, beta2, adam_eps, max_grad_norm, partial_scratch, counters, norm_out);
     return PB_OK;
 }
 

@@ -10,10 +10,12 @@ n-step/gather into the agent's static batch), update (fused loss heads, clip+Ada
 priority write-back are captured into a single graph, replayed once per iteration.
 
 Data parallel (SURVEY 8e): every rank owns a shard (ring + trees) fed by its own collectors.
-Per iteration: one all-gather of the 64-byte shard state blocks, global stratified sampling with
-owner-computes placement (no transition crosses NVLink), one all-reduce of the flat gradient arena
-fused with clip + Adam.  Both exchanges run as our own kernels over NVLink peer memory
-(csrc/peer.cu); PB_DP_EXCHANGE=nccl (or ranks that cannot map each other) falls back to NCCL.
+Per iteration: every rank puts its 64-byte shard state block into every rank's slot after its
+priority write-back, the next batch's global stratified sampling waits for those puts itself and
+places each stratum on its owner (no transition crosses NVLink), and one all-reduce of the flat
+gradient arena is fused with clip + Adam.  Both exchanges run as our own kernels over NVLink peer
+memory (csrc/peer.cu); PB_DP_EXCHANGE=nccl (or ranks that cannot map each other) falls back to
+NCCL, which all-gathers the states right before the sampling.
 
 Software pipelining (``prefetch``, ``step(ingest=...)``): the priority write-back, the fused ingest
 of new collector steps and the NEXT iteration's sample + gather run on parallel branches of the
@@ -98,10 +100,6 @@ class LearnerStep:
                     # The shard states travel by PUT right after the priority write-back (no rank waits there) and the
                     # global sampling kernel waits for them itself: the exchange hides behind the backward pass, and the
                     # gradient exchange + clip + Adam is one launch whose CTAs wait on the signal pad themselves.
-                    self.state_by_put = os.environ.get("PB_PEER_STATE_PUT", "1") != "0"
-                    if not self.state_by_put:
-                        # one handshake per step: the states ride on the gradient exchange's barrier (one step stale)
-                        opt.peer_state = self.tree.state
                     self.all_state = self.peer.all_state
                     self._states_synced = False
                 except Exception as e:                                   # e.g. ranks on different boxes
@@ -110,15 +108,11 @@ class LearnerStep:
             if self.peer is None:
                 opt.allreduce = lambda flat: dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.pg)
             self.exchange = "peer" if self.peer is not None else "nccl"
-        if self.peer is None:
-            self.state_by_put = False
         self.launches_per_step = None
         self._side = None
         self._trace = None               # enable_trace(): device buffer of timeline marks
-        import os as _os
-        self.overlap_write_back = _os.environ.get("PB_OVERLAP_WRITEBACK", "1") != "0"
+        self._u_in_block = False         # the step's host uniforms ride in the fused ingest's staging block
         self._defer_mode, self._defer_ok = 0, False             # weight-gradient joins: see _capture / ops._JOINS
-        self._defer_enabled = _os.environ.get("PB_DEFER_WGRAD", "1") != "0"
 
     # ------------------------------------------------------------------------------------
     def _setup_prefetch(self):
@@ -176,30 +170,25 @@ class LearnerStep:
         return v, arena
 
     def sync_shard_states(self):
-        """Collective (every rank, same stream order): exchange the shard state blocks NOW.  The step graph gathers them
-        on its gradient exchange for the next step; this primes the first step and re-synchronises after anything
-        outside the step changed a tree (ingest, a manual priority update)."""
+        """Collective (every rank, same stream order): put this shard's state block to every rank NOW.  The step graph
+        puts it after its priority write-back for the next batch's sampling; this primes the first step and
+        re-synchronises after anything outside the step changed a tree (ingest, a manual priority update)."""
         if self.peer is not None:
-            if self.state_by_put:
-                self.peer.state_put(self.tree.state)
-            else:
-                self.peer.state_allgather(self.tree.state)
+            self.peer.state_put(self.tree.state)
             self._states_synced = True
 
     def _sample_gather(self, u, out, tag=""):
         """(shard states of all ranks ->) sample + fused n-step gather into ``out`` (live or shadow views)."""
         tree, ring = self.tree, self.ring
         if self.world_size > 1:
-            if self.peer is None:
-                import torch.distributed as dist
-                dist.all_gather_into_tensor(self.all_state.view(-1), tree.state, group=self.pg)
-                self._mark(tag + "shard_states_gathered")
-            if self.state_by_put:
+            if self.peer is not None:
                 # the kernel waits for the latest put of every rank (this step's tail, or sync_shard_states)
                 tree.sample_global_peer(self.peer, self.B_global, u, idx_out=out["idx"], weight_out=out["weight"],
                                         stratum_out=self.stratum)
             else:
-                # all_state was gathered by the previous step's exchange (or sync_shard_states)
+                import torch.distributed as dist
+                dist.all_gather_into_tensor(self.all_state.view(-1), tree.state, group=self.pg)
+                self._mark(tag + "shard_states_gathered")
                 tree.sample_global(self.world_size, self.rank, self.all_state, self.B_global, u,
                                    idx_out=out["idx"], weight_out=out["weight"], stratum_out=self.stratum)
         else:
@@ -224,9 +213,7 @@ class LearnerStep:
     def _body(self, refresh_table, draw, consume=False):
         tree, ring, agent, b = self.tree, self.ring, self.agent, self.buffer
         u = None if draw else self.u            # None: uniforms are drawn inside the sampling kernel
-        u_sel = consume and getattr(self, "_u_in_block", False)
-        dp_peer = self.peer is not None and not self.state_by_put       # states ride on the gradient exchange
-        dp_put = self.peer is not None and self.state_by_put
+        u_sel = consume and self._u_in_block
         mark = self._mark
         mark("start")
         if self.prefetch:
@@ -248,8 +235,6 @@ class LearnerStep:
         def write_back(td):
             self.td = td
             mark("loss_ready")
-            if not self.overlap_write_back:
-                return
             self._side.wait_stream(cur)
             side2 = _ops.fork_stream(self.device, "ingest") if consume else None
             if consume:
@@ -264,12 +249,12 @@ class LearnerStep:
                 if consume:
                     self.ingest.consume_tree()         # default priorities of the new steps, after the write-back
                     self._side.wait_stream(side2)
-                if dp_put:
+                if self.peer is not None:
                     self.peer.state_put(tree.state)            # this shard's new state -> every rank; nobody waits here
                     mark("tail:state_put")
-                if self.prefetch and u_sel:
-                    self.ingest.select_uniforms(self.u, after_counter_inc=True)
-                if self.prefetch and not dp_peer:
+                if self.prefetch:
+                    if u_sel:
+                        self.ingest.select_uniforms(self.u, after_counter_inc=True)
                     self._sample_gather(u, self._shadow, tag="tail:")      # next iteration's batch
                     mark("tail:next_batch_ready")
 
@@ -286,48 +271,12 @@ class LearnerStep:
             self._defer_ok = all(q in held for q in wgrad_ptrs)
         agent._static_distribution_loss, agent._static_q_loss, agent._static_total_loss = dl, ql, total
         mark("backward_done")
-        if dp_peer:
-            opt = agent.optimizer
-            if self.overlap_write_back:
-                cur.wait_stream(self._side)            # the tree state rides on the exchange: the tail must be done
-            pre = None
-            if self.prefetch:
-                pre = _ops.fork_stream(self.device, "prefetch")
-
-                def fork_prefetch():
-                    # the next batch needs THIS exchange's shard states: sampled beside the pulls + optimizer sweep
-                    pre.wait_stream(cur)
-                    with torch.cuda.stream(pre):
-                        self._sample_gather(u, self._shadow, tag="tail:")
-                        mark("tail:next_batch_ready")
-                opt.peer_after_exchange = fork_prefetch
-            try:
-                agent._optimizer_step(refresh_table=refresh_table)
-            finally:
-                opt.peer_after_exchange = None
-            if pre is not None:
-                cur.wait_stream(pre)
-        else:
-            agent._optimizer_step(refresh_table=refresh_table)
+        agent._optimizer_step(refresh_table=refresh_table)
         mark("optimizer_done")
         if self.loss_host is not None and total is not None:
             # device -> host read of the step's result as a node of the same graph (pinned scalar)
             self.loss_host.copy_(total.detach(), non_blocking=True)
-        if self.overlap_write_back:
-            if not dp_peer:
-                cur.wait_stream(self._side)
-        else:
-            if dp_peer:
-                raise _lib.PbError("PB_OVERLAP_WRITEBACK=0 needs the put-based state exchange under data parallelism")
-            tree.update_priority(idx, self.td, sorted=self.sorted)
-            if consume:
-                self.ingest.consume()
-            if dp_put:
-                self.peer.state_put(tree.state)
-            if self.prefetch:
-                if u_sel:
-                    self.ingest.select_uniforms(self.u, after_counter_inc=True)
-                self._sample_gather(u, self._shadow, tag="tail:")
+        cur.wait_stream(self._side)
         mark("end")
         return total
 
@@ -390,58 +339,37 @@ class LearnerStep:
         scatter into the ring and default priorities run inside the step graph, after the priority write-back and
         concurrently with backward / Adam (FusedIngest); they are sampleable from the next iteration on."""
         self.buffer._flush()
+        main = torch.cuda.current_stream(self.device).cuda_stream
         if ingest_block is not None:
             # a block planned by plan_ingest (uniforms inside), resident on the device: D2D into the staging slot
             if self.ingest is None:
                 raise _lib.PbError("plan_ingest() first")
-            main = torch.cuda.current_stream(self.device).cuda_stream
             parity = self.ingest.stage_device(ingest_block, main)
-            draw, consume, u_in_block = False, True, True
-            self._u_in_block = True
-            key = (draw, consume, u_in_block, self.ring.generation, float(self.tree._beta))
-            if self.use_cuda_graph and (self.graph is None or key != self._graph_key):
-                self._capture(draw, consume)
-                self._primed = False
-            if self.prefetch and (not self._primed or getattr(self.buffer, "_mutations", 0) != self._seen_mutations):
-                self._prime()
-            elif self.peer is not None and (not self._states_synced
-                                            or getattr(self.buffer, "_mutations", 0) != self._seen_mutations):
-                self.sync_shard_states()
-                self._seen_mutations = getattr(self.buffer, "_mutations", 0)
-            if not self.use_cuda_graph:
-                total = self._body(refresh_table=True, draw=draw, consume=consume)
-            else:
-                self.graph.replay()
-                total = self.agent._static_total_loss
-            self.ingest.mark_consumed(parity, main)
-            self.agent.n_updates += 1
-            return total
-        draw = u is None
-        # host uniforms + fused ingest: the uniforms ride in the ingest's staging block (one H2D copy per iteration) and
-        # are picked inside the graph by the replay counter
-        u_in_block = (not draw) and ingest is not None and isinstance(u, torch.Tensor) and u.device.type == "cpu" \
-            and u.dtype == torch.float64 and u.numel() == self.u.numel()
-        if u_in_block:
-            pass
-        elif not draw:
-            if u.device.type == "cpu" and u.dtype == torch.float64 and u.is_contiguous() and u.numel() == self.u.numel():
-                # host uniforms (pinned): one raw async copy on the step's stream
-                _lib.check(self._lib.pb_copy_h2d_async(self.u.data_ptr(), u.data_ptr(), 8 * self.u.numel(),
-                                                       torch.cuda.current_stream(self.device).cuda_stream), "pb_copy_h2d_async")
-            else:
-                self.u.copy_(u, non_blocking=True)
-        consume, parity = ingest is not None, None
-        if consume:
-            n = len(ingest[0])
-            if self.ingest is None or self.ingest.n != n:
-                from .experience.ring import FusedIngest
-                self.ingest = FusedIngest(self.ring, self.tree, n, n_uniforms=self.u.numel())
-            main = torch.cuda.current_stream(self.device).cuda_stream
-            parity = self.ingest.stage(*ingest, main_stream=main, u=u.numpy() if u_in_block else None)
-        self._u_in_block = u_in_block
+            draw, consume, self._u_in_block = False, True, True
+        else:
+            draw = u is None
+            # host uniforms + fused ingest: the uniforms ride in the ingest's staging block (one H2D copy per iteration)
+            # and are picked inside the graph by the replay counter
+            u_in_block = (not draw) and ingest is not None and isinstance(u, torch.Tensor) and u.device.type == "cpu" \
+                and u.dtype == torch.float64 and u.numel() == self.u.numel()
+            if not draw and not u_in_block:
+                if u.device.type == "cpu" and u.dtype == torch.float64 and u.is_contiguous() and u.numel() == self.u.numel():
+                    # host uniforms (pinned): one raw async copy on the step's stream
+                    _lib.check(self._lib.pb_copy_h2d_async(self.u.data_ptr(), u.data_ptr(), 8 * self.u.numel(), main),
+                               "pb_copy_h2d_async")
+                else:
+                    self.u.copy_(u, non_blocking=True)
+            consume, parity = ingest is not None, None
+            if consume:
+                n = len(ingest[0])
+                if self.ingest is None or self.ingest.n != n:
+                    from .experience.ring import FusedIngest
+                    self.ingest = FusedIngest(self.ring, self.tree, n, n_uniforms=self.u.numel())
+                parity = self.ingest.stage(*ingest, main_stream=main, u=u.numpy() if u_in_block else None)
+            self._u_in_block = u_in_block
         # the captured kernels hold the ring descriptor and beta BY VALUE: a grown aux pool (ring.generation) or a
         # new beta (learner.py:105-107 writes _sampler._beta every iteration) re-captures
-        key = (draw, consume, u_in_block, self.ring.generation, float(self.tree._beta))
+        key = (draw, consume, self._u_in_block, self.ring.generation, float(self.tree._beta))
         if self.use_cuda_graph and (self.graph is None or key != self._graph_key):
             if self.graph is not None and key[3] != self._graph_key[3]:
                 torch.cuda.synchronize(self.device)
@@ -501,7 +429,7 @@ class LearnerStep:
         with torch.cuda.stream(side):
             for it in range(3):
                 # first iteration: probe whether the weight-gradient joins can move to the optimizer (ops._JOINS)
-                self._defer_mode = (1 if it == 0 else (2 if self._defer_ok else 0)) if self._defer_enabled else 0
+                self._defer_mode = 1 if it == 0 else (2 if self._defer_ok else 0)
                 self._body(refresh_table=True, draw=draw)
         torch.cuda.current_stream(self.device).wait_stream(side)
         if flat:
@@ -511,8 +439,7 @@ class LearnerStep:
         torch.cuda.set_rng_state(rng, self.device)
         ag.quantile_rng_restore(q_rng)
         self._states_synced = False                         # the warm-up's exchanges carried warm-up tree states
-        self._graph_key = (draw, consume, getattr(self, "_u_in_block", False), self.ring.generation,
-                           float(self.tree._beta))
+        self._graph_key = (draw, consume, self._u_in_block, self.ring.generation, float(self.tree._beta))
         opt.zero_grad(set_to_none=True)
         self.graph = None                                   # release the previous graph's pool before capturing anew
         self.graph = torch.cuda.CUDAGraph()

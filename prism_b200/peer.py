@@ -142,20 +142,18 @@ class PeerGroup:
             raise _lib.PbError("peer exchange: a rank did not arrive within %.0f s (status 0x%x, rank %d of %d)"
                                % (WAIT_TIMEOUT_S, st, self.rank, self.world))
 
-    def allreduce_adam(self, opt, state=None, mark=None, after_exchange=None):
+    def allreduce_adam(self, opt, mark=None):
         """Sum the gradient arenas over the ranks and apply clip + Adam on every replica (csrc/peer.cu).
 
-        ONE cross-GPU handshake per step for small arenas: the exchange of the 64-byte shard state blocks (``state``:
-        this rank's tree state, gathered into ``self.all_state`` for the NEXT step's global sampling) is the barrier
-        that tells every rank all gradients are packed.  The arena is double-buffered by the parity of that exchange's
-        count, so a fast rank packing its next gradient never overwrites what a slower rank still pulls -- no trailing
-        barrier.  ``after_exchange``: called right after the handshake (LearnerStep forks the prefetch of the next batch
-        there, beside the pulls and the optimizer sweep)."""
+        ONE cross-GPU handshake per step for small arenas: it tells every rank all gradients are packed (the fused
+        launch signals on channel 1 itself; the multi-launch schedules run ``state_allgather`` of a dummy block).  The
+        arena is double-buffered by the parity of the handshake count, so a fast rank packing its next gradient never
+        overwrites what a slower rank still pulls -- no trailing barrier."""
         lib, st = _lib.load(), self._stream()
         mark = mark or (lambda name: None)                        # timeline marks of LearnerStep.enable_trace()
-        if (FUSED_EXCHANGE and state is None and after_exchange is None
-                and self.n <= int(lib.pb_peer_allreduce_adam_max_n()) and self.n * 4 * self.world <= ONE_SHOT_MAX_BYTES):
-            # small arena, nothing riding on the handshake: handshake + pulls + global norm + clip + Adam in ONE launch
+        if (FUSED_EXCHANGE and self.n <= int(lib.pb_peer_allreduce_adam_max_n())
+                and self.n * 4 * self.world <= ONE_SHOT_MAX_BYTES):
+            # small arena: handshake + pulls + global norm + clip + Adam in ONE launch
             _lib.check(lib.pb_peer_allreduce_adam(C.byref(self.c), self.n, opt.arena.data_ptr(), opt.exp_avg.data_ptr(),
                                                   opt.exp_avg_sq.data_ptr(), opt.step_count.data_ptr(), opt.lr,
                                                   opt.betas[0], opt.betas[1], opt.eps, opt.max_grad_norm,
@@ -164,10 +162,8 @@ class PeerGroup:
             self._n_gathers += 1                                  # channel 1 advanced: the other half of the arena is next
             mark("opt:applied")
             return
-        self.state_allgather(self._dummy_state if state is None else state)     # every rank packed its gradient
+        self.state_allgather(self._dummy_state)                   # every rank packed its gradient
         mark("opt:exchanged")
-        if after_exchange is not None:
-            after_exchange()
         if self.n * 4 * self.world <= ONE_SHOT_MAX_BYTES:
             # small arena: pulling every rank's gradient whole costs less than a second cross-GPU barrier
             n_part = C.c_int(0)

@@ -47,9 +47,9 @@ def run(label, setup=None):
 
 
 def no_tc():
-    old = ops.TENSOR_CORE_LINEAR
-    ops.TENSOR_CORE_LINEAR = False
-    return lambda: setattr(ops, "TENSOR_CORE_LINEAR", old)
+    old = ops.TC_MIN_FLOPS
+    ops.TC_MIN_FLOPS = float("inf")
+    return lambda: setattr(ops, "TC_MIN_FLOPS", old)
 
 
 def no_narrow():

@@ -36,22 +36,16 @@ def test_peer_allreduce_adam_matches_single_rank_step(world, n, one_shot, monkey
     _run_allreduce_adam(world, n)
 
 
-@pytest.mark.parametrize("world,n,two_phase", [(2, 4096, 0), (4, 4096, 0), (8, 4096, 0), (8, 4096, 1), (8, 40_000, 1),
-                                               (4, 40_000, 1), (2, 100_000, 0), (4, 100_000, 0), (2, 400_004, 0)])
-def test_peer_fused_allreduce_adam_matches_single_rank_step(world, n, two_phase, monkeypatch):
-    """Small arenas: handshake + pulls + global norm + clip + Adam as ONE launch per rank (peer_allreduce_adam_kernel):
-    one-shot pulls up to 4 ranks, two-phase (reduce-scatter by pull, all-gather by push, a second flag round) at 8.
+@pytest.mark.parametrize("world,n", [(2, 4096), (4, 4096), (8, 4096), (8, 40_000), (4, 40_000), (2, 100_000),
+                                     (4, 100_000), (2, 400_004)])
+def test_peer_fused_allreduce_adam_matches_single_rank_step(world, n, monkeypatch):
+    """Small arenas: handshake + pulls + global norm + clip + Adam as ONE launch per rank (peer_allreduce_adam_kernel),
+    every rank pulling every other rank's whole arena.
     Sizes are bounded here because the loopback ranks share one GPU: every rank's CTAs must be resident at once (in the
     multi-process set-up each rank has its own GPU; tests/test_gpu_multiprocess.py runs that)."""
-    from prism_b200 import _lib, peer as peer_mod
+    from prism_b200 import peer as peer_mod
     monkeypatch.setattr(peer_mod, "FUSED_EXCHANGE", True)
-    lib = _lib.load()
-    old = lib.pb_peer_two_phase_min(-1)
-    lib.pb_peer_two_phase_min(2 if two_phase else 0)
-    try:
-        _run_allreduce_adam(world, n)
-    finally:
-        lib.pb_peer_two_phase_min(old)
+    _run_allreduce_adam(world, n)
 
 
 def _run_allreduce_adam(world, n):
