@@ -534,6 +534,34 @@ int pb_peer_state_put(const pb_peer_group *g, const void *state64, void *stream)
 int pb_tree_sample_global_peer(const pb_tree *t, const pb_peer_group *g, long long n_global, const double *u, float beta,
                                long long *idx_out, float *weight_out, long long *stratum_out, void *stream);
 
+/* ------------------------------------------------------------------------- *
+ * Uniform replay (the reference's default, use_per = False: torchrl's uniform ReplayBuffer).
+ * The whole sampler is one 64-byte pb_per_state block; only len, seq, status, owned_lo / owned_n and pad[1..3]
+ * (rng ticket, call number, seed -- as for pb_tree_sample) are used, so pb_peer_state_put carries it unchanged.
+ * Every entry returns PB_E_ARG for a NULL state before it launches anything.
+ * ------------------------------------------------------------------------- */
+/* seq = the given value, len = min(seq, size), seed = pad[3], call number 0, status 0 (one single-thread launch) */
+int pb_uniform_init(pb_per_state *state, long long size, long long seq, int seed, void *stream);
+/* seq += n, len = min(seq, size): one single-thread launch, capturable (the ring's fused ingest) */
+int pb_uniform_extend(pb_per_state *state, long long size, long long n, void *stream);
+/* mode 0 iid: idx = (long long)(u_k * len); mode 1 stratified: idx = (long long)((k + u_k) / n * len) -- fp64,
+ * round-to-nearest, in that order; clamped to len - 1; weight 1.  u == NULL draws u_k on the device (Philox4x32-10,
+ * key pad[3], counter (k, pad[2]); the last CTA advances the call number).  len == 0 sets PB_ST_EMPTY. */
+int pb_uniform_sample(pb_per_state *state, long long n, const double *u, int mode, long long *idx_out,
+                      float *weight_out, void *stream);
+/* Global stratified uniform sampling over the concatenation of n_ranks shards (all_state: their gathered state
+ * blocks, only len is read): total = sum of len_r, g_k = (long long)((k + u_k) / n_global * total) clamped to
+ * total - 1, owner from the prefix sums of len_r, local index g_k - prefix[rank].  This rank's strata form one
+ * contiguous run; outputs are compacted to [0, owned_n) and the run is written to owned_lo / owned_n.  Rows past it
+ * get idx -1, weight 0, stratum -1.  stratum_out optional. */
+int pb_uniform_sample_global(pb_per_state *state, int n_ranks, int rank, const pb_per_state *all_state,
+                             long long n_global, const double *u, long long *idx_out, float *weight_out,
+                             long long *stratum_out, void *stream);
+/* pb_uniform_sample_global on the states of the latest pb_peer_state_put exchange (bounded wait as for
+ * pb_tree_sample_global_peer: bit 2 of *g->status on a timeout). */
+int pb_uniform_sample_global_peer(pb_per_state *state, const pb_peer_group *g, long long n_global, const double *u,
+                                  long long *idx_out, float *weight_out, long long *stratum_out, void *stream);
+
 /* LayerNorm over the last dimension of a (rows x F) fp32 matrix, forward and backward (csrc/ln.cu), for the
  * (T*B)-row IQN activations (nn.LayerNorm in ffnn_model.py:17-18, iqn_model.py:42-46).  F % 4 == 0, F <= 4096,
  * 16-byte aligned pointers.  gamma / beta may be NULL (no affine); mean_out / rstd_out may be NULL (no backward).

@@ -140,6 +140,11 @@ SIGNATURES = {
     "pb_peer_state_put": [_PEER, _P, _P],
     "pb_peer_trace": [_I, _P, _I],
     "pb_tree_sample_global_peer": [_TREE, _PEER, _LL, _P, _F, _P, _P, _P, _P],
+    "pb_uniform_init": [_P, _LL, _LL, _I, _P],
+    "pb_uniform_extend": [_P, _LL, _LL, _P],
+    "pb_uniform_sample": [_P, _LL, _P, _I, _P, _P, _P],
+    "pb_uniform_sample_global": [_P, _I, _I, _P, _LL, _P, _P, _P, _P, _P],
+    "pb_uniform_sample_global_peer": [_P, _PEER, _LL, _P, _P, _P, _P, _P],
     "pb_layer_norm_supported": [_LL, _I],
     "pb_layer_norm_bwd_blocks": [_LL, _I],
     "pb_layer_norm_fwd": [_LL, _I, _F, _P, _P, _P, _P, _P, _P, _P],

@@ -104,4 +104,97 @@ __device__ __forceinline__ float warp_max(float v)
     return v;
 }
 
+__device__ __forceinline__ unsigned long long global_ns()
+{
+    unsigned long long v;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(v));
+    return v;
+}
+
+// ---------------------------------------------------------------------------------
+// device-side uniforms of the replay samplers (per_tree.cu, uniform.cu): Philox4x32-10 keyed by the shard seed,
+// counter = (sample number, call number).  Every rank of a sharded buffer draws the same u_k without communication;
+// the call number lives in the state block (pad[2], seed pad[3]) and is advanced by the last CTA of the launch (ticket
+// pad[1]), so a replayed CUDA graph gets fresh numbers every iteration with no extra launch.
+// ---------------------------------------------------------------------------------
+__device__ __forceinline__ double philox_uniform(unsigned seed, unsigned call, unsigned long long k)
+{
+    unsigned c0 = (unsigned)k, c1 = (unsigned)(k >> 32), c2 = call, c3 = 0x50455221u;
+    unsigned k0 = seed, k1 = 0x9E3779B9u ^ seed;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const unsigned hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const unsigned hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    // 53 random bits -> [0, 1)
+    return ((double)(c0 >> 5) * 67108864.0 + (double)(c1 >> 6)) * (1.0 / 9007199254740992.0);
+}
+
+__device__ __forceinline__ void rng_advance(pb_per_state *st)
+{
+    // call after a __syncthreads(): every thread of this CTA has read the call number
+    if (threadIdx.x == 0) {
+        __threadfence();
+        const int ticket = atomicAdd(&st->pad[1], 1);
+        if (ticket == (int)(gridDim.x * gridDim.y) - 1) {
+            st->pad[2] += 1;
+            st->pad[1] = 0;
+        }
+    }
+}
+
+// peer wait of the global samplers (pb_tree_sample_global_peer, pb_uniform_sample_global_peer): the shard states were
+// PUT into this rank's slots by every rank (peer_state_put_kernel, csrc/peer.cu); every CTA waits on the local signal
+// pad until all ranks' puts of the current exchange have landed (bounded: gives up after timeout_ns and raises bit 2 of
+// *status), then reads the slot.
+struct PeerWait {
+    const unsigned long long *flags;      // local pad, channel 2: [src] = number of that rank's completed puts
+    const unsigned long long *epoch;      // local count of this rank's own puts (the exchange to wait for)
+    const unsigned char *slots;           // local state area: slot (2 + (epoch & 1)) holds the blocks of that exchange
+    unsigned int *status;
+    unsigned long long timeout_ns;
+    int slot_bytes;                       // bytes per slot
+};
+
+// gathered shard states may sit in peer-mapped memory that other GPUs write: read them past this SM's L1
+__device__ __forceinline__ float ld_state_f32(const float *p)
+{
+    float v;
+    asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ long long ld_state_s64(const long long *p)
+{
+    long long v;
+    asm volatile("ld.volatile.global.s64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+// every thread of the CTA: wait for the puts of G ranks (pw.flags set), returns the slot holding their state blocks
+__device__ __forceinline__ const pb_per_state *peer_wait_states(const PeerWait &pw, int G)
+{
+    const unsigned long long e = *pw.epoch;
+    if (threadIdx.x < G) {
+        const unsigned long long *f = pw.flags + threadIdx.x;
+        unsigned long long v;
+        asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(f) : "memory");
+        if (v < e) {
+            const unsigned long long t0 = global_ns();
+            unsigned spins = 0;
+            for (;;) {
+                asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(f) : "memory");
+                if (v >= e) break;
+                if ((++spins & 1023u) == 0 && pw.timeout_ns && global_ns() - t0 > pw.timeout_ns) {
+                    if (pw.status) atomicOr(pw.status, 1u << 2);
+                    break;
+                }
+            }
+        }
+    }
+    __syncthreads();
+    return reinterpret_cast<const pb_per_state *>(pw.slots + (size_t)(2 + (e & 1)) * pw.slot_bytes);
+}
+
 }  // namespace pb

@@ -92,12 +92,6 @@ constexpr int TRACE_SLOTS = 48;
 __device__ unsigned long long g_trace[TRACE_SLOTS];
 __device__ int g_trace_on;
 
-__device__ __forceinline__ unsigned long long global_ns()
-{
-    unsigned long long v;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(v));
-    return v;
-}
 // `on` = g_trace_on read ONCE at kernel entry (TRACE_ON).  Call from one thread per CTA (or per warp).
 #define TRACE_ON() (__ldg(&g_trace_on))
 __device__ __forceinline__ void trace_max(int on, int slot)
@@ -937,39 +931,7 @@ __device__ __forceinline__ float is_weight(float leaf, float p_min, float beta, 
     return (float)pow_cold((double)ratio, -(double)beta);
 }
 
-// ---------------------------------------------------------------------------------
-// device-side uniforms: Philox4x32-10 keyed by the shard seed, counter = (sample number, call number).
-// Every rank of a sharded buffer draws the same u_k without communication; the call number lives in
-// the state block and is advanced by the last CTA of the launch (ticket), so a replayed CUDA graph
-// gets fresh numbers every iteration with no extra launch.
-// ---------------------------------------------------------------------------------
-__device__ __forceinline__ double philox_uniform(unsigned seed, unsigned call, unsigned long long k)
-{
-    unsigned c0 = (unsigned)k, c1 = (unsigned)(k >> 32), c2 = call, c3 = 0x50455221u;
-    unsigned k0 = seed, k1 = 0x9E3779B9u ^ seed;
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const unsigned hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const unsigned hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    // 53 random bits -> [0, 1)
-    return ((double)(c0 >> 5) * 67108864.0 + (double)(c1 >> 6)) * (1.0 / 9007199254740992.0);
-}
-
-__device__ __forceinline__ void rng_advance(const TreeView &t)
-{
-    // call after a __syncthreads(): every thread of this CTA has read the call number
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const int ticket = atomicAdd(&t.st->pad[1], 1);
-        if (ticket == (int)(gridDim.x * gridDim.y) - 1) {
-            t.st->pad[2] += 1;
-            t.st->pad[1] = 0;
-        }
-    }
-}
+// device-side uniforms: philox_uniform / rng_advance (common.cuh), keyed by the state block's seed and call number
 
 __device__ __forceinline__ float stratified_mass(long long k, double uk, long long n, float total)
 {
@@ -1030,7 +992,7 @@ __global__ void __launch_bounds__(256) tree_sample_kernel(TreeView t, long long 
         }
     }
     if (threadIdx.x == 0) trace_max(tr_on, TR_SAMPLE_END);
-    if (!u) { __syncthreads(); rng_advance(t); }
+    if (!u) { __syncthreads(); rng_advance(t.st); }
 }
 
 // ---------------------------------------------------------------------------------
@@ -1215,7 +1177,7 @@ __global__ void __launch_bounds__(ST_THREADS) tree_sample_thread_kernel(TreeView
         }
     }
     if (threadIdx.x == 0) trace_max(tr_on, TR_SAMPLE_END);
-    if (!u) { __syncthreads(); rng_advance(t); }
+    if (!u) { __syncthreads(); rng_advance(t.st); }
 }
 
 // ---------------------------------------------------------------------------------
@@ -1231,20 +1193,6 @@ struct GlobalTop {
     float pmin;
     long long lo, hi;           // this rank owns strata [lo, hi)
 };
-
-// all_state may sit in peer-mapped memory that other GPUs write: read it past this SM's L1
-__device__ __forceinline__ float ld_state_f32(const float *p)
-{
-    float v;
-    asm volatile("ld.volatile.global.f32 %0, [%1];" : "=f"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ long long ld_state_s64(const long long *p)
-{
-    long long v;
-    asm volatile("ld.volatile.global.s64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
 
 __device__ __forceinline__ void build_top(GlobalTop *g, const pb_per_state *all_state, int G)
 {
@@ -1306,18 +1254,7 @@ __device__ long long first_owned(const GlobalTop &g, int G, long long n, int ran
     return hi;
 }
 
-// peer wait (pb_tree_sample_global_peer): the shard states were PUT into this rank's slots by every rank
-// (peer_state_put_kernel, csrc/peer.cu); every CTA waits on the local signal pad until all ranks' puts of the current
-// exchange have landed (bounded: gives up after timeout_ns and raises bit 2 of *status), then reads the slot.
-struct PeerWait {
-    const unsigned long long *flags;      // local pad, channel 2: [src] = number of that rank's completed puts
-    const unsigned long long *epoch;      // local count of this rank's own puts (the exchange to wait for)
-    const unsigned char *slots;           // local state area: slot (2 + (epoch & 1)) holds the blocks of that exchange
-    unsigned int *status;
-    unsigned long long timeout_ns;
-    int slot_bytes;                       // bytes per slot
-};
-
+// peer wait (pb_tree_sample_global_peer): PeerWait / peer_wait_states, common.cuh
 __global__ void __launch_bounds__(256) global_sample_kernel(TreeView t, const pb_per_state *all_state, int G, int rank,
                                                             long long n_global, const double *u, float beta,
                                                             long long *idx_out, float *w_out, long long *stratum_out,
@@ -1326,28 +1263,7 @@ __global__ void __launch_bounds__(256) global_sample_kernel(TreeView t, const pb
     pdl_wait();                                                   // programmatic dependent launch (PB_LAUNCH_PDL)
     pdl_trigger();
     __shared__ GlobalTop g;
-    if (pw.flags) {
-        const unsigned long long e = *pw.epoch;
-        if (threadIdx.x < G) {
-            const unsigned long long *f = pw.flags + threadIdx.x;
-            unsigned long long v;
-            asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(f) : "memory");
-            if (v < e) {
-                const unsigned long long t0 = global_ns();
-                unsigned spins = 0;
-                for (;;) {
-                    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(f) : "memory");
-                    if (v >= e) break;
-                    if ((++spins & 1023u) == 0 && pw.timeout_ns && global_ns() - t0 > pw.timeout_ns) {
-                        if (pw.status) atomicOr(pw.status, 1u << 2);
-                        break;
-                    }
-                }
-            }
-        }
-        __syncthreads();
-        all_state = reinterpret_cast<const pb_per_state *>(pw.slots + (size_t)(2 + (e & 1)) * pw.slot_bytes);
-    }
+    if (pw.flags) all_state = peer_wait_states(pw, G);
     build_top(&g, all_state, G);
     const unsigned call = (unsigned)t.st->pad[2], seed = (unsigned)t.st->pad[3];
     if (threadIdx.x < 32) {
@@ -1393,7 +1309,7 @@ __global__ void __launch_bounds__(256) global_sample_kernel(TreeView t, const pb
             }
         }
     }
-    if (!u) { __syncthreads(); rng_advance(t); }
+    if (!u) { __syncthreads(); rng_advance(t.st); }
 }
 
 // ---------------------------------------------------------------------------------

@@ -20,12 +20,16 @@ NCCL, which all-gathers the states right before the sampling.
 Software pipelining (``prefetch``, ``step(ingest=...)``): the priority write-back, the fused ingest
 of new collector steps and the NEXT iteration's sample + gather run on parallel branches of the
 same graph while backward / exchange / Adam proceed (DESIGN.md section 6).
+
+Uniform replay (``use_per=False``, the reference's default): the buffer has no priority store, so the step owns a
+UniformSampler (csrc/uniform.cu) in its place -- the same schedule without the priority write-back, weights 1.
 """
 import torch
 
 from . import _lib
 from .agents.optim import FlatAdam
 from .experience.per import PrioritizedTree
+from .experience.uniform import UniformSampler
 
 
 class LearnerStep:
@@ -33,10 +37,19 @@ class LearnerStep:
                  rank=0, world_size=1, pad_slack=None, exchange=None, prefetch=False):
         self.buffer, self.agent = buffer, agent
         self._lib = _lib.load()
+        buffer._flush()
         self.tree = buffer.buffer._sampler
         self.ring = buffer.buffer._storage
-        if self.ring is None or self.tree is None:
-            raise _lib.PbError("LearnerStep needs a prioritized buffer that already holds transitions")
+        if self.ring is None:
+            raise _lib.PbError("LearnerStep needs a buffer that already holds transitions")
+        # uniform replay: the step owns the sampler.  Its length lives on the device and advances when a replay
+        # consumes an ingest block; the host's ring.seq advances when a block is filled (planned or staged).  _seq_seen
+        # mirrors ring.seq through this step's own fills, _pending counts the filled steps no replay has consumed yet.
+        self.uniform = self.tree is None
+        if self.uniform:
+            self.tree = UniformSampler(self.ring.size, mode=buffer.buffer.sampling, seq=self.ring.seq,
+                                       device=self.ring.device)
+            self._seq_seen, self._pending = self.ring.seq, 0
         self.device = torch.device(buffer.device)
         self.B = int(batch_size or buffer.buffer._batch_size)
         self.world_size, self.rank, self.pg = int(world_size), int(rank), process_group
@@ -67,7 +80,6 @@ class LearnerStep:
         self._primed, self._seen_mutations = False, None
         self.loss_host = None            # enable_loss_readback(): pinned fp32 scalar written by every step
         # static batch, shared by the buffer (writes) and the agent (reads)
-        buffer._flush()
         self._n_rows = n_rows
         self._live = None
         if self.prefetch:
@@ -172,7 +184,8 @@ class LearnerStep:
     def sync_shard_states(self):
         """Collective (every rank, same stream order): put this shard's state block to every rank NOW.  The step graph
         puts it after its priority write-back for the next batch's sampling; this primes the first step and
-        re-synchronises after anything outside the step changed a tree (ingest, a manual priority update)."""
+        re-synchronises after anything outside the step changed a tree or, under uniform replay, the ring's length
+        (ingest, a manual priority update, ``empty()``)."""
         if self.peer is not None:
             self.peer.state_put(self.tree.state)
             self._states_synced = True
@@ -244,8 +257,9 @@ class LearnerStep:
                     self.ingest.consume_ring()
                     mark("tail:ring_ingested")
             with torch.cuda.stream(self._side):
-                tree.update_priority(idx, td, sorted=self.sorted)      # |td| is taken inside the kernel
-                mark("tail:priorities_written")
+                if not self.uniform:                                   # uniform replay: no priorities to write back
+                    tree.update_priority(idx, td, sorted=self.sorted)  # |td| is taken inside the kernel
+                    mark("tail:priorities_written")
                 if consume:
                     self.ingest.consume_tree()         # default priorities of the new steps, after the write-back
                     self._side.wait_stream(side2)
@@ -329,7 +343,28 @@ class LearnerStep:
         if self.ingest is None or self.ingest.n != n:
             from .experience.ring import FusedIngest
             self.ingest = FusedIngest(self.ring, self.tree, n, n_uniforms=self.u.numel())
-        return self.ingest.plan_block(*ingest, u=None if u is None else u.numpy() if isinstance(u, torch.Tensor) else u)
+        self._sync_uniform_length()
+        block = self.ingest.plan_block(*ingest, u=None if u is None else u.numpy() if isinstance(u, torch.Tensor) else u)
+        self._filled(n)
+        return block
+
+    def _filled(self, n):
+        """Host bookkeeping of uniform replay: this step's FusedIngest filled n more steps (ring.seq advanced)."""
+        if self.uniform:
+            self._seq_seen += n
+            self._pending += n
+
+    def _sync_uniform_length(self):
+        """Uniform replay: if something outside this step changed the ring (eager extend / extend_batch, an
+        ``ingest_graph`` push, ``empty()``, ``load``), set the device length to what the ring will hold once the
+        blocks already filled for this step are consumed.  Stream order makes the value right even while a push is
+        still in flight.  The next step samples its prefetched batch again and, under data parallelism, puts the state
+        block first (sync_shard_states)."""
+        if not self.uniform or self.ring.seq == self._seq_seen:
+            return
+        self.tree.resync(self.ring.seq - self._pending)
+        self._seq_seen = self.ring.seq
+        self._primed = self._states_synced = False
 
     def step(self, u=None, ingest=None, ingest_block=None):
         """Run one iteration.  ``u`` (optional): fp64 uniforms (device or pinned-host tensor, B_global
@@ -339,6 +374,7 @@ class LearnerStep:
         scatter into the ring and default priorities run inside the step graph, after the priority write-back and
         concurrently with backward / Adam (FusedIngest); they are sampleable from the next iteration on."""
         self.buffer._flush()
+        self._sync_uniform_length()
         main = torch.cuda.current_stream(self.device).cuda_stream
         if ingest_block is not None:
             # a block planned by plan_ingest (uniforms inside), resident on the device: D2D into the staging slot
@@ -366,10 +402,11 @@ class LearnerStep:
                     from .experience.ring import FusedIngest
                     self.ingest = FusedIngest(self.ring, self.tree, n, n_uniforms=self.u.numel())
                 parity = self.ingest.stage(*ingest, main_stream=main, u=u.numpy() if u_in_block else None)
+                self._filled(n)
             self._u_in_block = u_in_block
         # the captured kernels hold the ring descriptor and beta BY VALUE: a grown aux pool (ring.generation) or a
         # new beta (learner.py:105-107 writes _sampler._beta every iteration) re-captures
-        key = (draw, consume, self._u_in_block, self.ring.generation, float(self.tree._beta))
+        key = (draw, consume, self._u_in_block, self.ring.generation, self._beta_key())
         if self.use_cuda_graph and (self.graph is None or key != self._graph_key):
             if self.graph is not None and key[3] != self._graph_key[3]:
                 torch.cuda.synchronize(self.device)
@@ -388,8 +425,13 @@ class LearnerStep:
             total = self.agent._static_total_loss
         if consume:
             self.ingest.mark_consumed(parity, main)
+            if self.uniform:
+                self._pending -= self.ingest.n
         self.agent.n_updates += 1
         return total
+
+    def _beta_key(self):
+        return None if self.uniform else float(self.tree._beta)
 
     def enable_loss_readback(self):
         """Every following step also copies its total loss into ``self.loss_host`` (pinned fp32 scalar): the
@@ -439,7 +481,7 @@ class LearnerStep:
         torch.cuda.set_rng_state(rng, self.device)
         ag.quantile_rng_restore(q_rng)
         self._states_synced = False                         # the warm-up's exchanges carried warm-up tree states
-        self._graph_key = (draw, consume, self._u_in_block, self.ring.generation, float(self.tree._beta))
+        self._graph_key = (draw, consume, self._u_in_block, self.ring.generation, self._beta_key())
         opt.zero_grad(set_to_none=True)
         self.graph = None                                   # release the previous graph's pool before capturing anew
         self.graph = torch.cuda.CUDAGraph()
