@@ -399,7 +399,12 @@ int pb_adam_clip_step(long long n, float *param, const float *grad, float *exp_a
  * x (B, H, W, C) channels-last fp32 -> conv3x3 stride 1 no padding (weight (OC, C, 3, 3), torch layout)
  * + bias + ReLU -> out (B, OC*(H-2)*(W-2)) in NCHW-flatten order.
  * Backward (observations need no gradient): dw (OC, C, 3, 3), db (OC) from dout masked by out > 0;
- * partial_scratch holds pb_conv3x3_relu_bwd_groups(B) * (OC*C*9 + OC) floats. */
+ * partial_scratch holds pb_conv3x3_relu_bwd_groups(B) * (OC*C*9 + OC) floats.
+ * pb_conv3x3_relu_supported: 1 when both entries accept an H x W x C frame with OC filters (at most 2048 weights +
+ * biases, 4096 frame floats, 6272 output floats per image, 48 KB of shared memory per CTA), else 0: run the
+ * convolution elsewhere.  The backward takes the tensor cores for OC == 16, an output plane that is a multiple of 8
+ * and at most 64, and 4 <= C <= 10; every other accepted shape takes the FMA kernel. */
+int pb_conv3x3_relu_supported(int H, int W, int C, int OC);
 int pb_conv3x3_relu_fwd(int B, int H, int W, int C, int OC, const float *x, const float *w,
                         const float *bias, float *out, void *stream);
 int pb_conv3x3_relu_bwd_groups(int B);

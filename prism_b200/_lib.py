@@ -118,6 +118,7 @@ SIGNATURES = {
     "pb_grad_sumsq": [_LL, _P, _P, _P, _P, _P],
     "pb_adam_clip_apply": [_LL, _P, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _I, _P, _P],
     "pb_loss_combine": [_I, _P, _P, _P, _F, _P, _P, _P, _P],
+    "pb_conv3x3_relu_supported": [_I, _I, _I, _I],
     "pb_conv3x3_relu_fwd": [_I, _I, _I, _I, _I, _P, _P, _P, _P, _P],
     "pb_conv3x3_relu_bwd_groups": [_I],
     "pb_conv3x3_relu_bwd": [_I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P],

@@ -1,9 +1,10 @@
 """Embedding CNNs (MinAtar single-conv net, Nature-DQN three-conv net).
 
 Constructor arguments and ``model.<i>`` parameter names match the reference
-(prism/agents/models/minatar_cnn_model.py:7-46, atari_cnn_model.py:7-59).  Convolutions stay
-on cuDNN through PyTorch: the north star names only the IQN / MLP GEMMs and the PER path.
+(prism/agents/models/minatar_cnn_model.py:7-46, atari_cnn_model.py:7-59).  The MinAtar embedding runs on
+csrc/conv.cu; the Nature-DQN convolutions stay on cuDNN through PyTorch.
 """
+import functools
 import math
 
 import torch
@@ -25,12 +26,31 @@ def _sparse_conv_init(net, p_zero):
             flat[c, torch.randperm(fan_in)[:n_zero]] = 0.0
 
 
+@functools.lru_cache(maxsize=None)
+def _conv_kernel_supports(H, W, C, OC):
+    from ... import _lib
+    return bool(_lib.load().pb_conv3x3_relu_supported(H, W, C, OC))
+
+
+def _conv_kernel_takes(hwc, conv):
+    """A (H, W, C) frame goes through the conv kernel: its channels match the layer (a mismatch takes nn.Conv2d, which
+    reports it) and pb_conv3x3_relu_supported accepts the shape."""
+    H, W, C = (int(s) for s in hwc)
+    return C == conv.in_channels and _conv_kernel_supports(H, W, C, conv.out_channels)
+
+
 def _probe_dim(net, *shape):
     with torch.no_grad():
         return net(torch.zeros(1, *shape)).numel()
 
 
 class MinAtarModel(nn.Module):
+    """On CUDA, conv + bias + ReLU + flatten run as one kernel (``ops.conv3x3_relu_flatten``) whenever
+    ``pb_conv3x3_relu_supported`` accepts the frame (C <= 14 for 10x10 frames).  Other frames take ``self.model`` on
+    cuDNN, with cuDNN's TF32 path switched off process-wide at construction, as in ``NatureAtariCnn``: the backward
+    runs later in the autograd engine, so a context manager around ``forward`` would not cover it, and TF32 (~1e-3)
+    would miss the fp32 accuracy that the kernel and the reference hold."""
+
     def __init__(self, in_channels, act_fn=nn.ReLU, device="cpu", use_layer_norm=False, sparse_init_p=0.0):
         super().__init__()
         net = nn.Sequential(nn.Conv2d(in_channels, 16, kernel_size=3, stride=1), act_fn(), nn.Flatten())
@@ -38,11 +58,12 @@ class MinAtarModel(nn.Module):
         if sparse_init_p > 0:
             _sparse_conv_init(net, sparse_init_p)
         self.model = net.to(device)
+        torch.backends.cudnn.allow_tf32 = False
 
     def forward(self, x):
         # MinAtar observations are channels-last (10, 10, C)
         conv = self.model[0]
-        if x.is_cuda and isinstance(self.model[1], nn.ReLU) and x.dim() == 4 and x.shape[1] <= 16 and x.shape[2] <= 16:
+        if x.is_cuda and isinstance(self.model[1], nn.ReLU) and x.dim() == 4 and _conv_kernel_takes(x.shape[1:], conv):
             from .. import ops
             return ops.conv3x3_relu_flatten(x.float(), conv.weight, conv.bias)   # conv+bias+ReLU+flatten: one launch
         return self.model(x.permute(0, 3, 1, 2).float())

@@ -35,10 +35,12 @@ __host__ __device__ inline int frame_pitch(int W) { return ((W + 7) / 16) * 16 +
 
 // channels-last word i of a frame -> its word in the staged layout.  mC, mW = div_magic(C), div_magic(W): the staging
 // loop maps 8 words per thread, and two runtime divisions each were a third of the forward kernel's instructions.
-__device__ __forceinline__ unsigned div_magic(int d) { return 0xFFFFFFFFu / (unsigned)d + 1u; }   // n / d == umulhi(n, magic), n < 2^32 / d
+// n / d == umulhi(n, magic) for 2 <= d, n < 2^32 / d.  d = 1 would need 2^32: the magic wraps to 0.
+__device__ __forceinline__ unsigned div_magic(int d) { return 0xFFFFFFFFu / (unsigned)d + 1u; }
 __device__ __forceinline__ int frame_slot(int i, int H, int W, int C, int P, unsigned mC, unsigned mW)
 {
-    const int pix = (int)__umulhi((unsigned)i, mC), c = i - pix * C;
+    // W >= 3 always; a one-channel frame (C = 1) is its own pixel index
+    const int pix = C == 1 ? i : (int)__umulhi((unsigned)i, mC), c = i - pix * C;
     const int y = (int)__umulhi((unsigned)pix, mW), x = pix - y * W;
     return (c * H + y) * P + x;
 }
@@ -322,17 +324,35 @@ __global__ void __launch_bounds__(256) conv_bwd_reduce_kernel(int n_groups, int 
     }
 }
 
+// dynamic shared memory of the forward and of the FMA backward (the tensor-core backward is a fast path: a shape it
+// cannot stage takes the FMA kernel, so its own limit never refuses a shape)
+size_t fwd_smem(const ConvDims &d)
+{
+    const int ocp = (d.OC + OCG - 1) / OCG * OCG;
+    return sizeof(float) * (size_t)(d.H * frame_pitch(d.W) * d.C + ocp * d.C * 9);
+}
+size_t fma_bwd_smem(const ConvDims &d) { return sizeof(float) * (size_t)(d.H * d.W * d.C + d.OC * d.OH * d.OW); }
+
+// every limit of both entries: pb_conv3x3_relu_supported answers with the same function, so they cannot drift apart
 int check_dims(const ConvDims &d)
 {
     if (d.B <= 0 || d.H < 3 || d.W < 3 || d.C <= 0 || d.OC <= 0) return PB_E_ARG;
-    if (d.H * d.W * d.C > MAX_X || d.OC * d.C * 9 > MAX_W || d.OC * d.OH * d.OW > MAX_OUT) return PB_E_UNSUPPORTED;
-    if (d.OC * d.C * 9 + d.OC > 8 * 256) return PB_E_UNSUPPORTED;
+    const long long H = d.H, W = d.W, C = d.C, OC = d.OC;          // no int overflow for absurd arguments
+    if (H * W * C > MAX_X || OC * C * 9 > MAX_W || OC * (H - 2) * (W - 2) > MAX_OUT) return PB_E_UNSUPPORTED;
+    if (OC * C * 9 + OC > 8 * 256) return PB_E_UNSUPPORTED;         // FMA backward: 8 gradient elements per thread
+    if (fwd_smem(d) > 48 * 1024 || fma_bwd_smem(d) > 48 * 1024) return PB_E_UNSUPPORTED;
     return PB_OK;
 }
 
 }  // namespace
 
 extern "C" {
+
+int pb_conv3x3_relu_supported(int H, int W, int C, int OC)
+{
+    const ConvDims d = {1, H, W, C, OC, H - 2, W - 2};
+    return check_dims(d) == PB_OK ? 1 : 0;
+}
 
 int pb_conv3x3_relu_fwd(int B, int H, int W, int C, int OC, const float *x, const float *w, const float *bias,
                         float *out, void *stream)
@@ -342,8 +362,7 @@ int pb_conv3x3_relu_fwd(int B, int H, int W, int C, int OC, const float *x, cons
     if (rc) return rc;
     if (!x || !w || !out) return PB_E_ARG;
     const int ocp = (OC + 7) / 8 * 8;
-    const size_t smem = sizeof(float) * (size_t)(H * frame_pitch(W) * C + ocp * C * 9);
-    if (smem > 48 * 1024) return PB_E_UNSUPPORTED;
+    const size_t smem = fwd_smem(d);
     const int items = d.OH * d.OW * (ocp / 8);
     const int threads = items >= 256 ? 256 : (items + 31) / 32 * 32;
     PB_LAUNCH_PDL_CHAIN(conv3x3_relu_fwd_kernel, (unsigned)B, threads, smem, stream, d, x, w, bias, out);
@@ -384,8 +403,7 @@ int pb_conv3x3_relu_bwd(int B, int H, int W, int C, int OC, const float *x, cons
         }
     }
 fma_path:
-    const size_t smem = sizeof(float) * (size_t)(H * W * C + OC * d.OH * d.OW);
-    if (smem > 48 * 1024) return PB_E_UNSUPPORTED;
+    const size_t smem = fma_bwd_smem(d);
     // two gradient elements per thread for the MinAtar embedding (880 elements, 512 threads): several CTAs per SM, so
     // one CTA's staging loads overlap another's FMA loop and the 256 per-sample CTAs are resident in one wave
     const int ne_all = OC * C * 9 + OC;
