@@ -395,6 +395,28 @@ int pb_adam_clip_step(long long n, float *param, const float *grad, float *exp_a
                       long long *step_count, float lr, float beta1, float beta2, float adam_eps,
                       float max_grad_norm, float *norm_out, float *partial_scratch, void *stream);
 
+/* The same kernels with the update rule as a parameter: clip_grad_norm_ + {Adam, RMSprop, SGD} (the three optimizers of
+ * prism/factory/agent_factory.py:40-58), torch.optim's arithmetic in its foreach order.  Hyper-parameters (lr, h1, h2,
+ * eps) and the two state arrays per rule:
+ *   PB_OPT_ADAM               h1 = beta1, h2 = beta2       m = exp_avg, v = exp_avg_sq (bias correction from *step_count)
+ *   PB_OPT_RMSPROP            h1 = alpha, h2 unused        v = square_avg; m unused (may be NULL)
+ *   PB_OPT_RMSPROP_CENTERED   h1 = alpha, h2 unused        m = grad_avg, v = square_avg
+ *   PB_OPT_SGD                h1, h2, eps unused           none: m and v are neither read nor written (may be NULL)
+ * Every rule advances *step_count.  An unknown rule, or a NULL state array the rule reads, is PB_E_ARG (nothing is
+ * launched).  The PB_OPT_ADAM calls are the pb_adam_* entries above.  Each rule's fused kernel has its own occupancy:
+ * pb_opt_fused_max_n(rule) is its limit (0 for an unknown rule). */
+#define PB_OPT_ADAM 0
+#define PB_OPT_RMSPROP 1
+#define PB_OPT_RMSPROP_CENTERED 2
+#define PB_OPT_SGD 3
+long long pb_opt_fused_max_n(int rule);
+int pb_opt_fused_step(int rule, int n_tensors, const long long *table, float scale, long long n, float *param, float *grad,
+                      float *m, float *v, long long *step_count, float lr, float h1, float h2, float eps,
+                      float max_grad_norm, float *partial_scratch, float *norm_out, void *stream);
+int pb_opt_clip_apply(int rule, long long n, float *param, const float *grad, float *m, float *v,
+                      const long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                      const float *partial_scratch, int n_partials, float *norm_out, void *stream);
+
 /* MinAtarModel embedding (prism/agents/models/minatar_cnn_model.py:13-18, 41-44) in one launch:
  * x (B, H, W, C) channels-last fp32 -> conv3x3 stride 1 no padding (weight (OC, C, 3, 3), torch layout)
  * + bias + ReLU -> out (B, OC*(H-2)*(W-2)) in NCHW-flatten order.
@@ -527,6 +549,15 @@ long long pb_peer_allreduce_adam_max_n(void);
 int pb_peer_allreduce_adam(const pb_peer_group *g, long long n, float *param, float *exp_avg, float *exp_avg_sq,
                            long long *step_count, float lr, float beta1, float beta2, float adam_eps, float max_grad_norm,
                            float *partial_scratch, float *norm_out, void *stream);
+/* pb_peer_allreduce_adam / pb_peer_adam with the update rule as a parameter (rules, h1 / h2 and state arrays as for
+ * pb_opt_clip_apply).  pb_peer_allreduce_opt_max_n(rule) is the fused kernel's limit for that rule. */
+long long pb_peer_allreduce_opt_max_n(int rule);
+int pb_peer_allreduce_opt(int rule, const pb_peer_group *g, long long n, float *param, float *m, float *v,
+                          long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                          float *partial_scratch, float *norm_out, void *stream);
+int pb_peer_opt(int rule, const pb_peer_group *g, long long n, float *param, float *m, float *v,
+                const long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                float *norm_out, float *grad_out, void *stream);
 /* HOST, synchronous, measurement runs only: phase marks of pb_peer_allreduce_adam's kernel (%globaltimer ns: 0 CTA 0
  * starts, 1 handshake done, 2 pulled + summed, 3 the CTAs met, 4 Adam applied; latest CTA each), cleared on read. */
 int pb_peer_trace(int enable, unsigned long long *out, int n_out);

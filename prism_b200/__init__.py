@@ -8,10 +8,10 @@ from . import _lib
 from .config import Config, minatar_ids_iqn_config, minatar_dqn_per_config, atari_iqn_ids_config
 from .experience import (Batch, DevicePrioritizedReplayBuffer, PrioritizedTree, Timestep, TimestepBuffer,
                          TransitionRing, UniformSampler)
-from .agents import Agent, FlatAdam, action_selectors
+from .agents import Agent, FlatAdam, FlatOptimizer, FlatRMSprop, FlatSGD, action_selectors
 from .agents.models import CompositeModel, FFNNModel, IQNModel, MinAtarModel, NatureAtariCnn, QEnsemble
 from .factory import build_agent, build_exp_buffer, create_model
 
 __all__ = ["Config", "minatar_ids_iqn_config", "minatar_dqn_per_config", "atari_iqn_ids_config", "Batch", "DevicePrioritizedReplayBuffer", "PrioritizedTree", "Timestep", "TimestepBuffer",
-           "TransitionRing", "Agent", "FlatAdam", "action_selectors", "CompositeModel", "FFNNModel", "IQNModel",
+           "TransitionRing", "Agent", "FlatAdam", "FlatOptimizer", "FlatRMSprop", "FlatSGD", "action_selectors", "CompositeModel", "FFNNModel", "IQNModel",
            "MinAtarModel", "NatureAtariCnn", "QEnsemble", "UniformSampler", "build_agent", "build_exp_buffer", "create_model"]

@@ -117,6 +117,9 @@ SIGNATURES = {
     "pb_pack_grads_parity": [_I, _P, _F, _P, _P, _LL, _P, _P, _P, _P],
     "pb_grad_sumsq": [_LL, _P, _P, _P, _P, _P],
     "pb_adam_clip_apply": [_LL, _P, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _I, _P, _P],
+    "pb_opt_fused_max_n": [_I],
+    "pb_opt_fused_step": [_I, _I, _P, _F, _LL, _P, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
+    "pb_opt_clip_apply": [_I, _LL, _P, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _I, _P, _P],
     "pb_loss_combine": [_I, _P, _P, _P, _F, _P, _P, _P, _P],
     "pb_conv3x3_relu_supported": [_I, _I, _I, _I],
     "pb_conv3x3_relu_fwd": [_I, _I, _I, _I, _I, _P, _P, _P, _P, _P],
@@ -138,6 +141,9 @@ SIGNATURES = {
     "pb_peer_adam": [_PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
     "pb_peer_allreduce_adam_max_n": [],
     "pb_peer_allreduce_adam": [_PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
+    "pb_peer_allreduce_opt_max_n": [_I],
+    "pb_peer_allreduce_opt": [_I, _PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
+    "pb_peer_opt": [_I, _PEER, _LL, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
     "pb_peer_state_put": [_PEER, _P, _P],
     "pb_peer_trace": [_I, _P, _I],
     "pb_tree_sample_global_peer": [_TREE, _PEER, _LL, _P, _F, _P, _P, _P, _P],
@@ -180,7 +186,11 @@ SIGNATURES = {
     "pb_wire_index_timesteps": [_P, _LL, _LL, _P, _P],
 }
 _RESTYPES = {"pb_error_string": C.c_char_p, "pb_launch_count": C.c_longlong, "pb_peer_slice": C.c_longlong,
-             "pb_peer_allreduce_adam_max_n": C.c_longlong, "pb_adam_fused_max_n": C.c_longlong}
+             "pb_peer_allreduce_adam_max_n": C.c_longlong, "pb_adam_fused_max_n": C.c_longlong,
+             "pb_opt_fused_max_n": C.c_longlong, "pb_peer_allreduce_opt_max_n": C.c_longlong}
+
+# update rules of the pb_opt_* / pb_peer_*_opt entries (include/prism_b200.h)
+PB_OPT_ADAM, PB_OPT_RMSPROP, PB_OPT_RMSPROP_CENTERED, PB_OPT_SGD = 0, 1, 2, 3
 
 PB_E_POOL = -4
 ABI_VERSION = 2

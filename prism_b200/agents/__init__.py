@@ -1,3 +1,3 @@
 from .agent import Agent
 from . import action_selectors
-from .optim import FlatAdam, flatten_parameters
+from .optim import FlatAdam, FlatOptimizer, FlatRMSprop, FlatSGD, flatten_parameters

@@ -1,8 +1,8 @@
 """Agent -- acting forward, the learner update step, target sync, (de)serialisation.
 
 Same constructor and methods as the reference (prism/agents/agent.py:7-264).  The update step is
-    get_losses -> PER-weighted total -> backward -> clip_grad_norm_ -> Adam
-with the loss heads, the loss combine and clip+Adam running as fused libprism_b200 kernels, and
+    get_losses -> PER-weighted total -> backward -> clip_grad_norm_ -> Adam / RMSprop / SGD
+with the loss heads, the loss combine and clip + update running as fused libprism_b200 kernels, and
 the whole step captured in ONE CUDA graph when ``use_cuda_graph`` is set.
 
 Deliberate deviations from the reference (SURVEY appendix Q3):
@@ -20,7 +20,7 @@ import torch
 
 from . import ops
 from .action_selectors import GreedyActionSelector, IDSActionSelector
-from .optim import FlatAdam
+from .optim import FlatOptimizer
 
 
 class Agent(object):
@@ -30,7 +30,7 @@ class Agent(object):
         self.action_selector, self.eval_action_selector = action_selector, eval_action_selector
         self.max_grad_norm, self.use_cuda_graph = max_grad_norm, use_cuda_graph
         self.n_updates, self._is_eval = 0, False
-        if isinstance(optimizer, FlatAdam):
+        if isinstance(optimizer, FlatOptimizer):
             optimizer.max_grad_norm = float(max_grad_norm) if max_grad_norm else 0.0
         # static tensors of the captured update (names as upstream: learner.py and the logger read them)
         for name in ("per_weights", "distribution_loss", "q_loss", "total_loss", "new_per_weights", "batch"):
@@ -146,8 +146,8 @@ class Agent(object):
         return dist_loss, q_loss, total, td
 
     def _optimizer_step(self, refresh_table=True):
-        if isinstance(self.optimizer, FlatAdam):
-            self.optimizer.step(refresh_table=refresh_table)     # clip + Adam fused
+        if isinstance(self.optimizer, FlatOptimizer):
+            self.optimizer.step(refresh_table=refresh_table)     # clip + update fused
         else:
             torch.nn.utils.clip_grad_norm_(self.model.parameters(), self.max_grad_norm)
             self.optimizer.step()
@@ -185,7 +185,7 @@ class Agent(object):
         else:
             self._static_per_weights = torch.full((B,), float(per_weights), dtype=torch.float32, device=dev)
 
-        flat = isinstance(self.optimizer, FlatAdam)
+        flat = isinstance(self.optimizer, FlatOptimizer)
         snap = self.optimizer.snapshot() if flat else None
         # no autograd graph from an earlier (eager, other-stream) update may stay alive across the capture
         self._static_total_loss = self._static_distribution_loss = self._static_q_loss = None

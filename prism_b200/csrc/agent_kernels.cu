@@ -7,6 +7,7 @@
 //   pb_greedy_select   GreedyActionSelector                 prism/agents/action_selectors.py:70-82
 //   pb_loss_combine    PER-weighted total + new priorities  prism/agents/agent.py:58-66, composite_model.py:135-142
 //   pb_adam_clip_step  clip_grad_norm_ + Adam               prism/agents/agent.py:73-74, factory/agent_factory.py:44-47
+//   pb_opt_*           clip_grad_norm_ + Adam / RMSprop / SGD  factory/agent_factory.py:40-58
 //
 // The reference runs each of these as 10-30 tiny ATen kernels (plus their autograd
 // mirrors) with B*T'*T temporaries; here each is one launch, one warp per batch row,
@@ -270,6 +271,9 @@ __global__ void __launch_bounds__(1024) loss_combine_kernel(int B, const float *
 // (fp64 accumulate of fp32 squares is overkill; fp32 per thread, fp64 across), step++.
 // Kernel 2: every CTA re-reduces the <=1024 partials, derives the clip coefficient and
 // applies the update with 128-bit accesses.
+// adam_clip_kernel and adam_fused_kernel are templates on the update rule R (PB_OPT_*, common.cuh: OptRule,
+// opt_update); their names are the Adam family's.  For the RMSprop rules beta1 carries alpha and beta2 is unused; a
+// state slot the rule does not keep is never dereferenced.  R = PB_OPT_ADAM compiles to the code of the Adam-only kernels.
 // ---------------------------------------------------------------------------------
 constexpr int ADAM_THREADS = 256;
 constexpr int ADAM_MAX_PARTIALS = 4096;
@@ -361,6 +365,7 @@ __global__ void __launch_bounds__(ADAM_THREADS) grad_sumsq_kernel(long long n, c
     }
 }
 
+template <int R>
 __global__ void __launch_bounds__(ADAM_THREADS) adam_clip_kernel(long long n, float *__restrict__ param,
                                                                  const float *__restrict__ grad,
                                                                  float *__restrict__ exp_avg,
@@ -378,13 +383,15 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_clip_kernel(long long n, fl
     for (int k = threadIdx.x; k < n_partials; k += blockDim.x) acc += (double)partial[k];
     acc = warp_sum(acc);
     if (lane_id() == 0) red[threadIdx.x >> 5] = acc;
-    if (threadIdx.x == 32) {
-        // bias corrections: two fp64 pow() -- once per CTA (another warp than the one that finishes the norm), not once
-        // per thread
-        const double step = (double)(*step_count);
-        const float bc1 = (float)(1.0 - pow((double)beta1, step));
-        s_bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
-        s_step_size = lr / bc1;
+    if constexpr (R == PB_OPT_ADAM) {
+        if (threadIdx.x == 32) {
+            // bias corrections: two fp64 pow() -- once per CTA (another warp than the one that finishes the norm), not
+            // once per thread
+            const double step = (double)(*step_count);
+            const float bc1 = (float)(1.0 - pow((double)beta1, step));
+            s_bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
+            s_step_size = lr / bc1;
+        }
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -400,28 +407,39 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_clip_kernel(long long n, fl
     }
     __syncthreads();
     const float coef = s_coef;
-    const float bc2_sqrt = s_bc2_sqrt;
-    const float step_size = s_step_size;
+    const float bc2_sqrt = R == PB_OPT_ADAM ? s_bc2_sqrt : 0.0f;
+    const float step_size = R == PB_OPT_ADAM ? s_step_size : 0.0f;
     auto upd = [&](float &p, float g, float &m, float &v) {
         g *= coef;
-        m = m + (g - m) * (1.0f - beta1);                        // exp_avg.lerp_(grad, 1-beta1)
-        v = v * beta2 + (1.0f - beta2) * g * g;                  // mul_(beta2).addcmul_(g, g, 1-beta2)
-        const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
-        p = p - step_size * (m / denom);                         // addcdiv_(exp_avg, denom, -step_size)
+        if constexpr (R == PB_OPT_ADAM) {
+            m = m + (g - m) * (1.0f - beta1);                    // exp_avg.lerp_(grad, 1-beta1)
+            v = v * beta2 + (1.0f - beta2) * g * g;              // mul_(beta2).addcmul_(g, g, 1-beta2)
+            const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
+            p = p - step_size * (m / denom);                     // addcdiv_(exp_avg, denom, -step_size)
+        } else {
+            opt_update<R>(p, g, m, v, lr, beta1, adam_eps);      // beta1 = RMSprop's alpha (common.cuh)
+        }
     };
+    constexpr bool HM = OptRule<R>::has_m, HV = OptRule<R>::has_v;
     const long long n4 = n >> 2;
     float4 *p4 = reinterpret_cast<float4 *>(param);
     const float4 *g4 = reinterpret_cast<const float4 *>(grad);
     float4 *m4 = reinterpret_cast<float4 *>(exp_avg);
     float4 *v4 = reinterpret_cast<float4 *>(exp_avg_sq);
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
-        float4 p = p4[i], g = g4[i], m = m4[i], v = v4[i];
+        float4 p = p4[i], g = g4[i], m, v;
+        if constexpr (HM) m = m4[i];
+        if constexpr (HV) v = v4[i];
         upd(p.x, g.x, m.x, v.x); upd(p.y, g.y, m.y, v.y); upd(p.z, g.z, m.z, v.z); upd(p.w, g.w, m.w, v.w);
-        p4[i] = p; m4[i] = m; v4[i] = v;
+        p4[i] = p;
+        if constexpr (HM) m4[i] = m;
+        if constexpr (HV) v4[i] = v;
     }
     if (blockIdx.x == 0)
-        for (long long i = (n4 << 2) + threadIdx.x; i < n; i += blockDim.x)
-            upd(param[i], grad[i], exp_avg[i], exp_avg_sq[i]);
+        for (long long i = (n4 << 2) + threadIdx.x; i < n; i += blockDim.x) {
+            float unused = 0.0f;
+            upd(param[i], grad[i], HM ? exp_avg[i] : unused, HV ? exp_avg_sq[i] : unused);
+        }
 }
 
 
@@ -437,6 +455,7 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_clip_kernel(long long n, fl
 constexpr int FUSED_U = 8;
 constexpr int FUSED_MAX_TENSORS = 64;
 
+template <int R>
 __global__ void __launch_bounds__(ADAM_THREADS) adam_fused_kernel(const long long *__restrict__ table, int n_tensors,
                                                                   float scale, long long n, float *__restrict__ param,
                                                                   float *__restrict__ grad, float *__restrict__ exp_avg,
@@ -457,12 +476,20 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_fused_kernel(const long lon
     const long long stride = (long long)gridDim.x * blockDim.x, i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     float4 *p4 = reinterpret_cast<float4 *>(param), *m4 = reinterpret_cast<float4 *>(exp_avg),
            *v4 = reinterpret_cast<float4 *>(exp_avg_sq), *g4 = reinterpret_cast<float4 *>(grad);
+    constexpr bool HM = OptRule<R>::has_m, HV = OptRule<R>::has_v;
     float4 p0 = make_float4(0.f, 0.f, 0.f, 0.f), m0 = p0, v0 = p0;
-    if (i0 < n4) { p0 = p4[i0]; m0 = m4[i0]; v0 = v4[i0]; }
-    const double step = (double)step_now;
-    const float bc1 = (float)(1.0 - pow((double)beta1, step));
-    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
-    const float step_size = lr / bc1;
+    if (i0 < n4) {
+        p0 = p4[i0];
+        if constexpr (HM) m0 = m4[i0];
+        if constexpr (HV) v0 = v4[i0];
+    }
+    float bc2_sqrt = 0.0f, step_size = 0.0f;
+    if constexpr (R == PB_OPT_ADAM) {
+        const double step = (double)step_now;
+        const float bc1 = (float)(1.0 - pow((double)beta1, step));
+        bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
+        step_size = lr / bc1;
+    }
     __syncthreads();
     // ---- gather: arena offset -> (tensor, offset within it); tensors are laid out in table order, 16-byte aligned
     float4 gsum[FUSED_U];
@@ -529,20 +556,30 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_fused_kernel(const long lon
     const float coef = s_coef;
     auto upd = [&](float &p, float gg, float &m, float &v) {          // same arithmetic as adam_clip_kernel
         gg *= coef;
-        m = m + (gg - m) * (1.0f - beta1);
-        v = v * beta2 + (1.0f - beta2) * gg * gg;
-        const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
-        p = p - step_size * (m / denom);
+        if constexpr (R == PB_OPT_ADAM) {
+            m = m + (gg - m) * (1.0f - beta1);
+            v = v * beta2 + (1.0f - beta2) * gg * gg;
+            const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
+            p = p - step_size * (m / denom);
+        } else {
+            opt_update<R>(p, gg, m, v, lr, beta1, adam_eps);
+        }
     };
 #pragma unroll
     for (int k = 0; k < FUSED_U; ++k) {
         const long long i = i0 + k * stride;
         if (i < n4) {
             float4 p = p0, m = m0, v = v0;
-            if (k > 0) { p = p4[i]; m = m4[i]; v = v4[i]; }
+            if (k > 0) {
+                p = p4[i];
+                if constexpr (HM) m = m4[i];
+                if constexpr (HV) v = v4[i];
+            }
             const float4 gr = gsum[k];
             upd(p.x, gr.x, m.x, v.x); upd(p.y, gr.y, m.y, v.y); upd(p.z, gr.z, m.z, v.z); upd(p.w, gr.w, m.w, v.w);
-            p4[i] = p; m4[i] = m; v4[i] = v;
+            p4[i] = p;
+            if constexpr (HM) m4[i] = m;
+            if constexpr (HV) v4[i] = v;
         }
     }
     __syncthreads();
@@ -557,19 +594,43 @@ __global__ void __launch_bounds__(ADAM_THREADS) adam_fused_kernel(const long lon
     }
 }
 
-static int fused_max_blocks()
+// rule -> kernel instantiation (nullptr: unknown rule)
+static decltype(&adam_fused_kernel<PB_OPT_ADAM>) fused_kernel(int rule)
 {
-    static std::atomic<int> cached[64];
+    switch (rule) {
+    case PB_OPT_ADAM: return adam_fused_kernel<PB_OPT_ADAM>;
+    case PB_OPT_RMSPROP: return adam_fused_kernel<PB_OPT_RMSPROP>;
+    case PB_OPT_RMSPROP_CENTERED: return adam_fused_kernel<PB_OPT_RMSPROP_CENTERED>;
+    case PB_OPT_SGD: return adam_fused_kernel<PB_OPT_SGD>;
+    }
+    return nullptr;
+}
+
+static decltype(&adam_clip_kernel<PB_OPT_ADAM>) clip_kernel(int rule)
+{
+    switch (rule) {
+    case PB_OPT_ADAM: return adam_clip_kernel<PB_OPT_ADAM>;
+    case PB_OPT_RMSPROP: return adam_clip_kernel<PB_OPT_RMSPROP>;
+    case PB_OPT_RMSPROP_CENTERED: return adam_clip_kernel<PB_OPT_RMSPROP_CENTERED>;
+    case PB_OPT_SGD: return adam_clip_kernel<PB_OPT_SGD>;
+    }
+    return nullptr;
+}
+
+// CTAs of the rule's fused kernel that are resident at once (its grid never exceeds this: the CTAs meet at a counter)
+static int fused_max_blocks(int rule)
+{
+    static std::atomic<int> cached[4][64];
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-    int c = cached[dev].load(std::memory_order_relaxed);
+    int c = cached[rule][dev].load(std::memory_order_relaxed);
     if (c > 0) return c;
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, adam_fused_kernel, ADAM_THREADS, 0) != cudaSuccess || per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fused_kernel(rule), ADAM_THREADS, 0) != cudaSuccess || per_sm < 1)
         per_sm = 1;
     if (per_sm > 4) per_sm = 4;
     c = pb_sm_count() * per_sm;
-    cached[dev].store(c, std::memory_order_relaxed);
+    cached[rule][dev].store(c, std::memory_order_relaxed);
     return c;
 }
 
@@ -710,53 +771,78 @@ int pb_grad_sumsq(long long n, const float *grad, float *partial_scratch, long l
     return PB_OK;
 }
 
+int pb_opt_clip_apply(int rule, long long n, float *param, const float *grad, float *m, float *v,
+                      const long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                      const float *partial_scratch, int n_partials, float *norm_out, void *stream)
+{
+    if (pb_opt_check(rule, m, v)) return PB_E_ARG;
+    if (n <= 0 || !param || !grad || !step_count || !partial_scratch) return PB_E_ARG;
+    if (n_partials <= 0 || n_partials > ADAM_MAX_PARTIALS) return PB_E_ARG;
+    if ((((uintptr_t)param) | ((uintptr_t)grad) | ((uintptr_t)m) | ((uintptr_t)v)) & 15) return PB_E_ARG;
+    long long nb = ((n >> 2) + ADAM_THREADS - 1) / ADAM_THREADS;
+    if (nb < 1) nb = 1;
+    const long long cap = (long long)pb_sm_count() * 4;
+    if (nb > cap) nb = cap;
+    PB_LAUNCH_PDL_CHAIN(clip_kernel(rule), (unsigned)nb, ADAM_THREADS, 0, stream, n, param, grad, m, v, step_count,
+              lr, h1, h2, eps, max_grad_norm, partial_scratch, n_partials, norm_out);
+    return PB_OK;
+}
+
 int pb_adam_clip_apply(long long n, float *param, const float *grad, float *exp_avg, float *exp_avg_sq,
                        const long long *step_count, float lr, float beta1, float beta2, float adam_eps,
                        float max_grad_norm, const float *partial_scratch, int n_partials, float *norm_out,
                        void *stream)
 {
-    if (n <= 0 || !param || !grad || !exp_avg || !exp_avg_sq || !step_count || !partial_scratch) return PB_E_ARG;
-    if (n_partials <= 0 || n_partials > ADAM_MAX_PARTIALS) return PB_E_ARG;
-    if ((((uintptr_t)param) | ((uintptr_t)grad) | ((uintptr_t)exp_avg) | ((uintptr_t)exp_avg_sq)) & 15) return PB_E_ARG;
-    long long nb = ((n >> 2) + ADAM_THREADS - 1) / ADAM_THREADS;
-    if (nb < 1) nb = 1;
-    const long long cap = (long long)pb_sm_count() * 4;
-    if (nb > cap) nb = cap;
-    PB_LAUNCH_PDL_CHAIN(adam_clip_kernel, (unsigned)nb, ADAM_THREADS, 0, stream, n, param, grad, exp_avg, exp_avg_sq, step_count,
-              lr, beta1, beta2, adam_eps, max_grad_norm, partial_scratch, n_partials, norm_out);
-    return PB_OK;
+    return pb_opt_clip_apply(PB_OPT_ADAM, n, param, grad, exp_avg, exp_avg_sq, step_count, lr, beta1, beta2, adam_eps,
+                             max_grad_norm, partial_scratch, n_partials, norm_out, stream);
 }
 
 // load the optimizer kernels now (see pb_peer_preload)
 int pb_optimizer_preload(void)
 {
     cudaFuncAttributes a;
-    cudaError_t e = cudaFuncGetAttributes(&a, adam_clip_kernel);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, pack_grads_kernel);
+    cudaError_t e = cudaFuncGetAttributes(&a, pack_grads_kernel);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, grad_sumsq_kernel);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, adam_fused_kernel);
+    for (int rule = PB_OPT_ADAM; rule <= PB_OPT_SGD && e == cudaSuccess; ++rule) {
+        e = cudaFuncGetAttributes(&a, clip_kernel(rule));
+        if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, fused_kernel(rule));
+    }
     return e == cudaSuccess ? PB_OK : (int)e;
 }
 
-long long pb_adam_fused_max_n(void) { return (long long)fused_max_blocks() * ADAM_THREADS * FUSED_U * 4; }
+long long pb_opt_fused_max_n(int rule)
+{
+    if (!pb_opt_known(rule)) return 0;
+    return (long long)fused_max_blocks(rule) * ADAM_THREADS * FUSED_U * 4;
+}
+
+long long pb_adam_fused_max_n(void) { return pb_opt_fused_max_n(PB_OPT_ADAM); }
+
+int pb_opt_fused_step(int rule, int n_tensors, const long long *table, float scale, long long n, float *param, float *grad,
+                      float *m, float *v, long long *step_count, float lr, float h1, float h2, float eps,
+                      float max_grad_norm, float *partial_scratch, float *norm_out, void *stream)
+{
+    if (pb_opt_check(rule, m, v)) return PB_E_ARG;
+    if (n_tensors <= 0 || !table || n <= 0 || (n % 4) != 0 || !param || !grad || !step_count || !partial_scratch)
+        return PB_E_ARG;
+    if (n_tensors > FUSED_MAX_TENSORS || n > pb_opt_fused_max_n(rule)) return PB_E_UNSUPPORTED;
+    if ((((uintptr_t)param) | ((uintptr_t)grad) | ((uintptr_t)m) | ((uintptr_t)v)) & 15) return PB_E_ARG;
+    long long nb = ((n >> 2) + ADAM_THREADS - 1) / ADAM_THREADS;
+    const long long cap = fused_max_blocks(rule);
+    if (nb > cap) nb = cap;
+    if (nb < 1) nb = 1;
+    unsigned int *counters = reinterpret_cast<unsigned int *>(partial_scratch + 4092);    // zero between calls
+    PB_LAUNCH(fused_kernel(rule), (unsigned)nb, ADAM_THREADS, 0, stream, table, n_tensors, scale, n, param, grad, m, v,
+              step_count, lr, h1, h2, eps, max_grad_norm, partial_scratch, counters, norm_out);
+    return PB_OK;
+}
 
 int pb_adam_fused_step(int n_tensors, const long long *table, float scale, long long n, float *param, float *grad,
                        float *exp_avg, float *exp_avg_sq, long long *step_count, float lr, float beta1, float beta2,
                        float adam_eps, float max_grad_norm, float *partial_scratch, float *norm_out, void *stream)
 {
-    if (n_tensors <= 0 || !table || n <= 0 || (n % 4) != 0 || !param || !grad || !exp_avg || !exp_avg_sq || !step_count ||
-        !partial_scratch)
-        return PB_E_ARG;
-    if (n_tensors > FUSED_MAX_TENSORS || n > pb_adam_fused_max_n()) return PB_E_UNSUPPORTED;
-    if ((((uintptr_t)param) | ((uintptr_t)grad) | ((uintptr_t)exp_avg) | ((uintptr_t)exp_avg_sq)) & 15) return PB_E_ARG;
-    long long nb = ((n >> 2) + ADAM_THREADS - 1) / ADAM_THREADS;
-    const long long cap = fused_max_blocks();
-    if (nb > cap) nb = cap;
-    if (nb < 1) nb = 1;
-    unsigned int *counters = reinterpret_cast<unsigned int *>(partial_scratch + 4092);    // zero between calls
-    PB_LAUNCH(adam_fused_kernel, (unsigned)nb, ADAM_THREADS, 0, stream, table, n_tensors, scale, n, param, grad, exp_avg,
-              exp_avg_sq, step_count, lr, beta1, beta2, adam_eps, max_grad_norm, partial_scratch, counters, norm_out);
-    return PB_OK;
+    return pb_opt_fused_step(PB_OPT_ADAM, n_tensors, table, scale, n, param, grad, exp_avg, exp_avg_sq, step_count, lr,
+                             beta1, beta2, adam_eps, max_grad_norm, partial_scratch, norm_out, stream);
 }
 
 int pb_adam_clip_step(long long n, float *param, const float *grad, float *exp_avg, float *exp_avg_sq,

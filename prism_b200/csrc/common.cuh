@@ -46,6 +46,16 @@ bool pb_pdl_chain_enabled();
 #define PB_LAUNCH_PDL_CHAIN(kernel, grid, block, smem, stream, ...)                         \
     PB_LAUNCH_PDL_IF(pb_pdl_chain_enabled(), kernel, grid, block, smem, stream, __VA_ARGS__)
 
+// argument check of the rule-parameterised optimizer entries: PB_E_ARG for an unknown rule or a NULL state array that
+// the rule reads (m: Adam, centered RMSprop; v: every rule but SGD)
+static inline bool pb_opt_known(int rule) { return rule >= PB_OPT_ADAM && rule <= PB_OPT_SGD; }
+static inline int pb_opt_check(int rule, const void *m, const void *v)
+{
+    if (!pb_opt_known(rule)) return PB_E_ARG;
+    const bool has_m = rule == PB_OPT_ADAM || rule == PB_OPT_RMSPROP_CENTERED, has_v = rule != PB_OPT_SGD;
+    return ((has_m && !m) || (has_v && !v)) ? PB_E_ARG : PB_OK;
+}
+
 static inline int pb_ilog2(long long v) { int l = 0; while ((1LL << l) < v) ++l; return l; }
 static inline bool pb_is_pow2(long long v) { return v > 0 && (v & (v - 1)) == 0; }
 
@@ -195,6 +205,48 @@ __device__ __forceinline__ const pb_per_state *peer_wait_states(const PeerWait &
     }
     __syncthreads();
     return reinterpret_cast<const pb_per_state *>(pw.slots + (size_t)(2 + (e & 1)) * pw.slot_bytes);
+}
+
+// ---------------------------------------------------------------------------------
+// Update rules of the flat optimizers (PB_OPT_*), one instantiation of every clip + update kernel family per rule
+// (agent_kernels.cu, peer.cu).  State slots: m = Adam's exp_avg / centered RMSprop's grad_avg, v = Adam's exp_avg_sq /
+// RMSprop's square_avg; plain RMSprop keeps v only, SGD neither (its state pointers may be null).  Adam's arithmetic is
+// written out in each kernel; opt_update is every other rule, per element after clip_grad_norm_'s g *= coef, in the
+// order of torch's foreach implementation (torch/optim/rmsprop.py _multi_tensor_rmsprop, torch/optim/sgd.py
+// _multi_tensor_sgd).  Each foreach op is one rounding; inside one, ATen's functors compute a + s * op(b, c), which
+// the compiler contracts to fma(s, op(b, c), a):
+//   square_avg.mul_(alpha)                      v = v * alpha
+//   square_avg.addcmul_(g, g, 1 - alpha)        v = fma(1 - alpha, g * g, v)
+//   grad_avg.lerp_(g, w = 1 - alpha)            m = |w| < 0.5 ? fma(w, g - m, m) : fma(-(g - m), 1 - w, g)
+//                                                   (ATen's two-branch lerp, ATen/native/Lerp.h)
+//   avg = addcmul(square_avg, grad_avg, grad_avg, -1).sqrt_().add_(eps)     centered: sqrt(v - m * m) + eps
+//   avg = square_avg.sqrt().add_(eps)                                       not centered: sqrt(v) + eps
+//   param.addcdiv_(g, avg, -lr)                 p = fma(-lr, g / avg, p)
+//   SGD: param.add_(g, alpha=-lr)               p = fma(-lr, g, p)
+// ---------------------------------------------------------------------------------
+template <int R> struct OptRule {
+    static_assert(R == PB_OPT_ADAM || R == PB_OPT_RMSPROP || R == PB_OPT_RMSPROP_CENTERED || R == PB_OPT_SGD, "rule");
+    static constexpr bool has_m = R == PB_OPT_ADAM || R == PB_OPT_RMSPROP_CENTERED;   // reads / writes the m slot
+    static constexpr bool has_v = R != PB_OPT_SGD;                                     // reads / writes the v slot
+};
+
+template <int R>
+__device__ __forceinline__ void opt_update(float &p, float g, float &m, float &v, float lr, float alpha, float eps)
+{
+    if constexpr (R == PB_OPT_SGD) {
+        p = __fmaf_rn(-lr, g, p);
+    } else {
+        v = __fmaf_rn(1.0f - alpha, __fmul_rn(g, g), __fmul_rn(v, alpha));
+        float avg;
+        if constexpr (R == PB_OPT_RMSPROP_CENTERED) {
+            const float w = 1.0f - alpha, d = __fsub_rn(g, m);
+            m = fabsf(w) < 0.5f ? __fmaf_rn(w, d, m) : __fmaf_rn(-d, __fsub_rn(1.0f, w), g);
+            avg = __fadd_rn(__fsqrt_rn(__fsub_rn(v, __fmul_rn(m, m))), eps);
+        } else {
+            avg = __fadd_rn(__fsqrt_rn(v), eps);
+        }
+        p = __fmaf_rn(-lr, __fdiv_rn(g, avg), p);
+    }
 }
 
 }  // namespace pb

@@ -15,6 +15,8 @@
 //     (the all-gather half of the all-reduce is fused into the optimizer kernel), derives the global norm from the
 //     published partial sums in rank order (bit-identical on every rank) and updates the local parameter replica.
 // pb_peer_barrier is a 1-block epoch barrier (flags in peer memory, monotonically increasing: graph-replay safe).
+// peer_adam_kernel and peer_allreduce_adam_kernel are templates on the update rule (PB_OPT_*, common.cuh), as the
+// single-GPU optimizer kernels of agent_kernels.cu are: Adam, RMSprop (beta1 carries alpha) or SGD after the same clip.
 #include "common.cuh"
 
 namespace {
@@ -207,6 +209,7 @@ __global__ void __launch_bounds__(RS_THREADS) peer_pull_sum_kernel(pb_peer_group
     }
 }
 
+template <int R>
 __global__ void __launch_bounds__(256) peer_adam_kernel(pb_peer_group g, long long n, long long slice,
                                                         float *__restrict__ param, float *__restrict__ exp_avg,
                                                         float *__restrict__ exp_avg_sq,
@@ -221,17 +224,25 @@ __global__ void __launch_bounds__(256) peer_adam_kernel(pb_peer_group g, long lo
     coef = coef > 1.0f ? 1.0f : coef;
     if (!(max_grad_norm > 0.0f)) coef = 1.0f;
     if (blockIdx.x == 0 && threadIdx.x == 0 && norm_out) { norm_out[0] = total_norm; norm_out[1] = coef; }
-    const double step = (double)(*step_count);
-    const float bc1 = (float)(1.0 - pow((double)beta1, step));
-    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
-    const float step_size = lr / bc1;
+    float bc2_sqrt = 0.0f, step_size = 0.0f;
+    if constexpr (R == PB_OPT_ADAM) {
+        const double step = (double)(*step_count);
+        const float bc1 = (float)(1.0 - pow((double)beta1, step));
+        bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
+        step_size = lr / bc1;
+    }
     auto upd = [&](float &p, float gg, float &m, float &v) {                                 // same arithmetic as adam_clip_kernel
         gg *= coef;
-        m = m + (gg - m) * (1.0f - beta1);
-        v = v * beta2 + (1.0f - beta2) * gg * gg;
-        const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
-        p = p - step_size * (m / denom);
+        if constexpr (R == PB_OPT_ADAM) {
+            m = m + (gg - m) * (1.0f - beta1);
+            v = v * beta2 + (1.0f - beta2) * gg * gg;
+            const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
+            p = p - step_size * (m / denom);
+        } else {
+            opt_update<R>(p, gg, m, v, lr, beta1, adam_eps);
+        }
     };
+    constexpr bool HM = OptRule<R>::has_m, HV = OptRule<R>::has_v;
     const long long n4 = n >> 2;
     float4 *p4 = reinterpret_cast<float4 *>(param), *m4 = reinterpret_cast<float4 *>(exp_avg),
            *v4 = reinterpret_cast<float4 *>(exp_avg_sq);
@@ -239,9 +250,13 @@ __global__ void __launch_bounds__(256) peer_adam_kernel(pb_peer_group g, long lo
         const long long e = i << 2;
         const int owner = (int)(e / slice);
         const float4 gr = ld_peer_f4(g.reduced[owner] + e);                                   // all-gather fused into the sweep
-        float4 p = p4[i], m = m4[i], v = v4[i];
+        float4 p = p4[i], m, v;
+        if constexpr (HM) m = m4[i];
+        if constexpr (HV) v = v4[i];
         upd(p.x, gr.x, m.x, v.x); upd(p.y, gr.y, m.y, v.y); upd(p.z, gr.z, m.z, v.z); upd(p.w, gr.w, m.w, v.w);
-        p4[i] = p; m4[i] = m; v4[i] = v;
+        p4[i] = p;
+        if constexpr (HM) m4[i] = m;
+        if constexpr (HV) v4[i] = v;
         if (grad_out) *reinterpret_cast<float4 *>(grad_out + e) = gr;
     }
 }
@@ -266,6 +281,7 @@ __device__ __forceinline__ unsigned ld_acquire_gpu_u32(const unsigned *p)
     return v;
 }
 
+template <int R>
 __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer_group g, long long n,
                                                                          float *__restrict__ param,
                                                                          float *__restrict__ exp_avg,
@@ -290,12 +306,20 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
     const long long stride = (long long)gridDim.x * blockDim.x, i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     float4 *p4 = reinterpret_cast<float4 *>(param), *m4 = reinterpret_cast<float4 *>(exp_avg),
            *v4 = reinterpret_cast<float4 *>(exp_avg_sq), *r4 = reinterpret_cast<float4 *>(g.reduced[g.rank]);
+    constexpr bool HM = OptRule<R>::has_m, HV = OptRule<R>::has_v;
     float4 p0 = make_float4(0.f, 0.f, 0.f, 0.f), m0 = p0, v0 = p0;
-    if (i0 < n4) { p0 = p4[i0]; m0 = m4[i0]; v0 = v4[i0]; }
-    const double step = (double)step_now;
-    const float bc1 = (float)(1.0 - pow((double)beta1, step));
-    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
-    const float step_size = lr / bc1;
+    if (i0 < n4) {
+        p0 = p4[i0];
+        if constexpr (HM) m0 = m4[i0];
+        if constexpr (HV) v0 = v4[i0];
+    }
+    float bc2_sqrt = 0.0f, step_size = 0.0f;
+    if constexpr (R == PB_OPT_ADAM) {
+        const double step = (double)step_now;
+        const float bc1 = (float)(1.0 - pow((double)beta1, step));
+        bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, step));
+        step_size = lr / bc1;
+    }
     // (launched as a programmatic dependent of the pack kernel: everything above overlaps its tail)
     pdl_wait();
     // ---- handshake: CTA 0 tells every rank "my gradient is packed"; every CTA waits for all ranks on the local pad
@@ -367,20 +391,30 @@ __global__ void __launch_bounds__(FA_THREADS) peer_allreduce_adam_kernel(pb_peer
     const float coef = s_coef;
     auto upd = [&](float &p, float gg, float &m, float &v) {          // same arithmetic as adam_clip_kernel
         gg *= coef;
-        m = m + (gg - m) * (1.0f - beta1);
-        v = v * beta2 + (1.0f - beta2) * gg * gg;
-        const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
-        p = p - step_size * (m / denom);
+        if constexpr (R == PB_OPT_ADAM) {
+            m = m + (gg - m) * (1.0f - beta1);
+            v = v * beta2 + (1.0f - beta2) * gg * gg;
+            const float denom = sqrtf(v) / bc2_sqrt + adam_eps;
+            p = p - step_size * (m / denom);
+        } else {
+            opt_update<R>(p, gg, m, v, lr, beta1, adam_eps);
+        }
     };
 #pragma unroll
     for (int k = 0; k < FA_U; ++k) {
         const long long i = i0 + k * stride;
         if (i < n4) {
             float4 p = p0, m = m0, v = v0;
-            if (k > 0) { p = p4[i]; m = m4[i]; v = v4[i]; }
+            if (k > 0) {
+                p = p4[i];
+                if constexpr (HM) m = m4[i];
+                if constexpr (HV) v = v4[i];
+            }
             const float4 gr = sum[k];
             upd(p.x, gr.x, m.x, v.x); upd(p.y, gr.y, m.y, v.y); upd(p.z, gr.z, m.z, v.z); upd(p.w, gr.w, m.w, v.w);
-            p4[i] = p; m4[i] = m; v4[i] = v;
+            p4[i] = p;
+            if constexpr (HM) m4[i] = m;
+            if constexpr (HV) v4[i] = v;
             r4[i] = gr;                                               // the summed gradient (diagnostics, tests)
         }
     }
@@ -419,6 +453,29 @@ __global__ void __launch_bounds__(32) peer_state_put_kernel(pb_peer_group g, con
     if (lane == 0) g.epoch[2] = e;
 }
 
+// rule -> kernel instantiation (nullptr: unknown rule)
+static decltype(&peer_allreduce_adam_kernel<PB_OPT_ADAM>) allreduce_kernel(int rule)
+{
+    switch (rule) {
+    case PB_OPT_ADAM: return peer_allreduce_adam_kernel<PB_OPT_ADAM>;
+    case PB_OPT_RMSPROP: return peer_allreduce_adam_kernel<PB_OPT_RMSPROP>;
+    case PB_OPT_RMSPROP_CENTERED: return peer_allreduce_adam_kernel<PB_OPT_RMSPROP_CENTERED>;
+    case PB_OPT_SGD: return peer_allreduce_adam_kernel<PB_OPT_SGD>;
+    }
+    return nullptr;
+}
+
+static decltype(&peer_adam_kernel<PB_OPT_ADAM>) sweep_kernel(int rule)
+{
+    switch (rule) {
+    case PB_OPT_ADAM: return peer_adam_kernel<PB_OPT_ADAM>;
+    case PB_OPT_RMSPROP: return peer_adam_kernel<PB_OPT_RMSPROP>;
+    case PB_OPT_RMSPROP_CENTERED: return peer_adam_kernel<PB_OPT_RMSPROP_CENTERED>;
+    case PB_OPT_SGD: return peer_adam_kernel<PB_OPT_SGD>;
+    }
+    return nullptr;
+}
+
 int check_group(const pb_peer_group *g)
 {
     if (!g || g->world < 1 || g->world > PB_PEER_MAX || g->rank < 0 || g->rank >= g->world || !g->epoch) return PB_E_ARG;
@@ -452,10 +509,12 @@ int pb_peer_preload(void)
     cudaError_t e = cudaFuncGetAttributes(&a, peer_barrier_kernel);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_state_allgather_kernel);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_reduce_scatter_kernel);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_adam_kernel);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_pull_sum_kernel);
-    if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_allreduce_adam_kernel);
     if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, peer_state_put_kernel);
+    for (int rule = PB_OPT_ADAM; rule <= PB_OPT_SGD && e == cudaSuccess; ++rule) {
+        e = cudaFuncGetAttributes(&a, sweep_kernel(rule));
+        if (e == cudaSuccess) e = cudaFuncGetAttributes(&a, allreduce_kernel(rule));
+    }
     return e == cudaSuccess ? PB_OK : (int)e;
 }
 
@@ -539,45 +598,60 @@ int pb_peer_pull_sum(const pb_peer_group *g, long long n, float *partial_scratch
     return PB_OK;
 }
 
-// CTAs of the fused kernel that are resident at once (its grid never exceeds this: the CTAs meet at a counter)
-static int fa_max_blocks()
+// CTAs of the rule's fused kernel that are resident at once (its grid never exceeds this: the CTAs meet at a counter)
+static int fa_max_blocks(int rule)
 {
-    static std::atomic<int> cached[64];
+    static std::atomic<int> cached[4][64];
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-    int c = cached[dev].load(std::memory_order_relaxed);
+    int c = cached[rule][dev].load(std::memory_order_relaxed);
     if (c > 0) return c;
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, peer_allreduce_adam_kernel, FA_THREADS, 0) != cudaSuccess || per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, allreduce_kernel(rule), FA_THREADS, 0) != cudaSuccess || per_sm < 1)
         per_sm = 1;
     if (per_sm > 4) per_sm = 4;
     c = pb_sm_count() * per_sm;
-    cached[dev].store(c, std::memory_order_relaxed);
+    cached[rule][dev].store(c, std::memory_order_relaxed);
     return c;
 }
 
-long long pb_peer_allreduce_adam_max_n(void) { return (long long)fa_max_blocks() * FA_THREADS * FA_U * 4; }
+long long pb_peer_allreduce_opt_max_n(int rule)
+{
+    if (!pb_opt_known(rule)) return 0;
+    return (long long)fa_max_blocks(rule) * FA_THREADS * FA_U * 4;
+}
+
+long long pb_peer_allreduce_adam_max_n(void) { return pb_peer_allreduce_opt_max_n(PB_OPT_ADAM); }
 
 int pb_peer_allreduce_adam(const pb_peer_group *g, long long n, float *param, float *exp_avg, float *exp_avg_sq,
                            long long *step_count, float lr, float beta1, float beta2, float adam_eps, float max_grad_norm,
                            float *partial_scratch, float *norm_out, void *stream)
 {
+    return pb_peer_allreduce_opt(PB_OPT_ADAM, g, n, param, exp_avg, exp_avg_sq, step_count, lr, beta1, beta2, adam_eps,
+                                 max_grad_norm, partial_scratch, norm_out, stream);
+}
+
+int pb_peer_allreduce_opt(int rule, const pb_peer_group *g, long long n, float *param, float *m, float *v,
+                          long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                          float *partial_scratch, float *norm_out, void *stream)
+{
+    if (pb_opt_check(rule, m, v)) return PB_E_ARG;
     int rc = check_group(g);
     if (rc) return rc;
-    if (n <= 0 || (n % 4) != 0 || n > pb_peer_allreduce_adam_max_n()) return PB_E_ARG;
-    if (!param || !exp_avg || !exp_avg_sq || !step_count || !partial_scratch) return PB_E_ARG;
-    if ((((uintptr_t)param) | ((uintptr_t)exp_avg) | ((uintptr_t)exp_avg_sq)) & 15) return PB_E_ARG;
+    if (n <= 0 || (n % 4) != 0 || n > pb_peer_allreduce_opt_max_n(rule)) return PB_E_ARG;
+    if (!param || !step_count || !partial_scratch) return PB_E_ARG;
+    if ((((uintptr_t)param) | ((uintptr_t)m) | ((uintptr_t)v)) & 15) return PB_E_ARG;
     for (int p = 0; p < g->world; ++p)
         if (!g->grad[p]) return PB_E_ARG;
     if (!g->reduced[g->rank]) return PB_E_ARG;
     // one 128-bit element per thread while that fits the resident grid, then up to FA_U
     long long nb = ((n >> 2) + FA_THREADS - 1) / FA_THREADS;
-    const long long cap = fa_max_blocks();
+    const long long cap = fa_max_blocks(rule);
     if (nb > cap) nb = cap;
     if (nb < 1) nb = 1;
     unsigned int *counters = reinterpret_cast<unsigned int *>(partial_scratch + 4092);    // zero between calls
-    PB_LAUNCH_PDL(peer_allreduce_adam_kernel, (unsigned)nb, FA_THREADS, 0, stream, *g, n, param, exp_avg, exp_avg_sq, step_count,
-              lr, beta1, beta2, adam_eps, max_grad_norm, partial_scratch, counters, norm_out);
+    PB_LAUNCH_PDL(allreduce_kernel(rule), (unsigned)nb, FA_THREADS, 0, stream, *g, n, param, m, v, step_count, lr, h1, h2,
+                  eps, max_grad_norm, partial_scratch, counters, norm_out);
     return PB_OK;
 }
 
@@ -613,16 +687,25 @@ int pb_peer_adam(const pb_peer_group *g, long long n, float *param, float *exp_a
                  const long long *step_count, float lr, float beta1, float beta2, float adam_eps, float max_grad_norm,
                  float *norm_out, float *grad_out, void *stream)
 {
+    return pb_peer_opt(PB_OPT_ADAM, g, n, param, exp_avg, exp_avg_sq, step_count, lr, beta1, beta2, adam_eps, max_grad_norm,
+                       norm_out, grad_out, stream);
+}
+
+int pb_peer_opt(int rule, const pb_peer_group *g, long long n, float *param, float *m, float *v,
+                const long long *step_count, float lr, float h1, float h2, float eps, float max_grad_norm,
+                float *norm_out, float *grad_out, void *stream)
+{
+    if (pb_opt_check(rule, m, v)) return PB_E_ARG;
     int rc = check_group(g);
     if (rc) return rc;
-    if (n <= 0 || (n % 4) != 0 || !param || !exp_avg || !exp_avg_sq || !step_count) return PB_E_ARG;
-    if ((((uintptr_t)param) | ((uintptr_t)exp_avg) | ((uintptr_t)exp_avg_sq) | ((uintptr_t)grad_out)) & 15) return PB_E_ARG;
+    if (n <= 0 || (n % 4) != 0 || !param || !step_count) return PB_E_ARG;
+    if ((((uintptr_t)param) | ((uintptr_t)m) | ((uintptr_t)v) | ((uintptr_t)grad_out)) & 15) return PB_E_ARG;
     const long long slice = pb_peer_slice(n, g->world);
     long long nb = ((n >> 2) + 255) / 256;
     const long long cap = (long long)pb_sm_count() * 4;
     if (nb > cap) nb = cap;
-    PB_LAUNCH(peer_adam_kernel, (unsigned)nb, 256, 0, stream, *g, n, slice, param, exp_avg, exp_avg_sq, step_count, lr, beta1,
-              beta2, adam_eps, max_grad_norm, norm_out, grad_out);
+    PB_LAUNCH(sweep_kernel(rule), (unsigned)nb, 256, 0, stream, *g, n, slice, param, m, v, step_count, lr, h1, h2, eps,
+              max_grad_norm, norm_out, grad_out);
     return PB_OK;
 }
 

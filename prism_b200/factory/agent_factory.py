@@ -1,13 +1,12 @@
 """build_agent(config, obs_shape, n_actions) -> Agent: the seam of prism/factory/agent_factory.py:7-61.
 
 Same decisions from the same config fields (target network, IDS / e-greedy / greedy acting policy, Adam / RMSprop / SGD);
-what differs is what gets built: Adam becomes ``FlatAdam`` (clip + Adam fused over one flat arena), and the online and
-target parameters are laid out in identical arenas so the target sync is a single copy.
+what differs is what gets built: on CUDA the optimizer is a flat one (``FlatAdam`` / ``FlatRMSprop`` / ``FlatSGD``: clip +
+update fused over one flat arena), and the online and target parameters are laid out in identical arenas so the target
+sync is a single copy.
 """
-import torch
-
 from ..agents import Agent, action_selectors
-from ..agents.optim import FlatAdam, flatten_parameters
+from ..agents.optim import FlatAdam, FlatOptimizer, FlatRMSprop, FlatSGD, flatten_parameters
 from . import model_factory
 
 
@@ -22,16 +21,16 @@ def _acting_policy(cfg):
     return action_selectors.GreedyActionSelector()
 
 
-def _optimizer(cfg, model, arena, graphed):
+def _optimizer(cfg, model, arena):
     """agent_factory.py:40-58."""
     params = model.parameters()
     if cfg.use_adam:
         return FlatAdam(params, lr=cfg.learning_rate, betas=(cfg.adam_beta1, cfg.adam_beta2), eps=cfg.adam_epsilon,
                         max_grad_norm=cfg.max_grad_norm, arena=arena)
     if cfg.use_rmsprop:
-        return torch.optim.RMSprop(params, lr=cfg.learning_rate, alpha=cfg.rmsprop_alpha, eps=cfg.rmsprop_epsilon,
-                                   centered=True, capturable=graphed)
-    return torch.optim.SGD(params, lr=cfg.learning_rate)
+        return FlatRMSprop(params, lr=cfg.learning_rate, alpha=cfg.rmsprop_alpha, eps=cfg.rmsprop_epsilon, centered=True,
+                           max_grad_norm=cfg.max_grad_norm, arena=arena)
+    return FlatSGD(params, lr=cfg.learning_rate, max_grad_norm=cfg.max_grad_norm, arena=arena)
 
 
 def build_agent(config, obs_shape, n_actions):
@@ -51,8 +50,8 @@ def build_agent(config, obs_shape, n_actions):
             for p in target.parameters():
                 p.requires_grad_(False)
 
-    optimizer = _optimizer(config, online, arena, graphed)
-    if isinstance(optimizer, FlatAdam):
-        optimizer.layout_model = online        # checkpoints in torch.optim.Adam's format, reference parameter order
+    optimizer = _optimizer(config, online, arena)
+    if isinstance(optimizer, FlatOptimizer):
+        optimizer.layout_model = online        # checkpoints in torch.optim's formats, reference parameter order
     return Agent(online, _acting_policy(config), action_selectors.GreedyActionSelector(), optimizer, target, graphed,
                  config.max_grad_norm)

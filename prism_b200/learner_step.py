@@ -27,7 +27,7 @@ UniformSampler (csrc/uniform.cu) in its place -- the same schedule without the p
 import torch
 
 from . import _lib
-from .agents.optim import FlatAdam
+from .agents.optim import FlatOptimizer
 from .experience.per import PrioritizedTree
 from .experience.uniform import UniformSampler
 
@@ -95,8 +95,8 @@ class LearnerStep:
         opt = agent.optimizer
         self.peer = None
         if self.world_size > 1:
-            if not isinstance(opt, FlatAdam):
-                raise _lib.PbError("data parallel needs the FlatAdam arena (one exchange per step)")
+            if not isinstance(opt, FlatOptimizer):
+                raise _lib.PbError("data parallel needs a flat optimizer arena (one exchange per step)")
             import os
             import sys
             import torch.distributed as dist
@@ -301,7 +301,7 @@ class LearnerStep:
         self._trace = {"buf": torch.zeros(max_marks, dtype=torch.int64, device=self.device), "names": {}}
         from .agents import ops as _ops
         opt = self.agent.optimizer
-        if isinstance(opt, FlatAdam):
+        if isinstance(opt, FlatOptimizer):
             opt._mark = self._mark
         _ops.TRACE_MARK = self._mark                  # forward / backward phases inside the agent
         self.graph, self._primed = None, False
@@ -309,7 +309,7 @@ class LearnerStep:
     def disable_trace(self):
         from .agents import ops as _ops
         self._trace = None
-        if isinstance(self.agent.optimizer, FlatAdam):
+        if isinstance(self.agent.optimizer, FlatOptimizer):
             self.agent.optimizer._mark = None
         _ops.TRACE_MARK = None
         self.graph, self._primed = None, False
@@ -449,7 +449,7 @@ class LearnerStep:
 
     def _capture(self, draw, consume=False):
         opt = self.agent.optimizer
-        flat = isinstance(opt, FlatAdam)
+        flat = isinstance(opt, FlatOptimizer)
         # drop every reference to autograd graphs built on another stream (an eager update leaves its
         # loss tensors on the agent): their AccumulateGrad nodes would tie the capture to that stream
         ag = self.agent

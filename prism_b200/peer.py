@@ -15,7 +15,7 @@ import torch
 from . import _lib
 
 
-FUSED_EXCHANGE = __import__("os").environ.get("PB_PEER_FUSED", "1") != "0"   # one-launch exchange + Adam for small arenas
+FUSED_EXCHANGE = __import__("os").environ.get("PB_PEER_FUSED", "1") != "0"   # one-launch exchange + update for small arenas
 ONE_SHOT_MAX_BYTES = 32 * 1024 * 1024      # n * 4 * world up to which the one-shot (single barrier) all-reduce is used
 WAIT_TIMEOUT_S = float(__import__("os").environ.get("PB_PEER_TIMEOUT_S", "20"))   # bound of every cross-GPU flag wait
 
@@ -143,7 +143,9 @@ class PeerGroup:
                                % (WAIT_TIMEOUT_S, st, self.rank, self.world))
 
     def allreduce_adam(self, opt, mark=None):
-        """Sum the gradient arenas over the ranks and apply clip + Adam on every replica (csrc/peer.cu).
+        """Sum the gradient arenas over the ranks and apply clip + the optimizer's update on every replica
+        (csrc/peer.cu).  ``opt.rule`` (a ``_lib.PB_OPT_*``) selects Adam, RMSprop or SGD; an optimizer without one is
+        Adam, read through ``betas``.
 
         ONE cross-GPU handshake per step for small arenas: it tells every rank all gradients are packed (the fused
         launch signals on channel 1 itself; the multi-launch schedules run ``state_allgather`` of a dummy block).  The
@@ -151,14 +153,16 @@ class PeerGroup:
         overwrites what a slower rank still pulls -- no trailing barrier."""
         lib, st = _lib.load(), self._stream()
         mark = mark or (lambda name: None)                        # timeline marks of LearnerStep.enable_trace()
-        if (FUSED_EXCHANGE and self.n <= int(lib.pb_peer_allreduce_adam_max_n())
+        rule = getattr(opt, "rule", _lib.PB_OPT_ADAM)
+        h1, h2 = opt._hyper() if hasattr(opt, "_hyper") else opt.betas
+        m, v = _lib.ptr(opt.exp_avg), _lib.ptr(opt.exp_avg_sq)
+        if (FUSED_EXCHANGE and self.n <= int(lib.pb_peer_allreduce_opt_max_n(rule))
                 and self.n * 4 * self.world <= ONE_SHOT_MAX_BYTES):
-            # small arena: handshake + pulls + global norm + clip + Adam in ONE launch
-            _lib.check(lib.pb_peer_allreduce_adam(C.byref(self.c), self.n, opt.arena.data_ptr(), opt.exp_avg.data_ptr(),
-                                                  opt.exp_avg_sq.data_ptr(), opt.step_count.data_ptr(), opt.lr,
-                                                  opt.betas[0], opt.betas[1], opt.eps, opt.max_grad_norm,
-                                                  opt.partials.data_ptr(), opt.norm_out.data_ptr(), st),
-                       "pb_peer_allreduce_adam")
+            # small arena: handshake + pulls + global norm + clip + update in ONE launch
+            _lib.check(lib.pb_peer_allreduce_opt(rule, C.byref(self.c), self.n, opt.arena.data_ptr(), m, v,
+                                                 opt.step_count.data_ptr(), opt.lr, h1, h2, opt.eps, opt.max_grad_norm,
+                                                 opt.partials.data_ptr(), opt.norm_out.data_ptr(), st),
+                       "pb_peer_allreduce_opt")
             self._n_gathers += 1                                  # channel 1 advanced: the other half of the arena is next
             mark("opt:applied")
             return
@@ -170,10 +174,10 @@ class PeerGroup:
             _lib.check(lib.pb_peer_pull_sum(C.byref(self.c), self.n, opt.partials.data_ptr(), opt.step_count.data_ptr(),
                                             C.byref(n_part), st), "pb_peer_pull_sum")
             mark("opt:summed")
-            _lib.check(lib.pb_adam_clip_apply(self.n, opt.arena.data_ptr(), self.reduced.data_ptr(), opt.exp_avg.data_ptr(),
-                                              opt.exp_avg_sq.data_ptr(), opt.step_count.data_ptr(), opt.lr, opt.betas[0],
-                                              opt.betas[1], opt.eps, opt.max_grad_norm, opt.partials.data_ptr(), n_part.value,
-                                              opt.norm_out.data_ptr(), st), "pb_adam_clip_apply")
+            _lib.check(lib.pb_opt_clip_apply(rule, self.n, opt.arena.data_ptr(), self.reduced.data_ptr(), m, v,
+                                             opt.step_count.data_ptr(), opt.lr, h1, h2, opt.eps, opt.max_grad_norm,
+                                             opt.partials.data_ptr(), n_part.value, opt.norm_out.data_ptr(), st),
+                       "pb_opt_clip_apply")
             mark("opt:applied")
             return
         _lib.check(lib.pb_peer_reduce_scatter(C.byref(self.c), self.n, opt.partials.data_ptr(), opt.step_count.data_ptr(), st),
@@ -181,9 +185,9 @@ class PeerGroup:
         mark("opt:slice_reduced")
         _lib.check(lib.pb_peer_barrier(C.byref(self.c), st), "pb_peer_barrier")            # every slice reduced + norms published
         mark("opt:all_reduced")
-        _lib.check(lib.pb_peer_adam(C.byref(self.c), self.n, opt.arena.data_ptr(), opt.exp_avg.data_ptr(),
-                                    opt.exp_avg_sq.data_ptr(), opt.step_count.data_ptr(), opt.lr, opt.betas[0], opt.betas[1],
-                                    opt.eps, opt.max_grad_norm, opt.norm_out.data_ptr(), None, st), "pb_peer_adam")
+        _lib.check(lib.pb_peer_opt(rule, C.byref(self.c), self.n, opt.arena.data_ptr(), m, v, opt.step_count.data_ptr(),
+                                   opt.lr, h1, h2, opt.eps, opt.max_grad_norm, opt.norm_out.data_ptr(), None, st),
+                   "pb_peer_opt")
 
     def close(self):
         """Unmap the peers' blocks and free this rank's own.  Every rank must have finished its last exchange (the
