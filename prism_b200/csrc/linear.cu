@@ -51,6 +51,20 @@ struct GemmArgs {
     int n_seg, splits, act, m_tiles;
 };
 
+// r[q] = 0 where !(m[q] > 0): the ReLU mask of four consecutive elements.  The mask has the operand's layout but its own
+// base address, so a float4 load is taken only when it is 16-byte aligned itself.
+__device__ __forceinline__ void mask4(float (&r)[4], const float *m)
+{
+    if ((reinterpret_cast<uintptr_t>(m) & 15) == 0) {
+        const float4 v = *reinterpret_cast<const float4 *>(m);
+        r[0] = v.x > 0.f ? r[0] : 0.f; r[1] = v.y > 0.f ? r[1] : 0.f;
+        r[2] = v.z > 0.f ? r[2] : 0.f; r[3] = v.w > 0.f ? r[3] : 0.f;
+    } else {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) r[q] = m[q] > 0.f ? r[q] : 0.f;
+    }
+}
+
 template <bool KMAJOR>
 __device__ __forceinline__ void load_tile(float (&r)[4], const float *__restrict__ P, const float *__restrict__ mask,
                                           int ld, int row0, int k0, int rows, int kmax, int t, int half)
@@ -66,11 +80,7 @@ __device__ __forceinline__ void load_tile(float (&r)[4], const float *__restrict
         if (vec_ok && row < rows && k + 3 < kmax && (k & 3) == 0) {
             float4 v = *reinterpret_cast<const float4 *>(P + off);
             r[0] = v.x; r[1] = v.y; r[2] = v.z; r[3] = v.w;
-            if (mask) {
-                float4 m = *reinterpret_cast<const float4 *>(mask + off);
-                r[0] = m.x > 0.f ? r[0] : 0.f; r[1] = m.y > 0.f ? r[1] : 0.f;
-                r[2] = m.z > 0.f ? r[2] : 0.f; r[3] = m.w > 0.f ? r[3] : 0.f;
-            }
+            if (mask) mask4(r, mask + off);
         } else {
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
@@ -87,11 +97,7 @@ __device__ __forceinline__ void load_tile(float (&r)[4], const float *__restrict
         if (vec_ok && k < kmax && row + 3 < rows && (row & 3) == 0) {
             float4 v = *reinterpret_cast<const float4 *>(P + off);
             r[0] = v.x; r[1] = v.y; r[2] = v.z; r[3] = v.w;
-            if (mask) {
-                float4 m = *reinterpret_cast<const float4 *>(mask + off);
-                r[0] = m.x > 0.f ? r[0] : 0.f; r[1] = m.y > 0.f ? r[1] : 0.f;
-                r[2] = m.z > 0.f ? r[2] : 0.f; r[3] = m.w > 0.f ? r[3] : 0.f;
-            }
+            if (mask) mask4(r, mask + off);
         } else {
 #pragma unroll
             for (int q = 0; q < 4; ++q) {

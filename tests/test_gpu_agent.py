@@ -278,17 +278,28 @@ def test_learner_step_graph_after_eager_update():
     assert st["status"] == 0 and st["len"] == cap
 
 
-@pytest.mark.parametrize("K,M,N,J,shared,relu", [
-    (1, 256, 256, 1024, True, True), (1, 256, 4, 256, False, False), (10, 64, 256, 1024, True, True),
-    (10, 64, 3, 256, False, False), (3, 37, 19, 50, False, True), (1, 2048, 256, 1024, True, True),
-    (4, 5, 7, 3, True, False), (1, 512, 512, 3136, True, True),
-    # 16-byte aligned operands with ragged tiles: the cp.async kernel's zero-filled row / column / k tails (272 rows = the
-    # padded data-parallel batch); (3, 37, 19, 50) and (4, 5, 7, 3) above are unaligned: the register-staged kernel
-    (2, 272, 200, 1000, False, True), (1, 100, 36, 68, True, True), (3, 64, 64, 36, False, False)])
-def test_fused_linear_matches_torch(K, M, N, J, shared, relu):
-    """pb_linear_{fwd,bwd_input,bwd_weight} (cluster split-K GEMM, 3xTF32 products, fused bias/ReLU/mask/bias-grad;
-    cp.async operand tiles when aligned, register-staged otherwise) against torch fp64 math; tolerance 2e-5 relative of
-    the tensor's max (fp32 accumulation order)."""
+FUSED_LINEAR_CASES = [
+    (1, 256, 256, 1024, True, True, "linear:ffma"), (1, 256, 4, 256, False, False, "linear:narrow"),
+    (10, 64, 256, 1024, True, True, "linear:ffma"), (10, 64, 3, 256, False, False, "linear:narrow"),
+    (3, 37, 19, 50, False, True, "linear:ffma"), (1, 2048, 256, 1024, True, True, "linear:tc_gemm"),
+    (4, 5, 7, 3, True, False, "linear:ffma"), (1, 512, 512, 3136, True, True, "linear:tc_gemm"),
+    # 2 * 272 * 2 * 200 * 1000 = 2.2e8 FLOP reaches TC_MIN_FLOPS: tcgen05, not linear.cu
+    (2, 272, 200, 1000, False, True, "linear:tc_gemm"),
+    # 16-byte aligned operands with ragged tiles: the cp.async kernel's zero-filled row / column / k tails;
+    # (3, 37, 19, 50) and (4, 5, 7, 3) above are unaligned: the register-staged kernel
+    (1, 100, 36, 68, True, True, "linear:ffma"), (3, 64, 64, 36, False, False, "linear:ffma"),
+    # the data-parallel layer (272 rows = the padded batch): 16 live rows in the last M tile, an empty split in dW
+    (1, 272, 256, 1024, True, True, "linear:ffma")]
+
+
+@pytest.mark.parametrize("K,M,N,J,shared,relu,route", FUSED_LINEAR_CASES,
+                         ids=["-".join(map(str, c[:6])) for c in FUSED_LINEAR_CASES])     # the route is not part of the id
+def test_fused_linear_matches_torch(K, M, N, J, shared, relu, route):
+    """A dense layer through ops.linear_heads against torch fp64 math, on the route the test names: linear:ffma is
+    pb_linear_{fwd,bwd_input,bwd_weight} (cluster split-K GEMM, 3xTF32 products, fused bias/ReLU/mask/bias-grad;
+    cp.async operand tiles when aligned, register-staged otherwise; every path of it: tests/test_gpu_linear.py),
+    linear:tc_gemm the tcgen05 GEMM, linear:narrow the narrow output-layer kernels.  Tolerance 2e-5 relative of the
+    tensor's max (fp32 accumulation order)."""
     from prism_b200.agents import ops
     g = torch.Generator().manual_seed(K * 1000 + M + N + J)
     x = torch.randn((M, J) if shared else (K, M, J), generator=g)
@@ -306,7 +317,9 @@ def test_fused_linear_matches_torch(K, M, N, J, shared, relu):
         yr = yr.relu()
     yr.backward(gy.double())
     xd, wd, bd = (t.to(DEV).requires_grad_(True) for t in (x, w, b))
+    ops.route_counts(reset=True)
     y = ops.linear_heads(xd, wd, bd, relu=relu)
+    assert ops.route_counts() == {route: 1}, ops.route_counts()
     y.backward(gy.to(DEV))
     torch.cuda.synchronize()
     assert rel_err(y.detach().cpu().numpy(), yr.detach().numpy()) < 2e-5
@@ -816,7 +829,8 @@ def test_static_batch_overflow_is_refused_and_ring_growth_recaptures():
                     buf._nonterminal, buf._action)
 
 
-@pytest.mark.parametrize("M,N,J", [(32768, 18, 512), (2048, 3, 256), (1000, 6, 64), (777, 32, 1024), (4100, 4, 320)])
+@pytest.mark.parametrize("M,N,J", [(32768, 18, 512), (2048, 3, 256), (1000, 6, 64), (777, 32, 1024), (4100, 4, 320),
+                                   (2048, 9, 512), (600, 16, 128)])     # N 9..16: narrow_*_kernel<16>
 def test_narrow_linear_matches_fp64(M, N, J):
     """pb_narrow_linear_fwd / _bwd (the n_actions-wide output layer of the IQN head) against fp64 math + autograd."""
     from prism_b200.agents import ops
@@ -927,7 +941,7 @@ def test_sum_leading_matches_torch():
 
 
 @pytest.mark.parametrize("K,M,N,J,shared", [(10, 64, 3, 256, False), (10, 512, 18, 512, False), (1, 256, 4, 256, False),
-                                            (4, 100, 6, 128, True)])
+                                            (4, 100, 6, 128, True), (10, 64, 9, 256, False), (4, 300, 16, 512, True)])
 def test_narrow_linear_heads_matches_fp64(K, M, N, J, shared):
     """The n_actions-wide last layer of the K ensemble heads through the narrow kernels (batched over heads)."""
     from prism_b200.agents import ops
@@ -950,3 +964,36 @@ def test_narrow_linear_heads_matches_fp64(K, M, N, J, shared):
     assert rel_err(xd.grad.cpu().numpy(), x64.grad.numpy()) < 2e-6
     assert rel_err(wd.grad.cpu().numpy(), w64.grad.numpy()) < 2e-5
     assert rel_err(bd.grad.cpu().numpy(), b64.grad.numpy()) < 2e-5
+
+
+@pytest.mark.parametrize("K,M,N,J,shared", [(10, 256, 9, 256, False), (4, 4100, 16, 320, True)])
+def test_narrow_linear_split_reduce_equals_one_call(K, M, N, J, shared):
+    """pb_narrow_linear_bwd with dW = db = NULL, then pb_narrow_linear_bwd_reduce on a second stream ordered after it
+    (as the learner step's graph runs it) gives the same bits as the one-call form."""
+    from prism_b200 import _lib
+    lib = _lib.load()
+    g = torch.Generator().manual_seed(K * 13 + M + N)
+    x = torch.randn((M, J) if shared else (K, M, J), generator=g).to(DEV)
+    w = (torch.randn(K, N, J, generator=g) / J ** 0.5).to(DEV)
+    dy = torch.randn(K, M, N, generator=g).to(DEV)
+    xhs = 0 if shared else M * J
+    nb = lib.pb_narrow_linear_bwd_blocks(M)
+    nan = lambda *shape: torch.full(shape, float("nan"), device=DEV)
+    cur = torch.cuda.current_stream()
+    dx1, dw1, db1, part1 = nan(K, M, J), nan(K, N, J), nan(K, N), nan(K * nb * (N * J + N))
+    _lib.check(lib.pb_narrow_linear_bwd(K, M, N, J, x.data_ptr(), xhs, w.data_ptr(), dy.data_ptr(), dx1.data_ptr(),
+                                        dw1.data_ptr(), db1.data_ptr(), part1.data_ptr(), cur.cuda_stream))
+    dx2, dw2, db2, part2 = nan(K, M, J), nan(K, N, J), nan(K, N), nan(K * nb * (N * J + N))
+    _lib.check(lib.pb_narrow_linear_bwd(K, M, N, J, x.data_ptr(), xhs, w.data_ptr(), dy.data_ptr(), dx2.data_ptr(),
+                                        None, None, part2.data_ptr(), cur.cuda_stream))
+    side = torch.cuda.Stream()
+    side.wait_stream(cur)
+    _lib.check(lib.pb_narrow_linear_bwd_reduce(K, M, N, J, part2.data_ptr(), dw2.data_ptr(), db2.data_ptr(),
+                                               side.cuda_stream))
+    cur.wait_stream(side)
+    torch.cuda.synchronize()
+    for a, b in ((dx1, dx2), (dw1, dw2), (db1, db2)):
+        assert not torch.isnan(a).any() and torch.equal(a, b)
+    xe = x.double().cpu().expand(K, M, J) if shared else x.double().cpu()
+    assert rel_err(dw2.cpu().numpy(), (dy.double().cpu().transpose(1, 2) @ xe).numpy()) < 2e-5
+    assert rel_err(db2.cpu().numpy(), dy.double().cpu().sum(1).numpy()) < 2e-5
