@@ -350,6 +350,44 @@ int pb_ids_select(int N, int A, int K, int Nq, const float *q, const float *z, f
                   float eps, float rho_lower_bound, long long *action_out, float *scores_out,
                   void *stream);
 
+/* Value squashing (Config.loss_squish_fn_id; the (squish, unsquish) pairs of prism/agents/squish_functions.py):
+ *   PB_SQUASH_NONE              identity
+ *   PB_SQUASH_OBS_LOOK_FURTHER  h(x) = sign(x) (sqrt(|x| + 1) - 1) + eps x, eps = PB_SQUASH_OLF_EPS; h^-1 its inverse
+ *   PB_SQUASH_SYMLOG            h(x) = sign(x) log1p(|x|), h^-1(x) = sign(x) expm1(|x|)
+ * evaluated in cancellation-free fp32 forms (csrc/common.cuh).  The _sq entries below are the entries above with the
+ * kind as a last argument; the entries above are the _sq entries with PB_SQUASH_NONE.  An unknown kind is
+ * PB_E_UNSUPPORTED (nothing is launched).
+ *   pb_iqn_qh_loss_sq        y_bj = h(R_b + gdn_b * h^-1(z_next_target[j,b,a*])); a* from the raw online quantiles;
+ *                            theta and the gradient stay in network-output (squashed) space
+ *   pb_ens_q_loss_sq(_total) y_k = h(R + gdn * h^-1(q_next_target[k,b,a*_k]))
+ *   pb_ids_select_sq         every q and z element passes through h^-1 before the moments (scores_out included)
+ * pb_value_squash: y[i] = h(x[i]) (inverse = 0) or h^-1(x[i]) (inverse = 1) for n elements; x == y is allowed. */
+#define PB_SQUASH_NONE 0
+#define PB_SQUASH_OBS_LOOK_FURTHER 1
+#define PB_SQUASH_SYMLOG 2
+#define PB_SQUASH_OLF_EPS 1e-2f
+int pb_iqn_qh_loss_sq(int B, int T, int Tp, int A, const float *z_cur, const float *tau,
+                      const float *z_next_online, const float *z_next_target,
+                      const long long *action, const float *ret, const float *gdn,
+                      const uint8_t *nonterminal, float kappa, float loss_weight,
+                      const float *row_weight, float grad_scale, float *loss_out, float *grad_z_cur,
+                      void *stream, int squash);
+int pb_ens_q_loss_sq(int B, int A, int K, const float *q_cur, const float *q_next_online,
+                     const float *q_next_target, const long long *action, const float *ret,
+                     const float *gdn, const uint8_t *nonterminal, float loss_weight,
+                     const float *row_weight, float grad_scale, float *loss_out, float *grad_q_cur,
+                     void *stream, int squash);
+int pb_ens_q_loss_total_sq(int B, int A, int K, const float *q_cur, const float *q_next_online,
+                           const float *q_next_target, const long long *action, const float *ret, const float *gdn,
+                           const uint8_t *nonterminal, float loss_weight, const float *row_weight, float grad_scale,
+                           float *loss_out, float *grad_q_cur, const float *dist, float q_scale,
+                           const float *q_offset, float *total_out, float *td_out, unsigned int *ticket,
+                           void *stream, int squash);
+int pb_ids_select_sq(int N, int A, int K, int Nq, const float *q, const float *z, float lambda,
+                     float eps, float rho_lower_bound, long long *action_out, float *scores_out,
+                     void *stream, int squash);
+int pb_value_squash(long long n, const float *x, float *y, int squash, int inverse, void *stream);
+
 /* GreedyActionSelector (action_selectors.py:70-82): argmax_a mean_k q */
 int pb_greedy_select(int N, int A, int K, const float *q, long long *action_out, void *stream);
 

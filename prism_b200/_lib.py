@@ -109,6 +109,12 @@ SIGNATURES = {
     "pb_ens_q_loss": [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _F, _P, _F, _P, _P, _P],
     "pb_ens_q_loss_total": [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _F, _P, _F, _P, _P, _P, _F, _P, _P, _P, _P, _P],
     "pb_ids_select": [_I, _I, _I, _I, _P, _P, _F, _F, _F, _P, _P, _P],
+    "pb_iqn_qh_loss_sq": [_I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _F, _F, _P, _F, _P, _P, _P, _I],
+    "pb_ens_q_loss_sq": [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _F, _P, _F, _P, _P, _P, _I],
+    "pb_ens_q_loss_total_sq": [_I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _F, _P, _F, _P, _P, _P, _F, _P, _P, _P, _P, _P,
+                               _I],
+    "pb_ids_select_sq": [_I, _I, _I, _I, _P, _P, _F, _F, _F, _P, _P, _P, _I],
+    "pb_value_squash": [_LL, _P, _P, _I, _I, _P],
     "pb_greedy_select": [_I, _I, _I, _P, _P, _P],
     "pb_adam_clip_step": [_LL, _P, _P, _P, _P, _P, _F, _F, _F, _F, _F, _P, _P, _P],
     "pb_adam_fused_max_n": [],
@@ -191,6 +197,9 @@ _RESTYPES = {"pb_error_string": C.c_char_p, "pb_launch_count": C.c_longlong, "pb
 
 # update rules of the pb_opt_* / pb_peer_*_opt entries (include/prism_b200.h)
 PB_OPT_ADAM, PB_OPT_RMSPROP, PB_OPT_RMSPROP_CENTERED, PB_OPT_SGD = 0, 1, 2, 3
+# value squashing kinds of the *_sq entries and pb_value_squash, and the obs_look_further epsilon (include/prism_b200.h)
+PB_SQUASH_NONE, PB_SQUASH_OBS_LOOK_FURTHER, PB_SQUASH_SYMLOG = 0, 1, 2
+PB_SQUASH_OLF_EPS = 1e-2
 
 PB_E_POOL = -4
 ABI_VERSION = 2

@@ -5,6 +5,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .squish_functions import unsquash_kind
 
 
 class ActionSelector(object):
@@ -109,14 +110,18 @@ class IDSActionSelector(ActionSelector):
     """Information-directed sampling, deterministic branch (action_selectors.py:114-176).
 
     Reproduces the reference's naming quirk: the ensemble "variance" is torch.std and its "std"
-    is sqrt(std) (SURVEY appendix Q1)."""
+    is sqrt(std) (SURVEY appendix Q1).  With an unsquish function (squish_functions.py) every q and z value is read
+    through it, inside the selection kernel."""
+
+    squash = 0              # PB_SQUASH_NONE; also what a selector pickled before value squashing existed reads
 
     def __init__(self, lmbda, random_sample, epsilon, ids_rho_lower_bound, beta, unsquish_function=None):
         super().__init__()
         if random_sample:
             raise NotImplementedError("ids_use_random_samples=True is not used by any reference config")
-        if unsquish_function is not None:
-            raise NotImplementedError("value squashing is outside the hot-path scope")
+        # every q and z value is unsquashed inside the selection kernel: the function is recognised, not called
+        self.squash = unsquash_kind(unsquish_function)
+        self.unsquish_function = unsquish_function
         self.random_sample = random_sample
         self.beta = beta
         self.lmbda = lmbda
@@ -125,7 +130,7 @@ class IDSActionSelector(ActionSelector):
 
     def generate_action_probs(self, action_value_distribution, q_estimates, for_log=False):
         out = ops.ids_select(_head_major(q_estimates), action_value_distribution, self.lmbda, self.epsilon,
-                             self.ids_rho_lower_bound, return_scores=for_log)
+                             self.ids_rho_lower_bound, return_scores=for_log, squash=self.squash)
         action, scores = out if for_log else (out, None)
         probs = torch.nn.functional.one_hot(action, q_estimates.shape[1])
         if for_log:

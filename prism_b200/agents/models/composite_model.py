@@ -194,7 +194,9 @@ class CompositeModel(nn.Module):
         w = per_weights if isinstance(per_weights, torch.Tensor) else None
         off = None if theil is None else (theil.detach() * ens.ensemble_variation_coef).float()
         total, dist, mse, td = ops.fused_total_loss(z_cur, q_cur, tau, z_on, z_tg, q_on, q_tg, acts, returns, gamma,
-                                                    nonterm, w, off, T, Tp, kappa, dist_w, q_w)
+                                                    nonterm, w, off, T, Tp, kappa, dist_w, q_w,
+                                                    dist_squash=iqn.squash if iqn is not None else 0,
+                                                    q_squash=ens.squash if ens is not None else 0)
         if theil is not None:
             # the regulariser's own gradient: d total / d theil = -q_w * coef * mean(w)
             mean_w = w.mean() if w is not None else 1.0

@@ -16,6 +16,7 @@ import torch
 import torch.nn as nn
 
 from .. import ops
+from ..squish_functions import squash_kind
 from .ffnn_model import FFNNModel
 
 
@@ -28,9 +29,12 @@ class IQNModel(nn.Module):
                  distributional_loss_weight=1, sparse_init_p=0.0,
                  propagate_grad=True, risk_policy=None, device="cpu"):
         super().__init__()
-        if squish_function is not None or unsquish_function is not None or risk_policy is not None:
-            # every BASELINE config runs loss_squish_fn_id="none" and the neutral risk policy (SURVEY 2 row 9)
-            raise NotImplementedError("value squashing / risk policies are outside the hot-path scope")
+        if risk_policy is not None:
+            # every BASELINE config runs the neutral risk policy (SURVEY 2 row 9)
+            raise NotImplementedError("risk policies are outside the hot-path scope")
+        # value squashing of the targets happens inside the loss kernel: the pair is recognised, not called
+        self.squash = squash_kind(squish_function, unsquish_function)
+        self.squish_function, self.unsquish_function = squish_function, unsquish_function
         self.device = device
         self.n_actions = n_actions
         self.n_basis_elements = n_basis_elements
@@ -156,7 +160,7 @@ class IQNModel(nn.Module):
         return ops.quantile_huber_loss(z_cur, tau, z_next_online, z_next_target, batch_acts, batch_returns,
                                        dones_and_gamma, self.n_current_quantile_samples,
                                        self.n_next_quantile_samples, kappa=self.huber_k,
-                                       loss_weight=self.distributional_loss_weight)
+                                       loss_weight=self.distributional_loss_weight, squash=self.squash)
 
     def log(self, logger):
         pass

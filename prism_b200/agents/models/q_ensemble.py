@@ -13,6 +13,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import ops
+from ..squish_functions import squash_kind
 from .ffnn_model import FFNNModel
 
 
@@ -23,11 +24,12 @@ class QEnsemble(nn.Module):
                  squish_function=None, unsquish_function=None,
                  use_double_q_learning=True, sparse_init_p=0.0, device="cpu"):
         super().__init__()
-        if squish_function is not None or unsquish_function is not None:
-            raise NotImplementedError("value squashing is outside the hot-path scope")
         if q_loss_function is not None and not isinstance(q_loss_function, nn.MSELoss):
             # the reference's "huber" option silently falls back to MSE (model_factory.py:43-46)
             raise NotImplementedError("only the MSE Q loss exists in the reference")
+        # value squashing of the targets happens inside the loss kernel: the pair is recognised, not called
+        self.squash = squash_kind(squish_function, unsquish_function)
+        self.squish_function, self.unsquish_function = squish_function, unsquish_function
         self.device = device
         self.q_loss_weight = q_loss_weight
         self.use_double_q_learning = use_double_q_learning
@@ -159,7 +161,7 @@ class QEnsemble(nn.Module):
     def get_loss(self, embedded_obs, embedded_next_obs, batch_acts, batch_returns, dones_and_gamma, target_model=None):
         q_cur, q_next_online, q_next_target = self.q_tables(embedded_obs, embedded_next_obs, target_model)
         q_loss = ops.ensemble_q_loss(q_cur, q_next_online, q_next_target, batch_acts.view(-1), batch_returns,
-                                     dones_and_gamma, loss_weight=1.0)
+                                     dones_and_gamma, loss_weight=1.0, squash=self.squash)
         theil = self.theil_index()
         if theil is None:
             return q_loss if self.q_loss_weight == 1 else self.q_loss_weight * q_loss

@@ -74,7 +74,7 @@ def sum_leading(x):
 
 class _QuantileHuberLoss(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, z_cur, tau, z_next_online, z_next_target, action, ret, gdn, B, T, Tp, kappa, loss_weight):
+    def forward(ctx, z_cur, tau, z_next_online, z_next_target, action, ret, gdn, B, T, Tp, kappa, loss_weight, squash):
         _lib.require_cuda(z_cur, "z_cur")
         A = z_cur.shape[-1]
         z_cur_c, tau_c = _c(z_cur), _c(tau).view(-1)
@@ -82,10 +82,10 @@ class _QuantileHuberLoss(torch.autograd.Function):
         action_c, ret_c, gdn_c = _c(action, torch.int64).view(-1), _c(ret).view(-1), _c(gdn).view(-1)
         loss = torch.empty(B, dtype=torch.float32, device=z_cur.device)
         grad = torch.empty_like(z_cur_c)
-        _lib.check(_lib.load().pb_iqn_qh_loss(
+        _lib.check(_lib.load().pb_iqn_qh_loss_sq(
             B, T, Tp, A, z_cur_c.data_ptr(), tau_c.data_ptr(), zo.data_ptr(), zt.data_ptr(), action_c.data_ptr(),
             ret_c.data_ptr(), gdn_c.data_ptr(), None, float(kappa), float(loss_weight), None, 1.0, loss.data_ptr(),
-            grad.data_ptr(), _stream(z_cur)), "pb_iqn_qh_loss")
+            grad.data_ptr(), _stream(z_cur), int(squash)), "pb_iqn_qh_loss_sq")
         ctx.save_for_backward(grad)
         ctx.dims = (B, T, A)
         return loss
@@ -96,59 +96,74 @@ class _QuantileHuberLoss(torch.autograd.Function):
         B, T, A = ctx.dims
         # rows are quantile-major (r = i*B + b): scale row b of every quantile by dL/dloss_b
         gz = (grad.view(T, B, A) * grad_loss.view(1, B, 1)).view(T * B, A)
-        return (gz,) + (None,) * 11
+        return (gz,) + (None,) * 12
 
 
 def quantile_huber_loss(z_cur, tau, z_next_online, z_next_target, action, ret, gdn, n_cur, n_next, kappa=1.0,
-                        loss_weight=1.0):
+                        loss_weight=1.0, squash=_lib.PB_SQUASH_NONE):
     """IQN loss per batch row, (B,) -- target build, pairwise quantile-Huber and its gradient in
-    one kernel (prism/agents/models/iqn_model.py:110-201)."""
+    one kernel (prism/agents/models/iqn_model.py:110-201).  ``squash`` (PB_SQUASH_*): the targets are
+    h(R + gdn * h^-1(Z_target)) (squish_functions.py)."""
     B = action.numel()
     return _QuantileHuberLoss.apply(z_cur, tau, z_next_online, z_next_target, action, ret, gdn, B, int(n_cur),
-                                    int(n_next), kappa, loss_weight)
+                                    int(n_next), kappa, loss_weight, squash)
 
 
 class _EnsembleQLoss(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight):
+    def forward(ctx, q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight, squash):
         _lib.require_cuda(q_cur, "q_cur")
         K, B, A = q_cur.shape
         qc, qo, qt = _c(q_cur), _c(q_next_online), _c(q_next_target)
         action_c, ret_c, gdn_c = _c(action, torch.int64).view(-1), _c(ret).view(-1), _c(gdn).view(-1)
         loss = torch.empty(B, dtype=torch.float32, device=q_cur.device)
         grad = torch.empty_like(qc)
-        _lib.check(_lib.load().pb_ens_q_loss(
+        _lib.check(_lib.load().pb_ens_q_loss_sq(
             B, A, K, qc.data_ptr(), qo.data_ptr(), qt.data_ptr(), action_c.data_ptr(), ret_c.data_ptr(),
-            gdn_c.data_ptr(), None, float(loss_weight), None, 1.0, loss.data_ptr(), grad.data_ptr(), _stream(q_cur)),
-            "pb_ens_q_loss")
+            gdn_c.data_ptr(), None, float(loss_weight), None, 1.0, loss.data_ptr(), grad.data_ptr(), _stream(q_cur),
+            int(squash)), "pb_ens_q_loss_sq")
         ctx.save_for_backward(grad)
         return loss
 
     @staticmethod
     def backward(ctx, grad_loss):
         (grad,) = ctx.saved_tensors
-        return (grad * grad_loss.view(1, -1, 1),) + (None,) * 6
+        return (grad * grad_loss.view(1, -1, 1),) + (None,) * 7
 
 
-def ensemble_q_loss(q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight=1.0):
+def ensemble_q_loss(q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight=1.0, squash=_lib.PB_SQUASH_NONE):
     """Mean-over-heads MSE with per-head double-Q targets, (B,).  Tables are head-major (K, B, A)
-    (prism/agents/models/q_ensemble.py:62-84)."""
-    return _EnsembleQLoss.apply(q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight)
+    (prism/agents/models/q_ensemble.py:62-84).  ``squash`` (PB_SQUASH_*): the targets are h(R + gdn * h^-1(q_target))."""
+    return _EnsembleQLoss.apply(q_cur, q_next_online, q_next_target, action, ret, gdn, loss_weight, squash)
 
 
-def ids_select(q_kna, z_qna, lmbda, eps, rho_lower_bound, return_scores=False):
+def ids_select(q_kna, z_qna, lmbda, eps, rho_lower_bound, return_scores=False, squash=_lib.PB_SQUASH_NONE):
     """IDS information-ratio argmin (prism/agents/action_selectors.py:125-176).
-    q_kna: (K, N, A) head-major ensemble values; z_qna: (Nq, N, A)."""
+    q_kna: (K, N, A) head-major ensemble values; z_qna: (Nq, N, A).  ``squash`` (PB_SQUASH_*): every q and z value is
+    unsquashed (h^-1) before the moments."""
     _lib.require_cuda(q_kna, "q")
     K, N, A = q_kna.shape
     Nq = z_qna.shape[0]
     q, z = _c(q_kna), _c(z_qna)
     act = torch.empty(N, dtype=torch.int64, device=q.device)
     scores = torch.empty(N, A, dtype=torch.float32, device=q.device) if return_scores else None
-    _lib.check(_lib.load().pb_ids_select(N, A, K, Nq, q.data_ptr(), z.data_ptr(), float(lmbda), float(eps),
-                                         float(rho_lower_bound), act.data_ptr(), _lib.ptr(scores), _stream(q)),
-               "pb_ids_select")
+    _lib.check(_lib.load().pb_ids_select_sq(N, A, K, Nq, q.data_ptr(), z.data_ptr(), float(lmbda), float(eps),
+                                            float(rho_lower_bound), act.data_ptr(), _lib.ptr(scores), _stream(q),
+                                            int(squash)), "pb_ids_select_sq")
     return (act, scores) if return_scores else act
+
+
+def value_squash(x, squash, inverse=False):
+    """h(x) or h^-1(x) elementwise (pb_value_squash), a new fp32 tensor of x's shape.  ``squash``: PB_SQUASH_*.  The
+    squashing functions are applied to targets and to acting inputs, never differentiated: no backward."""
+    _lib.require_cuda(x, "x")
+    if x.requires_grad and torch.is_grad_enabled():
+        raise RuntimeError("value_squash has no backward: call it under torch.no_grad() or on a detached tensor")
+    xc = _c(x.detach())
+    out = torch.empty_like(xc)
+    _lib.check(_lib.load().pb_value_squash(xc.numel(), xc.data_ptr(), out.data_ptr(), int(squash), int(bool(inverse)),
+                                           _stream(xc)), "pb_value_squash")
+    return out
 
 
 def greedy_select(q_kna):
@@ -744,7 +759,7 @@ class _FusedTotalLoss(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, z_cur, q_cur, tau, z_on, z_tg, q_on, q_tg, action, ret, gamma, nonterm, w, q_offset, T, Tp,
-                kappa, dist_weight, q_weight):
+                kappa, dist_weight, q_weight, dist_squash, q_squash):
         ref = z_cur if z_cur is not None else q_cur
         _lib.require_cuda(ref, "tables")
         lib, stream, dev = _lib.load(), _stream(ref), ref.device
@@ -757,11 +772,11 @@ class _FusedTotalLoss(torch.autograd.Function):
             zc = _c(z_cur)
             dist = torch.empty(B, dtype=torch.float32, device=dev)
             gz = torch.empty_like(zc)
-            _lib.check(lib.pb_iqn_qh_loss(B, T, Tp, zc.shape[-1], zc.data_ptr(), _c(tau).view(-1).data_ptr(),
-                                          _c(z_on).data_ptr(), _c(z_tg).data_ptr(), action_c.data_ptr(),
-                                          ret_c.data_ptr(), gamma_c.data_ptr(), _lib.ptr(nt), float(kappa),
-                                          float(dist_weight), _lib.ptr(w_c), 1.0 / B, dist.data_ptr(), gz.data_ptr(),
-                                          stream), "pb_iqn_qh_loss")
+            _lib.check(lib.pb_iqn_qh_loss_sq(B, T, Tp, zc.shape[-1], zc.data_ptr(), _c(tau).view(-1).data_ptr(),
+                                             _c(z_on).data_ptr(), _c(z_tg).data_ptr(), action_c.data_ptr(),
+                                             ret_c.data_ptr(), gamma_c.data_ptr(), _lib.ptr(nt), float(kappa),
+                                             float(dist_weight), _lib.ptr(w_c), 1.0 / B, dist.data_ptr(), gz.data_ptr(),
+                                             stream, int(dist_squash)), "pb_iqn_qh_loss_sq")
         total = torch.empty((), dtype=torch.float32, device=dev)
         td = torch.empty(B, dtype=torch.float32, device=dev)
         if q_cur is not None:
@@ -771,11 +786,12 @@ class _FusedTotalLoss(torch.autograd.Function):
             gq = torch.empty_like(qc)
             # the ensemble loss kernel's last CTA also combines the heads' losses into the PER-weighted total and the TD
             # mix (agent.py:58-64): one launch less on the step's critical path
-            _lib.check(lib.pb_ens_q_loss_total(B, A, K, qc.data_ptr(), _c(q_on).data_ptr(), _c(q_tg).data_ptr(),
-                                               action_c.data_ptr(), ret_c.data_ptr(), gamma_c.data_ptr(), _lib.ptr(nt), 1.0,
-                                               _lib.ptr(w_c), float(q_weight) / B, mse.data_ptr(), gq.data_ptr(),
-                                               _lib.ptr(dist), float(q_weight), _lib.ptr(q_offset), total.data_ptr(),
-                                               td.data_ptr(), _loss_ticket(dev).data_ptr(), stream), "pb_ens_q_loss_total")
+            _lib.check(lib.pb_ens_q_loss_total_sq(B, A, K, qc.data_ptr(), _c(q_on).data_ptr(), _c(q_tg).data_ptr(),
+                                                  action_c.data_ptr(), ret_c.data_ptr(), gamma_c.data_ptr(), _lib.ptr(nt),
+                                                  1.0, _lib.ptr(w_c), float(q_weight) / B, mse.data_ptr(), gq.data_ptr(),
+                                                  _lib.ptr(dist), float(q_weight), _lib.ptr(q_offset), total.data_ptr(),
+                                                  td.data_ptr(), _loss_ticket(dev).data_ptr(), stream, int(q_squash)),
+                       "pb_ens_q_loss_total_sq")
         else:
             _lib.check(lib.pb_loss_combine(B, _lib.ptr(dist), None, _lib.ptr(w_c), float(q_weight),
                                            _lib.ptr(q_offset), total.data_ptr(), td.data_ptr(), stream), "pb_loss_combine")
@@ -789,17 +805,18 @@ class _FusedTotalLoss(torch.autograd.Function):
     def backward(ctx, g_total, *_):
         gz, gq = ctx.saved_tensors
         if g_total is None:
-            return (None,) * 18
+            return (None,) * 20
         if UNIT_TOTAL_GRAD:
             # Agent._loss_and_backward differentiates the scalar total itself: d total / d total = 1 exactly
-            return (gz, gq) + (None,) * 16
-        return (None if gz is None else gz * g_total, None if gq is None else gq * g_total) + (None,) * 16
+            return (gz, gq) + (None,) * 18
+        return (None if gz is None else gz * g_total, None if gq is None else gq * g_total) + (None,) * 18
 
 
 def fused_total_loss(z_cur, q_cur, tau, z_on, z_tg, q_on, q_tg, action, ret, gamma, nonterm, w, q_offset, T, Tp,
-                     kappa, dist_weight, q_weight):
+                     kappa, dist_weight, q_weight, dist_squash=_lib.PB_SQUASH_NONE, q_squash=_lib.PB_SQUASH_NONE):
+    """``dist_squash`` / ``q_squash`` (PB_SQUASH_*): value squashing of the IQN / ensemble targets."""
     return _FusedTotalLoss.apply(z_cur, q_cur, tau, z_on, z_tg, q_on, q_tg, action, ret, gamma, nonterm, w, q_offset,
-                                 T, Tp, kappa, dist_weight, q_weight)
+                                 T, Tp, kappa, dist_weight, q_weight, dist_squash, q_squash)
 
 
 class _ConvEmbed(torch.autograd.Function):

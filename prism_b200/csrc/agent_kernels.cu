@@ -5,6 +5,8 @@
 //   pb_ens_q_loss      QEnsemble.get_loss (MSE, double-Q)   prism/agents/models/q_ensemble.py:50-92
 //   pb_ids_select      IDSActionSelector                    prism/agents/action_selectors.py:125-176
 //   pb_greedy_select   GreedyActionSelector                 prism/agents/action_selectors.py:70-82
+//   pb_value_squash    squish / unsquish functions          prism/agents/squish_functions.py (the *_sq entries: the
+//                      loss and IDS kernels with value squashing as a template parameter, common.cuh)
 //   pb_loss_combine    PER-weighted total + new priorities  prism/agents/agent.py:58-66, composite_model.py:135-142
 //   pb_adam_clip_step  clip_grad_norm_ + Adam               prism/agents/agent.py:73-74, factory/agent_factory.py:44-47
 //   pb_opt_*           clip_grad_norm_ + Adam / RMSprop / SGD  factory/agent_factory.py:40-58
@@ -36,8 +38,10 @@ __global__ void cos_basis_kernel(long long n_rows, int n_basis, const float *__r
 }
 
 // ---------------------------------------------------------------------------------
-// quantile-Huber loss: one warp per batch row.  smem per warp: y[Tp], theta[T], tq[T].
+// quantile-Huber loss: one warp per batch row.  smem per warp: y[Tp], theta[T], tq[T].  S: value squashing of the
+// target (PB_SQUASH_*, common.cuh).
 // ---------------------------------------------------------------------------------
+template <int S>
 __global__ void __launch_bounds__(128) qh_loss_kernel(int B, int T, int Tp, int A, const float *__restrict__ z_cur,
                                                       const float *__restrict__ tau,
                                                       const float *__restrict__ z_next_online,
@@ -66,10 +70,10 @@ __global__ void __launch_bounds__(128) qh_loss_kernel(int B, int T, int Tp, int 
         acc = warp_sum(acc) / (float)Tp;
         if (acc > best_v) { best_v = acc; best_a = a; }
     }
-    // y_j = R + gamma^k * nonterminal * Z_target(s', tau'_j)[a*]   (:136-145)
+    // y_j = h(R + gamma^k * nonterminal * h^-1(Z_target(s', tau'_j)[a*]))   (:136-145)
     const float R = ret[b], g = nonterm ? __fmul_rn(gdn[b], nonterm[b] ? 1.0f : 0.0f) : gdn[b];
     for (int j = lane; j < Tp; j += 32)
-        y[j] = __fadd_rn(R, __fmul_rn(z_next_target[((size_t)j * B + b) * A + best_a], g));
+        y[j] = squash<S>(__fadd_rn(R, __fmul_rn(unsquash<S>(z_next_target[((size_t)j * B + b) * A + best_a]), g)));
     const int act = (int)action[b];
     for (int i = lane; i < T; i += 32) {
         theta[i] = z_cur[((size_t)i * B + b) * A + act];
@@ -106,6 +110,8 @@ __global__ void __launch_bounds__(128) qh_loss_kernel(int B, int T, int Tp, int 
 // ---------------------------------------------------------------------------------
 // ticket != NULL: the LAST CTA to finish also does what loss_combine_kernel does (total = mean(dist * w) + mean(q' * w)
 // with q' = q_scale * (loss - *q_offset), td_b = the TD mix) -- one launch less on the step's critical path.
+// S: value squashing of the target (PB_SQUASH_*, common.cuh).
+template <int S>
 __global__ void __launch_bounds__(128) ens_loss_kernel(int B, int A, int K, const float *__restrict__ q_cur,
                                                        const float *__restrict__ q_next_online,
                                                        const float *__restrict__ q_next_target,
@@ -135,7 +141,7 @@ __global__ void __launch_bounds__(128) ens_loss_kernel(int B, int A, int K, cons
                 float v = q_next_online[row + a];
                 if (v > bv) { bv = v; best = a; }                    // argmax(dim=-2), first index (q_ensemble.py:70)
             }
-            const float yk = __fadd_rn(R, __fmul_rn(q_next_target[row + best], g));  // (:80)
+            const float yk = squash<S>(__fadd_rn(R, __fmul_rn(unsquash<S>(q_next_target[row + best]), g)));  // (:80)
             const float diff = q_cur[row + act] - yk;
             acc += diff * diff;                                      // MSELoss(reduction='none') (:84)
             for (int a = 0; a < A; ++a) grad_q[row + a] = (a == act) ? gs * diff : 0.0f;
@@ -169,8 +175,9 @@ __global__ void __launch_bounds__(128) ens_loss_kernel(int B, int A, int K, cons
 }
 
 // ---------------------------------------------------------------------------------
-// IDS: one warp per state, lane = action (A <= 32).
+// IDS: one warp per state, lane = action (A <= 32).  S: every q and z value is read through h^-1 (PB_SQUASH_*).
 // ---------------------------------------------------------------------------------
+template <int S>
 __global__ void __launch_bounds__(128) ids_select_kernel(int N, int A, int K, int Nq, const float *__restrict__ q,
                                                          const float *__restrict__ z, float lambda, float eps,
                                                          float rho_lb, long long *__restrict__ action_out,
@@ -182,10 +189,10 @@ __global__ void __launch_bounds__(128) ids_select_kernel(int N, int A, int K, in
     const bool on = lane < A;
     // mean / unbiased std over heads (action_selectors.py:132-135; "variance" is std, "std" is sqrt(std))
     double mu = 0.0;
-    if (on) for (int k = 0; k < K; ++k) mu += (double)q[((size_t)k * N + n) * A + lane];
+    if (on) for (int k = 0; k < K; ++k) mu += (double)unsquash<S>(q[((size_t)k * N + n) * A + lane]);
     mu /= (double)K;
     double ss = 0.0;
-    if (on) for (int k = 0; k < K; ++k) { double d = (double)q[((size_t)k * N + n) * A + lane] - mu; ss += d * d; }
+    if (on) for (int k = 0; k < K; ++k) { double d = (double)unsquash<S>(q[((size_t)k * N + n) * A + lane]) - mu; ss += d * d; }
     const float mean = (float)mu;
     const float s1 = (float)sqrt(ss / (double)(K - 1));          // torch.std (unbiased); K==1 -> nan like torch
     const float s2 = sqrtf(s1);
@@ -196,10 +203,10 @@ __global__ void __launch_bounds__(128) ids_select_kernel(int N, int A, int K, in
     const float regret_sq = regret * regret;
     // unbiased variance of the return distribution over quantile samples (:141)
     double zm = 0.0;
-    if (on) for (int j = 0; j < Nq; ++j) zm += (double)z[((size_t)j * N + n) * A + lane];
+    if (on) for (int j = 0; j < Nq; ++j) zm += (double)unsquash<S>(z[((size_t)j * N + n) * A + lane]);
     zm /= (double)Nq;
     double zs = 0.0;
-    if (on) for (int j = 0; j < Nq; ++j) { double d = (double)z[((size_t)j * N + n) * A + lane] - zm; zs += d * d; }
+    if (on) for (int j = 0; j < Nq; ++j) { double d = (double)unsquash<S>(z[((size_t)j * N + n) * A + lane]) - zm; zs += d * d; }
     const float var_z = (float)(zs / (double)(Nq - 1));
     const float mean_var = warp_sum(on ? var_z : 0.0f) / (float)A;
     const float normalized = var_z / (eps + mean_var);           // (:142)
@@ -217,6 +224,14 @@ __global__ void __launch_bounds__(128) ids_select_kernel(int N, int A, int K, in
         if (os < bs || (os == bs && oi < bi)) { bs = os; bi = oi; }
     }
     if (lane == 0) action_out[n] = (bi == 0x7fffffff) ? 0 : bi;
+}
+
+// elementwise h / h^-1 (pb_value_squash)
+template <int S>
+__global__ void __launch_bounds__(256) value_squash_kernel(long long n, const float *x, float *y, int inverse)
+{
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)
+        y[e] = inverse ? unsquash<S>(x[e]) : squash<S>(x[e]);
 }
 
 __global__ void __launch_bounds__(128) greedy_select_kernel(int N, int A, int K, const float *__restrict__ q,
@@ -617,6 +632,12 @@ static decltype(&adam_clip_kernel<PB_OPT_ADAM>) clip_kernel(int rule)
     return nullptr;
 }
 
+// squash kind -> kernel instantiation (nullptr: unknown kind)
+#define PB_SQUASH_PICK(kernel, s)                                                                          \
+    ((s) == PB_SQUASH_NONE ? kernel<PB_SQUASH_NONE>                                                      \
+     : (s) == PB_SQUASH_OBS_LOOK_FURTHER ? kernel<PB_SQUASH_OBS_LOOK_FURTHER>                            \
+     : (s) == PB_SQUASH_SYMLOG ? kernel<PB_SQUASH_SYMLOG> : nullptr)
+
 // CTAs of the rule's fused kernel that are resident at once (its grid never exceeds this: the CTAs meet at a counter)
 static int fused_max_blocks(int rule)
 {
@@ -656,6 +677,17 @@ int pb_iqn_qh_loss(int B, int T, int Tp, int A, const float *z_cur, const float 
                    const uint8_t *nonterminal, float kappa, float loss_weight, const float *row_weight,
                    float grad_scale, float *loss_out, float *grad_z_cur, void *stream)
 {
+    return pb_iqn_qh_loss_sq(B, T, Tp, A, z_cur, tau, z_next_online, z_next_target, action, ret, gdn, nonterminal, kappa,
+                             loss_weight, row_weight, grad_scale, loss_out, grad_z_cur, stream, PB_SQUASH_NONE);
+}
+
+int pb_iqn_qh_loss_sq(int B, int T, int Tp, int A, const float *z_cur, const float *tau, const float *z_next_online,
+                      const float *z_next_target, const long long *action, const float *ret, const float *gdn,
+                      const uint8_t *nonterminal, float kappa, float loss_weight, const float *row_weight,
+                      float grad_scale, float *loss_out, float *grad_z_cur, void *stream, int squash)
+{
+    const auto kernel = PB_SQUASH_PICK(qh_loss_kernel, squash);
+    if (!kernel) return PB_E_UNSUPPORTED;
     if (B < 0 || T <= 0 || Tp <= 0 || A <= 0 || !(kappa > 0.0f)) return PB_E_ARG;
     if (B == 0) return PB_OK;
     if (!z_cur || !tau || !z_next_online || !z_next_target || !action || !ret || !gdn || !loss_out || !grad_z_cur)
@@ -663,7 +695,7 @@ int pb_iqn_qh_loss(int B, int T, int Tp, int A, const float *z_cur, const float 
     const int warps = 4;
     const size_t smem = sizeof(float) * warps * (size_t)(Tp + 2 * T);
     if (smem > 48 * 1024) return PB_E_UNSUPPORTED;
-    PB_LAUNCH(qh_loss_kernel, (unsigned)((B + warps - 1) / warps), warps * 32, smem, stream, B, T, Tp, A, z_cur, tau,
+    PB_LAUNCH(kernel, (unsigned)((B + warps - 1) / warps), warps * 32, smem, stream, B, T, Tp, A, z_cur, tau,
               z_next_online, z_next_target, action, ret, gdn, nonterminal, kappa, loss_weight, row_weight, grad_scale,
               loss_out, grad_z_cur);
     return PB_OK;
@@ -674,11 +706,22 @@ int pb_ens_q_loss(int B, int A, int K, const float *q_cur, const float *q_next_o
                   float loss_weight, const float *row_weight, float grad_scale, float *loss_out, float *grad_q_cur,
                   void *stream)
 {
+    return pb_ens_q_loss_sq(B, A, K, q_cur, q_next_online, q_next_target, action, ret, gdn, nonterminal, loss_weight,
+                            row_weight, grad_scale, loss_out, grad_q_cur, stream, PB_SQUASH_NONE);
+}
+
+int pb_ens_q_loss_sq(int B, int A, int K, const float *q_cur, const float *q_next_online, const float *q_next_target,
+                     const long long *action, const float *ret, const float *gdn, const uint8_t *nonterminal,
+                     float loss_weight, const float *row_weight, float grad_scale, float *loss_out, float *grad_q_cur,
+                     void *stream, int squash)
+{
+    const auto kernel = PB_SQUASH_PICK(ens_loss_kernel, squash);
+    if (!kernel) return PB_E_UNSUPPORTED;
     if (B < 0 || A <= 0 || K <= 0) return PB_E_ARG;
     if (B == 0) return PB_OK;
     if (!q_cur || !q_next_online || !q_next_target || !action || !ret || !gdn || !loss_out || !grad_q_cur)
         return PB_E_ARG;
-    PB_LAUNCH_PDL_CHAIN(ens_loss_kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
+    PB_LAUNCH_PDL_CHAIN(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
               action, ret, gdn, nonterminal, loss_weight, row_weight, grad_scale, loss_out, grad_q_cur,
               (const float *)nullptr, 1.0f, (const float *)nullptr, (float *)nullptr, (float *)nullptr, (unsigned int *)nullptr);
     return PB_OK;
@@ -690,12 +733,26 @@ int pb_ens_q_loss_total(int B, int A, int K, const float *q_cur, const float *q_
                         const float *dist, float q_scale, const float *q_offset, float *total_out, float *td_out,
                         unsigned int *ticket, void *stream)
 {
+    return pb_ens_q_loss_total_sq(B, A, K, q_cur, q_next_online, q_next_target, action, ret, gdn, nonterminal,
+                                  loss_weight, row_weight, grad_scale, loss_out, grad_q_cur, dist, q_scale, q_offset,
+                                  total_out, td_out, ticket, stream, PB_SQUASH_NONE);
+}
+
+int pb_ens_q_loss_total_sq(int B, int A, int K, const float *q_cur, const float *q_next_online,
+                           const float *q_next_target, const long long *action, const float *ret, const float *gdn,
+                           const uint8_t *nonterminal, float loss_weight, const float *row_weight, float grad_scale,
+                           float *loss_out, float *grad_q_cur, const float *dist, float q_scale,
+                           const float *q_offset, float *total_out, float *td_out, unsigned int *ticket,
+                           void *stream, int squash)
+{
+    const auto kernel = PB_SQUASH_PICK(ens_loss_kernel, squash);
+    if (!kernel) return PB_E_UNSUPPORTED;
     if (B < 0 || A <= 0 || K <= 0) return PB_E_ARG;
     if (B == 0) return PB_OK;
     if (!q_cur || !q_next_online || !q_next_target || !action || !ret || !gdn || !loss_out || !grad_q_cur || !total_out ||
         !ticket)
         return PB_E_ARG;
-    PB_LAUNCH_PDL_CHAIN(ens_loss_kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
+    PB_LAUNCH_PDL_CHAIN(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
               action, ret, gdn, nonterminal, loss_weight, row_weight, grad_scale, loss_out, grad_q_cur, dist, q_scale,
               q_offset, total_out, td_out, ticket);
     return PB_OK;
@@ -704,12 +761,35 @@ int pb_ens_q_loss_total(int B, int A, int K, const float *q_cur, const float *q_
 int pb_ids_select(int N, int A, int K, int Nq, const float *q, const float *z, float lambda, float eps,
                   float rho_lower_bound, long long *action_out, float *scores_out, void *stream)
 {
+    return pb_ids_select_sq(N, A, K, Nq, q, z, lambda, eps, rho_lower_bound, action_out, scores_out, stream,
+                            PB_SQUASH_NONE);
+}
+
+int pb_ids_select_sq(int N, int A, int K, int Nq, const float *q, const float *z, float lambda, float eps,
+                     float rho_lower_bound, long long *action_out, float *scores_out, void *stream, int squash)
+{
+    const auto kernel = PB_SQUASH_PICK(ids_select_kernel, squash);
+    if (!kernel) return PB_E_UNSUPPORTED;
     if (N < 0 || A <= 0 || K <= 0 || Nq <= 0) return PB_E_ARG;
     if (A > 32) return PB_E_UNSUPPORTED;
     if (N == 0) return PB_OK;
     if (!q || !z || !action_out) return PB_E_ARG;
-    PB_LAUNCH(ids_select_kernel, (unsigned)((N + 3) / 4), 128, 0, stream, N, A, K, Nq, q, z, lambda, eps,
+    PB_LAUNCH(kernel, (unsigned)((N + 3) / 4), 128, 0, stream, N, A, K, Nq, q, z, lambda, eps,
               rho_lower_bound, action_out, scores_out);
+    return PB_OK;
+}
+
+int pb_value_squash(long long n, const float *x, float *y, int squash, int inverse, void *stream)
+{
+    const auto kernel = PB_SQUASH_PICK(value_squash_kernel, squash);
+    if (!kernel) return PB_E_UNSUPPORTED;
+    if (n < 0 || (inverse != 0 && inverse != 1)) return PB_E_ARG;
+    if (n == 0) return PB_OK;
+    if (!x || !y) return PB_E_ARG;
+    long long nb = (n + 255) / 256;
+    const long long cap = (long long)pb_sm_count() * 16;
+    if (nb > cap) nb = cap;
+    PB_LAUNCH(kernel, (unsigned)nb, 256, 0, stream, n, x, y, inverse);
     return PB_OK;
 }
 

@@ -249,4 +249,47 @@ __device__ __forceinline__ void opt_update(float &p, float g, float &m, float &v
     }
 }
 
+// ---------------------------------------------------------------------------------
+// Value squashing (PB_SQUASH_*, Config.loss_squish_fn_id): h maps returns into the space the networks predict in, h^-1
+// maps predictions back.  S = PB_SQUASH_NONE is the identity and adds no instruction to a kernel templated on S.
+//   PB_SQUASH_OBS_LOOK_FURTHER  h(x)    = sign(x) (sqrt(|x| + 1) - 1) + eps x                   (Pohlen et al. 2018)
+//                               h^-1(x) = sign(x) ((t - 1)^2 + 2 (t - 1)),  t = (sqrt(1 + 4 eps (|x| + 1 + eps)) - 1) / (2 eps)
+//   PB_SQUASH_SYMLOG            h(x)    = sign(x) log1p(|x|),  h^-1(x) = sign(x) expm1(|x|)
+// The textbook forms cancel in fp32 (sqrt(a + 1) - 1 near a = 0, and the 1/(2 eps)-scaled difference of h^-1, up to
+// 1.2e-5 max(1, |x|)); the forms below have no cancellation: sqrt(a + 1) - 1 = a / (sqrt(a + 1) + 1) and, with
+// s = sqrt(1 + 4 eps (a + 1 + eps)), t - 1 = 2 a / (s + 1 + 2 eps).  Explicit _rn operations: no FMA contraction, so
+// tests/squash_oracle.py restates the same roundings.  copysignf keeps the sign of +-0 and propagates NaN.
+// ---------------------------------------------------------------------------------
+template <int S>
+__device__ __forceinline__ float squash(float x)
+{
+    static_assert(S == PB_SQUASH_NONE || S == PB_SQUASH_OBS_LOOK_FURTHER || S == PB_SQUASH_SYMLOG, "squash kind");
+    if constexpr (S == PB_SQUASH_OBS_LOOK_FURTHER) {
+        const float a = fabsf(x);
+        const float r = __fdiv_rn(a, __fadd_rn(__fsqrt_rn(__fadd_rn(a, 1.0f)), 1.0f));
+        return __fadd_rn(copysignf(r, x), __fmul_rn(PB_SQUASH_OLF_EPS, x));
+    } else if constexpr (S == PB_SQUASH_SYMLOG) {
+        return copysignf(log1pf(fabsf(x)), x);
+    } else {
+        return x;
+    }
+}
+
+template <int S>
+__device__ __forceinline__ float unsquash(float x)
+{
+    static_assert(S == PB_SQUASH_NONE || S == PB_SQUASH_OBS_LOOK_FURTHER || S == PB_SQUASH_SYMLOG, "squash kind");
+    if constexpr (S == PB_SQUASH_OBS_LOOK_FURTHER) {
+        constexpr float e = PB_SQUASH_OLF_EPS;
+        const float a = fabsf(x);
+        const float s = __fsqrt_rn(__fadd_rn(1.0f, __fmul_rn(4.0f * e, __fadd_rn(a, 1.0f + e))));
+        const float tm1 = __fdiv_rn(__fmul_rn(2.0f, a), __fadd_rn(s, 1.0f + 2.0f * e));
+        return copysignf(__fmul_rn(tm1, __fadd_rn(tm1, 2.0f)), x);
+    } else if constexpr (S == PB_SQUASH_SYMLOG) {
+        return copysignf(expm1f(fabsf(x)), x);
+    } else {
+        return x;
+    }
+}
+
 }  // namespace pb

@@ -11,10 +11,11 @@ from . import model_factory
 
 
 def _acting_policy(cfg):
-    """agent_factory.py:20-38.  Value squashing is unused by every BASELINE config: no unsquish function."""
+    """agent_factory.py:20-38.  IDS gets the config's unsquish function; greedy and e-greedy get none (as upstream)."""
     if cfg.use_ids:
         return action_selectors.IDSActionSelector(cfg.ids_lambda, cfg.ids_use_random_samples, cfg.ids_epsilon,
-                                                  cfg.ids_rho_lower_bound, cfg.ids_beta, None)
+                                                  cfg.ids_rho_lower_bound, cfg.ids_beta,
+                                                  model_factory.squish_functions(cfg)[1])
     if cfg.use_e_greedy:
         return action_selectors.EGreedyActionSelector(cfg.e_greedy_initial_epsilon, cfg.e_greedy_final_epsilon,
                                                       cfg.e_greedy_decay_timesteps, cfg.seed)

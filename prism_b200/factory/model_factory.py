@@ -2,12 +2,13 @@
 
 The seam of prism/factory/model_factory.py:49-153: an embedding network chosen by ``embedding_model_type``, an IQN
 distribution head when ``use_iqn``, and a Q ensemble (K heads under IDS, one head under plain DQN), all reading the
-reference's Config field names.  Value squashing and risk policies are outside the hot-path scope (no BASELINE config
-uses them) and are refused rather than ignored.
+reference's Config field names.  ``loss_squish_fn_id`` selects the (squish, unsquish) pair of
+agents/squish_functions.py that both heads receive (model_factory.py passes it the same way).
 """
 import torch.nn as nn
 
 from ..agents.models import CompositeModel, FFNNModel, IQNModel, MinAtarModel, NatureAtariCnn, QEnsemble
+from ..agents.squish_functions import get_squish_functions
 
 _ACTIVATIONS = {"tanh": nn.Tanh, "gelu": nn.GELU, "sigmoid": nn.Sigmoid, "swish": nn.SiLU}     # anything else: ReLU
 
@@ -16,6 +17,11 @@ def _squish_id(cfg):
     sq = getattr(cfg, "loss_squish_fn_id", "none")
     # two reference configs carry a trailing comma and hold the 1-tuple ("none",) (SURVEY appendix Q9)
     return sq[0] if isinstance(sq, tuple) else sq
+
+
+def squish_functions(cfg):
+    """(squish, unsquish) for the config's loss_squish_fn_id; (None, None) for "none" and any unknown id."""
+    return get_squish_functions(_squish_id(cfg))
 
 
 def _embedding(cfg, state_shape, act):
@@ -44,14 +50,14 @@ def _q_ensemble(cfg, head_args, heads, layers, width, variation_coef):
 
 def create_model(env_state_shape, env_n_actions, config):
     cfg = config
-    if _squish_id(cfg) in ("obs_look_further", "symlog"):
-        raise NotImplementedError("value squashing is outside the hot-path scope (no BASELINE config uses it)")
+    squish, unsquish = squish_functions(cfg)
     act = _ACTIVATIONS.get(cfg.embedding_model_act_fn_id, nn.ReLU)
     embedding = _embedding(cfg, env_state_shape, act)
     # what every head on top of the embedding shares
     head_args = dict(n_input_features=cfg.embedding_model_final_dim, n_actions=env_n_actions, model_activation=act,
                      use_layer_norm=cfg.use_layer_norm, sparse_init_p=cfg.sparse_init_p,
-                     use_double_q_learning=cfg.use_double_q_learning, device=cfg.device)
+                     use_double_q_learning=cfg.use_double_q_learning, squish_function=squish,
+                     unsquish_function=unsquish, device=cfg.device)
 
     distribution = None
     if cfg.use_iqn:
