@@ -474,7 +474,8 @@ int pb_conv3x3_relu_bwd(int B, int H, int W, int C, int OC, const float *x, cons
 
 /* Dense layers of the Q heads / IQN MLP (nn.Linear inside nn.Sequential in the reference:
  * prism/agents/models/ffnn_model.py:61-76, q_ensemble.py:26-48, iqn_model.py:30-46), one launch
- * each, batched over K heads, fp32 FFMA, split-K across a thread-block cluster (DSMEM reduce).
+ * each, batched over K heads, 3xTF32 tensor-core products, split-K across a thread-block cluster
+ * (DSMEM reduce).
  *   fwd:        Y[k] (M x N) = act(X[k] (M x J) . W[k]^T (N x J) + b[k]);  act 0 none / 1 ReLU;
  *               x_head_stride = 0 shares one X between all heads
  *   bwd_input:  dX[k] (M x J) = (dY[k] . [Ymask[k] > 0]) . W[k];  Ymask NULL = no activation;

@@ -721,7 +721,7 @@ int pb_ens_q_loss_sq(int B, int A, int K, const float *q_cur, const float *q_nex
     if (B == 0) return PB_OK;
     if (!q_cur || !q_next_online || !q_next_target || !action || !ret || !gdn || !loss_out || !grad_q_cur)
         return PB_E_ARG;
-    PB_LAUNCH_PDL_CHAIN(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
+    PB_LAUNCH(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
               action, ret, gdn, nonterminal, loss_weight, row_weight, grad_scale, loss_out, grad_q_cur,
               (const float *)nullptr, 1.0f, (const float *)nullptr, (float *)nullptr, (float *)nullptr, (unsigned int *)nullptr);
     return PB_OK;
@@ -752,7 +752,7 @@ int pb_ens_q_loss_total_sq(int B, int A, int K, const float *q_cur, const float 
     if (!q_cur || !q_next_online || !q_next_target || !action || !ret || !gdn || !loss_out || !grad_q_cur || !total_out ||
         !ticket)
         return PB_E_ARG;
-    PB_LAUNCH_PDL_CHAIN(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
+    PB_LAUNCH(kernel, (unsigned)((B + 3) / 4), 128, 0, stream, B, A, K, q_cur, q_next_online, q_next_target,
               action, ret, gdn, nonterminal, loss_weight, row_weight, grad_scale, loss_out, grad_q_cur, dist, q_scale,
               q_offset, total_out, td_out, ticket);
     return PB_OK;
@@ -807,7 +807,7 @@ int pb_loss_combine(int B, const float *dist, const float *q, const float *w, fl
                     float *total_out, float *td_out, void *stream)
 {
     if (B <= 0 || (!dist && !q)) return PB_E_ARG;
-    PB_LAUNCH_PDL_CHAIN(loss_combine_kernel, 1, 1024, 0, stream, B, dist, q, w, q_scale, q_offset, total_out, td_out);
+    PB_LAUNCH(loss_combine_kernel, 1, 1024, 0, stream, B, dist, q, w, q_scale, q_offset, total_out, td_out);
     return PB_OK;
 }
 
@@ -830,7 +830,7 @@ int pb_pack_grads_parity(int n_tensors, const long long *table, float scale, flo
     if (per > 128) per = 128;
     if (per < PACK_BLOCKS_PER_TENSOR) per = PACK_BLOCKS_PER_TENSOR;
     dim3 grid((unsigned)per, (unsigned)n_tensors);
-    PB_LAUNCH_PDL_CHAIN(pack_grads_kernel, grid, ADAM_THREADS, 0, stream, table, scale, flat, epoch, stride, partial_scratch,
+    PB_LAUNCH(pack_grads_kernel, grid, ADAM_THREADS, 0, stream, table, scale, flat, epoch, stride, partial_scratch,
               step_count);
     if (n_partials_out_h) *n_partials_out_h = n_tensors * per;
     return PB_OK;
@@ -863,7 +863,7 @@ int pb_opt_clip_apply(int rule, long long n, float *param, const float *grad, fl
     if (nb < 1) nb = 1;
     const long long cap = (long long)pb_sm_count() * 4;
     if (nb > cap) nb = cap;
-    PB_LAUNCH_PDL_CHAIN(clip_kernel(rule), (unsigned)nb, ADAM_THREADS, 0, stream, n, param, grad, m, v, step_count,
+    PB_LAUNCH(clip_kernel(rule), (unsigned)nb, ADAM_THREADS, 0, stream, n, param, grad, m, v, step_count,
               lr, h1, h2, eps, max_grad_norm, partial_scratch, n_partials, norm_out);
     return PB_OK;
 }

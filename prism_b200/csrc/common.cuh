@@ -21,14 +21,10 @@ extern std::atomic<long long> g_pb_launches;
 // Same, as a PROGRAMMATIC DEPENDENT LAUNCH: the kernel may be scheduled while its predecessor on the stream (or the
 // graph branch it is captured on) is still running; it must call pb::pdl_wait() before touching anything the
 // predecessor wrote.  Chains of short dependent kernels (the priority store's sample -> mark -> lines -> rebuild) save
-// the launch latency at every boundary.  PB_NO_PDL=1 launches them the ordinary way.
-// Two groups: the priority-store kernels (PB_LAUNCH_PDL; on by default) and the kernels of the agent's update chain
-// (PB_LAUNCH_PDL_CHAIN; OFF by default: measured -- a dependent kernel that is resident early holds SM slots while it
-// waits, and in the step graph those slots belong to the GEMMs of the parallel branches: 86.8 vs 83.8 us per step).
-// PB_PDL=all | per | none selects; PB_NO_PDL=1 is "none".
-bool pb_pdl_enabled();
-bool pb_pdl_chain_enabled();
-#define PB_LAUNCH_PDL_IF(enabled, kernel, grid, block, smem, stream, ...)                   \
+// the launch latency at every boundary.  The kernels of the agent's update chain are launched the ordinary way
+// (PB_LAUNCH): a dependent kernel that is resident early holds SM slots while it waits, and in the step graph those
+// slots belong to the GEMMs of the parallel branches (measured: 86.8 vs 83.8 us per step with PDL on that chain).
+#define PB_LAUNCH_PDL(kernel, grid, block, smem, stream, ...)                               \
     do {                                                                                    \
         cudaLaunchConfig_t pb_cfg_ = {};                                                    \
         pb_cfg_.gridDim = dim3(grid); pb_cfg_.blockDim = dim3(block);                       \
@@ -36,15 +32,11 @@ bool pb_pdl_chain_enabled();
         cudaLaunchAttribute pb_at_[1];                                                      \
         pb_at_[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                  \
         pb_at_[0].val.programmaticStreamSerializationAllowed = 1;                           \
-        pb_cfg_.attrs = pb_at_; pb_cfg_.numAttrs = (enabled) ? 1 : 0;                       \
+        pb_cfg_.attrs = pb_at_; pb_cfg_.numAttrs = 1;                                       \
         cudaError_t pb_e_ = cudaLaunchKernelEx(&pb_cfg_, kernel, __VA_ARGS__);              \
         g_pb_launches.fetch_add(1, std::memory_order_relaxed);                              \
         if (pb_e_ != cudaSuccess) return (int)pb_e_;                                        \
     } while (0)
-#define PB_LAUNCH_PDL(kernel, grid, block, smem, stream, ...)                               \
-    PB_LAUNCH_PDL_IF(pb_pdl_enabled(), kernel, grid, block, smem, stream, __VA_ARGS__)
-#define PB_LAUNCH_PDL_CHAIN(kernel, grid, block, smem, stream, ...)                         \
-    PB_LAUNCH_PDL_IF(pb_pdl_chain_enabled(), kernel, grid, block, smem, stream, __VA_ARGS__)
 
 // argument check of the rule-parameterised optimizer entries: PB_E_ARG for an unknown rule or a NULL state array that
 // the rule reads (m: Adam, centered RMSprop; v: every rule but SGD)

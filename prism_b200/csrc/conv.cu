@@ -10,7 +10,6 @@
 // accumulates its share in registers, partial sums are combined by a second tiny launch in a fixed
 // order (deterministic).
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -365,7 +364,7 @@ int pb_conv3x3_relu_fwd(int B, int H, int W, int C, int OC, const float *x, cons
     const size_t smem = fwd_smem(d);
     const int items = d.OH * d.OW * (ocp / 8);
     const int threads = items >= 256 ? 256 : (items + 31) / 32 * 32;
-    PB_LAUNCH_PDL_CHAIN(conv3x3_relu_fwd_kernel, (unsigned)B, threads, smem, stream, d, x, w, bias, out);
+    PB_LAUNCH(conv3x3_relu_fwd_kernel, (unsigned)B, threads, smem, stream, d, x, w, bias, out);
     return PB_OK;
 }
 
@@ -380,36 +379,31 @@ int pb_conv3x3_relu_bwd(int B, int H, int W, int C, int OC, const float *x, cons
     if (!x || !out || !dout || !partial_scratch || !dw) return PB_E_ARG;
     const int groups = pb_conv3x3_relu_bwd_groups(B);
     const int ne = OC * C * 9 + OC;
-    {
-        // 16 output channels, output plane a multiple of 8: the tensor-core kernel (PB_CONV_MMA=0: the FMA kernel)
-        static int mma_ok = -1;
-        if (mma_ok < 0) { const char *e = getenv("PB_CONV_MMA"); mma_ok = (e && e[0] == '0') ? 0 : 1; }
-        const int plane = d.OH * d.OW, nt = (C * 9 + 1 + 7) / 8;
-        const size_t msmem = sizeof(float) * (size_t)(H * frame_pitch(W) * C + 16 * CM_GSTRIDE + plane + nt * 8);
-        if (mma_ok && OC == 16 && (plane % 8) == 0 && plane <= 64 && nt >= 5 && nt <= CM_MAX_NT && msmem <= 48 * 1024) {
-            const unsigned grid = (unsigned)groups;
-#define PB_CONV_MMA_CASE(NTV)                                                                                      \
-            case NTV: PB_LAUNCH_PDL_CHAIN(conv3x3_relu_bwd_mma_kernel<NTV>, grid, CM_WARPS * 32, msmem, stream, d, x, out, \
-                                          dout, partial_scratch, groups); break;
-            switch (nt) {
-                PB_CONV_MMA_CASE(5) PB_CONV_MMA_CASE(6) PB_CONV_MMA_CASE(7) PB_CONV_MMA_CASE(8) PB_CONV_MMA_CASE(9)
-                PB_CONV_MMA_CASE(10) PB_CONV_MMA_CASE(11) PB_CONV_MMA_CASE(12)
-                default: goto fma_path;
-            }
-#undef PB_CONV_MMA_CASE
-            PB_LAUNCH_PDL_CHAIN(conv_bwd_reduce_kernel, (unsigned)((ne + 7) / 8), 256, 0, stream, groups, OC * C * 9, OC,
-                                partial_scratch, dw, db);
-            return PB_OK;
+    // 16 output channels, output plane a multiple of 8: the tensor-core kernel.  NT = (9C + 8) / 8 n-tiles: C = 4..10
+    // gives 5, 6, 7, 8, 10, 11, 12 (no C gives 9)
+    const int plane = d.OH * d.OW, nt = (C * 9 + 1 + 7) / 8;
+    const size_t msmem = sizeof(float) * (size_t)(H * frame_pitch(W) * C + 16 * CM_GSTRIDE + plane + nt * 8);
+    if (OC == 16 && (plane % 8) == 0 && plane <= 64 && nt >= 5 && nt <= CM_MAX_NT && msmem <= 48 * 1024) {
+        const unsigned grid = (unsigned)groups;
+#define PB_CONV_TC_CASE(NTV)                                                                                       \
+        case NTV: PB_LAUNCH(conv3x3_relu_bwd_mma_kernel<NTV>, grid, CM_WARPS * 32, msmem, stream, d, x, out, dout, \
+                            partial_scratch, groups); break;
+        switch (nt) {
+            PB_CONV_TC_CASE(5) PB_CONV_TC_CASE(6) PB_CONV_TC_CASE(7) PB_CONV_TC_CASE(8)
+            PB_CONV_TC_CASE(10) PB_CONV_TC_CASE(11) PB_CONV_TC_CASE(12)
         }
+#undef PB_CONV_TC_CASE
+        PB_LAUNCH(conv_bwd_reduce_kernel, (unsigned)((ne + 7) / 8), 256, 0, stream, groups, OC * C * 9, OC,
+                  partial_scratch, dw, db);
+        return PB_OK;
     }
-fma_path:
     const size_t smem = fma_bwd_smem(d);
     // two gradient elements per thread for the MinAtar embedding (880 elements, 512 threads): several CTAs per SM, so
     // one CTA's staging loads overlap another's FMA loop and the 256 per-sample CTAs are resident in one wave
     const int ne_all = OC * C * 9 + OC;
     const int bthreads = ne_all > 256 ? 512 : 256;
-    PB_LAUNCH_PDL_CHAIN(conv3x3_relu_bwd_kernel, (unsigned)groups, bthreads, smem, stream, d, x, out, dout, partial_scratch);
-    PB_LAUNCH_PDL_CHAIN(conv_bwd_reduce_kernel, (unsigned)((ne + 7) / 8), 256, 0, stream, groups, OC * C * 9, OC,
+    PB_LAUNCH(conv3x3_relu_bwd_kernel, (unsigned)groups, bthreads, smem, stream, d, x, out, dout, partial_scratch);
+    PB_LAUNCH(conv_bwd_reduce_kernel, (unsigned)((ne + 7) / 8), 256, 0, stream, groups, OC * C * 9, OC,
               partial_scratch, dw, db);
     return PB_OK;
 }

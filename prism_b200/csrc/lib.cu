@@ -1,6 +1,5 @@
 // lib.cu -- library-level entry points of libprism_b200.so
 #include "common.cuh"
-#include <stdlib.h>
 
 std::atomic<long long> g_pb_launches{0};
 
@@ -16,22 +15,6 @@ int pb_sm_count()
     cached[dev].store(n, std::memory_order_relaxed);
     return n;
 }
-
-static int pdl_mode()                                  // 0 none, 1 priority store only (default), 2 all
-{
-    static const int mode = [] {
-        const char *no = getenv("PB_NO_PDL");
-        if (no && no[0] == '1') return 0;
-        const char *e = getenv("PB_PDL");
-        if (!e) return 1;
-        if (e[0] == 'a') return 2;
-        if (e[0] == 'n') return 0;
-        return 1;
-    }();
-    return mode;
-}
-bool pb_pdl_enabled() { return pdl_mode() >= 1; }
-bool pb_pdl_chain_enabled() { return pdl_mode() >= 2; }
 
 namespace {
 // device timeline mark: the GPU's nanosecond clock at the point of the stream (or graph branch) it was enqueued on

@@ -8,13 +8,12 @@
 //     forward   Y = act(X W^T + b)                       (bias + ReLU fused)
 //     backward  dX = (dY . relu') W,  dW = (dY . relu')^T X,  db = colsum(dY . relu')   (mask fused on load,
 //               bias gradient fused into the dW launch)
-// batched over the K ensemble heads, fp32 FFMA (the reference's math: parity 1e-4 needs fp32 products),
+// batched over the K ensemble heads, products as 3xTF32 on the tensor cores (fp32-grade: parity 1e-4 needs it),
 // and fills the chip on small problems with split-K over a THREAD-BLOCK CLUSTER: the S CTAs of a
 // cluster each reduce a slice of the inner dimension and combine their 64x64 partial tiles through
 // distributed shared memory in a fixed order -- deterministic, no atomics, no workspace, one launch.
 #include "common.cuh"
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 namespace cg = cooperative_groups;
 
@@ -22,9 +21,8 @@ namespace {
 
 using namespace pb;
 
-constexpr int TM = 64, TN = 64, TK = 32, PAD = 8;   // NS x (A,B) stages of 32 x 72 floats (18 KB each; a row stride of 72 words
+constexpr int TM = 64, TN = 64, TK = 32, PAD = 8;   // 2 x (A,B) stages of 32 x 72 floats (18 KB each; a row stride of 72 words
                                                     // makes the tensor-core fragment loads conflict-free); C tile aliases them
-constexpr int NS = 4;                               // stages: a split's whole K range (<= NS chunks) is fetched at once
 
 
 // phase marks of one launch for measurement runs (pb_gemm_trace; profiles/kernel_chain.py): slot 0 <- the EARLIEST
@@ -126,16 +124,10 @@ __device__ __forceinline__ void store_tile(float (*S)[TM + PAD], const float (&r
 }
 
 // C[i][j] = epilogue( sum_seg sum_k A(i,k) B(k,j) )   grid: (n tiles, m tiles * batch, splits); cluster (1,1,splits)
-// FLIGHT: a split's whole K range (3..NS chunks) is fetched before the first chunk is consumed (NS stages of shared
-// memory, 3 CTAs per SM: the step runs three such forward GEMMs -- online, bootstrap x 2 -- on parallel graph branches and
-// all 384 CTAs must stay resident); otherwise the classic two-stage pipeline (4 CTAs per SM: the two backward GEMMs of
-// a layer, 512 CTAs, run side by side).
-//
-// TC: the products run on the tensor cores as 3xTF32 (mma.sync m16n8k8; every operand is split in registers into a TF32
+// The products run on the tensor cores as 3xTF32 (mma.sync m16n8k8; every operand is split in registers into a TF32
 // hi part and its fp32 residual lo, and each k step issues lo.hi + hi.lo + hi.hi into fp32 accumulators -- error ~1e-6,
-// the same recipe as csrc/tc_gemm.cu): a third of the issue slots of the FFMA loop, which is what bounds the step's
-// three concurrent forward GEMMs (0.4 GFLOP on the FFMA pipe).  These tiles are far too small and too many for the
-// persistent tcgen05 kernel (one 128 x N tile per SM, 200 KB of shared memory: it serialised the step's graph branches).
+// the same recipe as csrc/tc_gemm.cu).  These tiles are far too small and too many for the persistent tcgen05 kernel
+// (one 128 x N tile per SM, 200 KB of shared memory: it serialised the step's graph branches).
 __device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2])
 {
     asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
@@ -181,34 +173,33 @@ __device__ __forceinline__ void splitk_reduce(cg::cluster_group &cluster, float 
     }
 }
 
-// Everything after the K loop, shared by the two kernels below: (TC) fragments -> C tile -> 4 x 4 thread tiles; bias /
+// Everything after the K loop, shared by the two kernels below: fragments -> C tile -> 4 x 4 thread tiles; bias /
 // activation / store when the tile is complete; otherwise the split-K meeting in distributed shared memory.
-template <bool ROWSUM, bool TC>
+template <bool ROWSUM>
 __device__ __forceinline__ void finish_tile(const GemmArgs &g, float (*Cs)[TN + PAD], float *Rs, float (&cf)[4][4], float rsum,
-                                            float (&acc)[4][4], float (&rs)[4], int batch, int i0, int j0, bool want_rowsum,
-                                            int tr_on)
+                                            int batch, int i0, int j0, bool want_rowsum, int tr_on)
 {
     const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
     const int lane = t & 31, gq = lane >> 2, tq = lane & 3;
     const int wm = ((t >> 5) & 3) * 16, wn = (t >> 7) * 32;
-    if (TC) {
-        // fragments -> the C tile (it aliases the stages: every warp is past its last read, see the barriers above) ->
-        // the 4 x 4 thread tiles the epilogue and the split-K reduction work with
+    // fragments -> the C tile (it aliases the stages: every warp is past its last read, see the barriers in the
+    // callers) -> the 4 x 4 thread tiles the epilogue and the split-K reduction work with
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-            *reinterpret_cast<float2 *>(&Cs[wm + gq][wn + nt * 8 + 2 * tq]) = make_float2(cf[nt][0], cf[nt][1]);
-            *reinterpret_cast<float2 *>(&Cs[wm + gq + 8][wn + nt * 8 + 2 * tq]) = make_float2(cf[nt][2], cf[nt][3]);
-        }
-        if (ROWSUM && t < TM) Rs[t] = rsum;
-        __syncthreads();
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            const float4 v = *reinterpret_cast<const float4 *>(&Cs[(ty << 2) + r][tx << 2]);
-            acc[r][0] = v.x; acc[r][1] = v.y; acc[r][2] = v.z; acc[r][3] = v.w;
-            if (ROWSUM) rs[r] = Rs[(ty << 2) + r];
-        }
-        __syncthreads();                                           // the split-K path rewrites the C tile below
+    for (int nt = 0; nt < 4; ++nt) {
+        *reinterpret_cast<float2 *>(&Cs[wm + gq][wn + nt * 8 + 2 * tq]) = make_float2(cf[nt][0], cf[nt][1]);
+        *reinterpret_cast<float2 *>(&Cs[wm + gq + 8][wn + nt * 8 + 2 * tq]) = make_float2(cf[nt][2], cf[nt][3]);
     }
+    if (ROWSUM && t < TM) Rs[t] = rsum;
+    __syncthreads();
+    float acc[4][4];
+    float rs[4] = {};
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+        const float4 v = *reinterpret_cast<const float4 *>(&Cs[(ty << 2) + r][tx << 2]);
+        acc[r][0] = v.x; acc[r][1] = v.y; acc[r][2] = v.z; acc[r][3] = v.w;
+        if (ROWSUM) rs[r] = Rs[(ty << 2) + r];
+    }
+    __syncthreads();                                               // the split-K path rewrites the C tile below
     float *C = g.C + batch * g.c_bs;
     const float *bias = g.bias ? g.bias + batch * g.bias_bs : nullptr;
     auto emit = [&](int i, int j, float v) {
@@ -263,19 +254,20 @@ __device__ __forceinline__ void finish_tile(const GemmArgs &g, float (*Cs)[TN + 
         }
     };
     const int rank = (int)cluster.block_rank();
-    switch (g.splits) {
+    switch (g.splits) {                                    // 2, 4 or 8 (pick_splits)
         case 2: splitk_reduce<2>(cluster, &Cs[0][0], Rs, rank, t, i0, j0, emit4, want_rowsum ? g.colsum + batch * g.colsum_bs : nullptr, g.M); break;
         case 4: splitk_reduce<4>(cluster, &Cs[0][0], Rs, rank, t, i0, j0, emit4, want_rowsum ? g.colsum + batch * g.colsum_bs : nullptr, g.M); break;
-        case 8: splitk_reduce<8>(cluster, &Cs[0][0], Rs, rank, t, i0, j0, emit4, want_rowsum ? g.colsum + batch * g.colsum_bs : nullptr, g.M); break;
-        default: splitk_reduce<16>(cluster, &Cs[0][0], Rs, rank, t, i0, j0, emit4, want_rowsum ? g.colsum + batch * g.colsum_bs : nullptr, g.M); break;
+        default: splitk_reduce<8>(cluster, &Cs[0][0], Rs, rank, t, i0, j0, emit4, want_rowsum ? g.colsum + batch * g.colsum_bs : nullptr, g.M); break;
     }
     gemm_mark(tr_on, 5);
     cluster.sync();                                        // nobody exits while its tile is still being read
     gemm_mark(tr_on, 6);
 }
 
-template <bool A_KMAJOR, bool B_KMAJOR, bool ROWSUM, bool FLIGHT, bool TC>
-__global__ void __launch_bounds__(256, FLIGHT ? 3 : 4) gemm_kernel(GemmArgs g)
+// Operand tiles staged through registers in a two-stage pipeline, 4 CTAs per SM: the kernel for operands the cp.async
+// kernel below cannot copy in 16-byte pieces.
+template <bool A_KMAJOR, bool B_KMAJOR, bool ROWSUM>
+__global__ void __launch_bounds__(256, 4) gemm_kernel(GemmArgs g)
 {
     pdl_wait();                                                   // programmatic dependent launch (PB_LAUNCH_PDL)
     pdl_trigger();
@@ -284,11 +276,10 @@ __global__ void __launch_bounds__(256, FLIGHT ? 3 : 4) gemm_kernel(GemmArgs g)
     extern __shared__ __align__(16) float tiles[];
     __shared__ float Rs[TM];
     float (*As)[TK][TM + PAD] = reinterpret_cast<float (*)[TK][TM + PAD]>(tiles);
-    constexpr int STAGES = FLIGHT ? NS : 2;
-    float (*Bs)[TK][TN + PAD] = reinterpret_cast<float (*)[TK][TN + PAD]>(tiles + STAGES * TK * (TM + PAD));
+    float (*Bs)[TK][TN + PAD] = reinterpret_cast<float (*)[TK][TN + PAD]>(tiles + 2 * TK * (TM + PAD));
     float (*Cs)[TN + PAD] = reinterpret_cast<float (*)[TN + PAD]>(tiles);      // reused once the K loop is over
 
-    const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
+    const int t = threadIdx.x;
     const int batch = blockIdx.y / g.m_tiles, mt = blockIdx.y % g.m_tiles;
     const int i0 = mt * TM, j0 = blockIdx.x * TN;
     const int split = blockIdx.z;
@@ -300,9 +291,6 @@ __global__ void __launch_bounds__(256, FLIGHT ? 3 : 4) gemm_kernel(GemmArgs g)
     const int total = g.n_seg * chunks_per_seg;
     const int per = (total + g.splits - 1) / g.splits;
     const int it0 = split * per, it1 = min(total, it0 + per);
-
-    float acc[4][4] = {};
-    float rs[4] = {};
     const bool want_rowsum = ROWSUM && g.colsum != nullptr && blockIdx.x == 0;
 
     auto fetch = [&](int it, float (&ra)[2][4], float (&rb)[2][4]) {
@@ -320,16 +308,15 @@ __global__ void __launch_bounds__(256, FLIGHT ? 3 : 4) gemm_kernel(GemmArgs g)
             store_tile<B_KMAJOR>(Bs[b], rb[h], t, h);
         }
     };
-    // tensor-core path: warp w owns rows wm .. wm+15, columns wn .. wn+31 of the tile (one m16 x four n8 fragments)
+    // warp w owns rows wm .. wm+15, columns wn .. wn+31 of the tile (one m16 x four n8 fragments)
     const int lane = t & 31, gq = lane >> 2, tq = lane & 3;
     const int wm = ((t >> 5) & 3) * 16, wn = (t >> 7) * 32;
     float cf[4][4] = {};
-    float rsum = 0.f;                                              // ROWSUM on the TC path: thread t < 64 sums row t
+    float rsum = 0.f;                                              // ROWSUM: thread t < 64 sums row t
     auto compute = [&](int b) {
-        if (TC) {
-            // a warp whose 16 rows lie past M has nothing to add (zero-filled rows): the padded static batch of the
-            // data-parallel step (272 rows: a fifth tile with one live warp row) stays cheap
-            if (i0 + wm < g.M) {
+        // a warp whose 16 rows lie past M has nothing to add (zero-filled rows): the padded static batch of the
+        // data-parallel step (272 rows: a fifth tile with one live warp row) stays cheap
+        if (i0 + wm < g.M) {
 #pragma unroll
             for (int k0 = 0; k0 < TK; k0 += 8) {
                 uint32_t ah[4], al[4];
@@ -347,64 +334,31 @@ __global__ void __launch_bounds__(256, FLIGHT ? 3 : 4) gemm_kernel(GemmArgs g)
                     mma_tf32(cf[nt], ah, bh);
                 }
             }
-            }
-            if (ROWSUM && t < TM) {
+        }
+        if (ROWSUM && t < TM) {
 #pragma unroll
-                for (int k = 0; k < TK; ++k) rsum += As[b][k][t];
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < TK; ++k) {
-                const float4 a = *reinterpret_cast<const float4 *>(&As[b][k][ty << 2]);
-                const float4 bb = *reinterpret_cast<const float4 *>(&Bs[b][k][tx << 2]);
-                const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {bb.x, bb.y, bb.z, bb.w};
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) acc[r][c] = fmaf(av[r], bv[c], acc[r][c]);
-                    if (ROWSUM) rs[r] += av[r];
-                }
-            }
+            for (int k = 0; k < TK; ++k) rsum += As[b][k][t];
         }
     };
-    if (FLIGHT) {
-        // the split's whole K range fits the stages: EVERY global load is requested before the first one is consumed
-        // (one memory latency per launch instead of one per chunk -- these layers are latency-, not FLOP-bound),
-        // then one barrier and an uninterrupted FFMA loop
-        float ra[STAGES][2][4], rb[STAGES][2][4];
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s)
-            if (it0 + s < it1) fetch(it0 + s, ra[s], rb[s]);
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s)
-            if (it0 + s < it1) stash(s, ra[s], rb[s]);
+    float ra[2][4], rb[2][4];
+    int buf = 0;
+    if (it0 < it1) {
+        fetch(it0, ra, rb);
+        stash(0, ra, rb);
+    }
+    __syncthreads();
+    gemm_mark(tr_on, 1);
+    for (int it = it0; it < it1; ++it) {
+        const bool more = it + 1 < it1;
+        if (more) fetch(it + 1, ra, rb);
+        compute(buf);
+        if (more) stash(buf ^ 1, ra, rb);
         __syncthreads();
-        gemm_mark(tr_on, 1);
-#pragma unroll
-        for (int s = 0; s < STAGES; ++s)
-            if (it0 + s < it1) compute(s);
-        __syncthreads();                                           // the C tile aliases the stages
-    } else {
-        float ra[2][4], rb[2][4];
-        int buf = 0;
-        if (it0 < it1) {
-            fetch(it0, ra, rb);
-            stash(0, ra, rb);
-        }
-        __syncthreads();
-        gemm_mark(tr_on, 1);
-        for (int it = it0; it < it1; ++it) {
-            const bool more = it + 1 < it1;
-            if (more) fetch(it + 1, ra, rb);
-            compute(buf);
-            if (more) stash(buf ^ 1, ra, rb);
-            __syncthreads();
-            buf ^= 1;
-        }
+        buf ^= 1;
     }
 
     gemm_mark(tr_on, 2);
-    finish_tile<ROWSUM, TC>(g, Cs, Rs, cf, rsum, acc, rs, batch, i0, j0, want_rowsum, tr_on);
+    finish_tile<ROWSUM>(g, Cs, Rs, cf, rsum, batch, i0, j0, want_rowsum, tr_on);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -495,8 +449,6 @@ __global__ void __launch_bounds__(256, STAGES == 2 ? 4 : 3) gemm_async_kernel(Ge
     const int lane = t & 31, gq = lane >> 2, tq = lane & 3;
     const int wm = ((t >> 5) & 3) * 16, wn = (t >> 7) * 32;
     float cf[4][4] = {};
-    float acc[4][4] = {};
-    float rs[4] = {};
     float rsum = 0.f;
     const bool want_rowsum = ROWSUM && g.colsum != nullptr && blockIdx.x == 0;
     const bool live = i0 + wm < g.M;                               // a warp whose 16 rows lie past M has nothing to add
@@ -549,26 +501,63 @@ __global__ void __launch_bounds__(256, STAGES == 2 ? 4 : 3) gemm_async_kernel(Ge
     cp_async_wait<0>();
     __syncthreads();                                               // the C tile aliases the stages
     gemm_mark(tr_on, 2);
-    finish_tile<ROWSUM, true>(g, Cs, Rs, cf, rsum, acc, rs, batch, i0, j0, want_rowsum, tr_on);
+    finish_tile<ROWSUM>(g, Cs, Rs, cf, rsum, batch, i0, j0, want_rowsum, tr_on);
 }
 
 int pick_splits(long long tiles, int total_chunks)
 {
-    static int forced = -1;                         // PB_GEMM_SPLITS=n pins the split factor (tuning experiments)
-    if (forced < 0) { const char *e = getenv("PB_GEMM_SPLITS"); forced = e ? atoi(e) : 0; }
-    if (forced == 1 || forced == 2 || forced == 4 || forced == 8 || forced == 16) return total_chunks >= forced ? forced : 1;
-    static int max_split = -1;                      // PB_GEMM_MAX_SPLIT=16 allows the non-portable 16-CTA cluster
-    if (max_split < 0) { const char *e = getenv("PB_GEMM_MAX_SPLIT"); max_split = e ? atoi(e) : 8; }
     const int sms = pb_sm_count();
     int s = 1;
-    while (s < max_split && tiles * (s * 2) <= 2LL * sms && total_chunks / (s * 2) >= 2) s *= 2;
+    while (s < 8 && tiles * (s * 2) <= 2LL * sms && total_chunks / (s * 2) >= 2) s *= 2;
     return s;
 }
 
-template <bool AK, bool BK, bool ROWSUM, bool FLIGHT, bool TC>
-int launch_gemm_v(GemmArgs g, int batch, int n_tiles, void *stream);
+// one launch of a GEMM kernel: grid (n tiles, m tiles * batch, splits), the splits of a tile forming one cluster
+int launch_cluster(void (*kernel)(GemmArgs), const GemmArgs &g, int batch, int n_tiles, size_t smem, void *stream)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)n_tiles, (unsigned)(g.m_tiles * batch), (unsigned)g.splits);
+    cfg.blockDim = dim3(256);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = (unsigned)g.splits;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, g);
+    g_pb_launches.fetch_add(1, std::memory_order_relaxed);
+    if (e != cudaSuccess) return (int)e;
+    e = cudaGetLastError();
+    return e == cudaSuccess ? PB_OK : (int)e;
+}
+
+template <bool AK, bool BK, bool ROWSUM>
+int launch_gemm_reg(GemmArgs g, int batch, int n_tiles, void *stream)
+{
+    constexpr int SMEM = 2 * 2 * TK * (TM + PAD) * 4;
+    static PbPerDeviceOnce smem_set;                // one flag per template instantiation
+    if (!smem_set.done()) {
+        cudaError_t e = cudaFuncSetAttribute(gemm_kernel<AK, BK, ROWSUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+        if (e != cudaSuccess) return (int)e;
+        smem_set.mark();
+    }
+    return launch_cluster(gemm_kernel<AK, BK, ROWSUM>, g, batch, n_tiles, SMEM, stream);
+}
+
 template <bool AK, bool BK, bool ROWSUM, int STAGES>
-int launch_gemm_async(GemmArgs g, int batch, int n_tiles, void *stream);
+int launch_gemm_async(GemmArgs g, int batch, int n_tiles, void *stream)
+{
+    static PbPerDeviceOnce smem_set;                // one flag per template instantiation
+    if (!smem_set.done()) {
+        cudaError_t e = cudaFuncSetAttribute(gemm_async_kernel<AK, BK, ROWSUM, STAGES>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, STAGES * 3 * TILE_WORDS * 4);
+        if (e != cudaSuccess) return (int)e;
+        smem_set.mark();
+    }
+    const size_t smem = (size_t)STAGES * (g.mask ? 3 : 2) * TILE_WORDS * 4;
+    return launch_cluster(gemm_async_kernel<AK, BK, ROWSUM, STAGES>, g, batch, n_tiles, smem, stream);
+}
 
 bool async_eligible(const GemmArgs &g, bool ak, bool bk)
 {
@@ -588,100 +577,12 @@ int launch_gemm(GemmArgs g, int batch, void *stream)
     const int total_chunks = g.n_seg * ((g.K + TK - 1) / TK);
     g.splits = pick_splits((long long)g.m_tiles * n_tiles * batch, total_chunks);
     const int per = (total_chunks + g.splits - 1) / g.splits;      // chunks per split
-    // PB_GEMM_FLIGHT=1 selects the in-flight variant for splits of 3-4 chunks.  Off by default: measured equal on one
-    // GPU (the forward GEMMs are issue-, not load-bound) and its 3 CTAs per SM cannot hold the three 160-CTA forward
-    // GEMMs of the data-parallel step (272 padded rows) at once, the two-stage variant's 4 per SM can.
-    static int flight_ok = -1;
-    if (flight_ok < 0) { const char *e = getenv("PB_GEMM_FLIGHT"); flight_ok = (e && e[0] == '1') ? 1 : 0; }
-    static int tc_ok = -1;                                         // PB_GEMM_MMA=0: FFMA products (fp32 exactly)
-    if (tc_ok < 0) { const char *e = getenv("PB_GEMM_MMA"); tc_ok = (e && e[0] == '0') ? 0 : 1; }
-    const bool flight = flight_ok && per >= 3 && per <= NS;
-    // 16-byte aligned operands (every layer of the learner step): the cp.async kernel.  PB_GEMM_ASYNC=0: never.
-    static int async_ok = -1;
-    if (async_ok < 0) { const char *e = getenv("PB_GEMM_ASYNC"); async_ok = (e && e[0] == '0') ? 0 : 1; }
-    if (tc_ok && async_ok && async_eligible(g, AK, BK)) {
+    // 16-byte aligned operands (every layer of the learner step): the cp.async kernel
+    if (async_eligible(g, AK, BK)) {
         if (per <= 2) return launch_gemm_async<AK, BK, ROWSUM, 2>(g, batch, n_tiles, stream);
         return launch_gemm_async<AK, BK, ROWSUM, 4>(g, batch, n_tiles, stream);
     }
-    if (tc_ok) {
-        if (flight) return launch_gemm_v<AK, BK, ROWSUM, true, true>(g, batch, n_tiles, stream);
-        return launch_gemm_v<AK, BK, ROWSUM, false, true>(g, batch, n_tiles, stream);
-    }
-    if (flight) return launch_gemm_v<AK, BK, ROWSUM, true, false>(g, batch, n_tiles, stream);
-    return launch_gemm_v<AK, BK, ROWSUM, false, false>(g, batch, n_tiles, stream);
-}
-
-template <bool AK, bool BK, bool ROWSUM, bool FLIGHT, bool TC>
-int launch_gemm_v(GemmArgs g, int batch, int n_tiles, void *stream)
-{
-    constexpr int SMEM = (FLIGHT ? NS : 2) * 2 * TK * (TM + PAD) * 4;
-    if (g.splits > 8) {
-        static PbPerDeviceOnce allowed;             // one flag per template instantiation
-        if (!allowed.done()) {
-            cudaError_t ea = cudaFuncSetAttribute(gemm_kernel<AK, BK, ROWSUM, FLIGHT, TC>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            if (ea != cudaSuccess) return (int)ea;
-            allowed.mark();
-        }
-    }
-    {
-        static PbPerDeviceOnce smem_set;            // one flag per template instantiation
-        if (!smem_set.done()) {
-            cudaError_t es = cudaFuncSetAttribute(gemm_kernel<AK, BK, ROWSUM, FLIGHT, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
-            if (es != cudaSuccess) return (int)es;
-            smem_set.mark();
-        }
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)n_tiles, (unsigned)(g.m_tiles * batch), (unsigned)g.splits);
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = SMEM;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = (unsigned)g.splits;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see PB_LAUNCH_PDL; the kernel waits itself
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pb_pdl_chain_enabled() ? 2 : 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_kernel<AK, BK, ROWSUM, FLIGHT, TC>, g);
-    g_pb_launches.fetch_add(1, std::memory_order_relaxed);
-    if (e != cudaSuccess) return (int)e;
-    e = cudaGetLastError();
-    return e == cudaSuccess ? PB_OK : (int)e;
-}
-
-template <bool AK, bool BK, bool ROWSUM, int STAGES>
-int launch_gemm_async(GemmArgs g, int batch, int n_tiles, void *stream)
-{
-    const int smem = STAGES * (g.mask ? 3 : 2) * TILE_WORDS * 4;
-    {
-        static PbPerDeviceOnce attrs_set;           // one flag per template instantiation
-        if (!attrs_set.done()) {
-            cudaError_t e = cudaFuncSetAttribute(gemm_async_kernel<AK, BK, ROWSUM, STAGES>,
-                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, STAGES * 3 * TILE_WORDS * 4);
-            if (e != cudaSuccess) return (int)e;
-            e = cudaFuncSetAttribute(gemm_async_kernel<AK, BK, ROWSUM, STAGES>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            if (e != cudaSuccess) return (int)e;
-            attrs_set.mark();
-        }
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)n_tiles, (unsigned)(g.m_tiles * batch), (unsigned)g.splits);
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = (size_t)smem;
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = (unsigned)g.splits;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;      // see PB_LAUNCH_PDL; the kernel waits itself
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pb_pdl_chain_enabled() ? 2 : 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_async_kernel<AK, BK, ROWSUM, STAGES>, g);
-    g_pb_launches.fetch_add(1, std::memory_order_relaxed);
-    if (e != cudaSuccess) return (int)e;
-    e = cudaGetLastError();
-    return e == cudaSuccess ? PB_OK : (int)e;
+    return launch_gemm_reg<AK, BK, ROWSUM>(g, batch, n_tiles, stream);
 }
 
 }  // namespace

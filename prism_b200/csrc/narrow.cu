@@ -289,7 +289,7 @@ int pb_narrow_linear_fwd(int K, long long M, int N, int J, const float *x, long 
             if (e != cudaSuccess) return (int)e;                                                                   \
             once.mark();                                                                                           \
         }                                                                                                          \
-        PB_LAUNCH_PDL_CHAIN(narrow_fwd_kernel<NP>, grid, 256, smem, stream, M, N, J / 4, x4, x_head_stride / 4, w4, bias, y); \
+        PB_LAUNCH(narrow_fwd_kernel<NP>, grid, 256, smem, stream, M, N, J / 4, x4, x_head_stride / 4, w4, bias, y); \
     } while (0)
     switch (narrow_np(N)) {
         case 4: PB_NARROW_FWD(4); break;
@@ -317,14 +317,14 @@ int pb_narrow_linear_bwd(int K, long long M, int N, int J, const float *x, long 
     float *dbp = partials ? partials + (size_t)K * nb * N * J : nullptr;
     const dim3 grid((unsigned)nb, (unsigned)K);
     switch (narrow_np(N)) {
-        case 4: PB_LAUNCH_PDL_CHAIN(narrow_bwd_kernel<4>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
-        case 8: PB_LAUNCH_PDL_CHAIN(narrow_bwd_kernel<8>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
-        case 16: PB_LAUNCH_PDL_CHAIN(narrow_bwd_kernel<16>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
-        default: PB_LAUNCH_PDL_CHAIN(narrow_bwd_kernel<32>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
+        case 4: PB_LAUNCH(narrow_bwd_kernel<4>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
+        case 8: PB_LAUNCH(narrow_bwd_kernel<8>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
+        case 16: PB_LAUNCH(narrow_bwd_kernel<16>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
+        default: PB_LAUNCH(narrow_bwd_kernel<32>, grid, J / 2, 0, stream, M, N, J, x, x_head_stride, w, dy, dx, dWp, dbp, rpc); break;
     }
     if (dW || db) {
         const long long n = (long long)N * J;
-        PB_LAUNCH_PDL_CHAIN(narrow_reduce_kernel, dim3((unsigned)((n + N + 31) / 32), (unsigned)K), 256, 0, stream, nb, n, N, dWp, dbp,
+        PB_LAUNCH(narrow_reduce_kernel, dim3((unsigned)((n + N + 31) / 32), (unsigned)K), 256, 0, stream, nb, n, N, dWp, dbp,
                   dW, db);
     }
     return PB_OK;
@@ -337,8 +337,8 @@ int pb_narrow_linear_bwd_reduce(int K, long long M, int N, int J, const float *p
     if (!dW && !db) return PB_OK;
     const int nb = pb_narrow_linear_bwd_blocks(M);
     const long long n = (long long)N * J;
-    PB_LAUNCH_PDL_CHAIN(narrow_reduce_kernel, dim3((unsigned)((n + N + 31) / 32), (unsigned)K), 256, 0, stream, nb, n, N, partials,
-                        partials + (size_t)K * nb * N * J, dW, db);
+    PB_LAUNCH(narrow_reduce_kernel, dim3((unsigned)((n + N + 31) / 32), (unsigned)K), 256, 0, stream, nb, n, N, partials,
+              partials + (size_t)K * nb * N * J, dW, db);
     return PB_OK;
 }
 

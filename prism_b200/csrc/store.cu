@@ -438,7 +438,7 @@ int pb_store_gather(const pb_store *st, long long n, const long long *idx, float
     if (!idx || !obs_out || !next_obs_out || !ret_out || !gamma_out || !nonterm_out || !action_out) return PB_E_ARG;
     dim3 grid((unsigned)n, (unsigned)(2 * v.fs));
     const int threads = v.row_bytes >= 4096 ? 256 : 128;
-    PB_LAUNCH_PDL_CHAIN(store_gather_kernel, grid, threads, 0, stream, v, n, idx, obs_out, next_obs_out, ret_out, gamma_out,
+    PB_LAUNCH(store_gather_kernel, grid, threads, 0, stream, v, n, idx, obs_out, next_obs_out, ret_out, gamma_out,
               nonterm_out, action_out);
     return PB_OK;
 }

@@ -676,15 +676,9 @@ int launch_bn(int a_mn, int b_mn, const CUtensorMap &ta, const CUtensorMap &tb, 
     return launch_cfg<BN, BK, 1, 0>(ta, tb, tc, g, grid, stream);
 }
 
-// K block per tile width.  PB_TC_BK=16|32 overrides (tuning runs).
+// K block per tile width
 int pick_bk(int bn, int K)
 {
-    static int forced = -1;
-    if (forced < 0) {
-        const char *e = getenv("PB_TC_BK");
-        forced = e ? atoi(e) : 0;
-    }
-    if (forced == 16 || forced == 32) return forced;
     return (bn == 256 && K >= 256) ? 16 : 32;    // 4 x 48 KB stages instead of 2 x 96 KB once the K loop is long
 }
 
@@ -795,10 +789,8 @@ int pb_tc_gemm(int batch, int kbatches, int M, int N, int K,
         g.tma_store = 1;
     }
 
-    if (bk == 16) {
-        if (best_bn == 256) rc = launch_bn<256, 16>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);
-        else if (best_bn == 128) rc = launch_bn<128, 16>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);
-        else rc = launch_bn<64, 16>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);
+    if (bk == 16) {                                                    // only at bn 256 (pick_bk)
+        rc = launch_bn<256, 16>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);
     } else {
         if (best_bn == 256) rc = launch_bn<256, 32>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);
         else if (best_bn == 128) rc = launch_bn<128, 32>(a_major, b_major, ta, tb, tc, g, (int)grid, stream);

@@ -3,7 +3,7 @@ float64 autograd of torch's conv2d, at every path its backward dispatches to:
 
 - the 3xTF32 tensor-core backward (``conv3x3_relu_bwd_mma_kernel<NT>``, NT = (9C + 8) / 8): every reachable NT,
 - the FMA backward (``conv3x3_relu_bwd_kernel``): too few taps, an output plane that is not a multiple of 8 or
-  exceeds 64, OC != 16, and PB_CONV_MMA=0 at the tensor-core shapes,
+  exceeds 64, OC != 16,
 - batches past 296, where one CTA accumulates more than one sample before the fixed-order reduction.
 
 Frames are real-valued: a binary frame splits exactly into its TF32 high part, so it cannot notice a missing
@@ -13,11 +13,7 @@ single-pass TF32 product sits near 1e-3 and a dropped low-part product near 1e-4
 Also here: pb_conv3x3_relu_supported against a Python mirror of the kernel's limits (no GPU needed), and
 MinAtarModel's cuDNN path for the frames the kernel refuses."""
 import ctypes as C
-import json
-import os
 import re
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -26,8 +22,6 @@ import torch.nn.functional as F
 from helpers import rel_err
 
 DEV = "cuda:0"
-HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 
 FWD_BAR = 2e-5
 GRAD_BAR = 2e-5             # also at B 4096 (14 samples per CTA): dW 6.9e-6, db 3.0e-6 measured on a B200 at 1000 W
@@ -57,8 +51,8 @@ def mirror_supported(H, W, C_, OC):
 
 
 def backward_path(H, W, C_, OC):
-    """The backward pb_conv3x3_relu_bwd launches (PB_CONV_MMA unset), as the tensor-core condition in that entry
-    (conv.cu) decides it: 'mma_nt<NT>' for the tensor-core kernel, 'fma_<reason>' for the FMA kernel."""
+    """The backward pb_conv3x3_relu_bwd launches, as the tensor-core condition in that entry (conv.cu) decides it:
+    'mma_nt<NT>' for the tensor-core kernel, 'fma_<reason>' for the FMA kernel."""
     plane, nt = (H - 2) * (W - 2), (9 * C_ + 1 + 7) // 8
     if OC != 16:
         return "fma_oc"
@@ -233,37 +227,6 @@ def test_conv_without_bias(case):
     _, dw, db = ops._ConvEmbed.backward(out.grad_fn, gy.to(DEV))
     torch.cuda.synchronize()
     assert db is None and dw.shape == (OC, C_, 3, 3)
-
-
-FMA_CHILD_CASES = [(256, 10, 10, c, 16, "randn") for c in (4, 6, 10)]
-
-
-def fma_child_main():
-    """Body of the PB_CONV_MMA=0 child: the FMA backward at the tensor-core shapes (the switch is read once per
-    process, so it cannot be flipped inside the parent)."""
-    assert os.environ.get("PB_CONV_MMA") == "0"
-    res = []
-    for case in FMA_CHILD_CASES:
-        x, w, b, gy = make_inputs(*case)
-        kernels = backward_kernels(lambda: run_kernel(x, w, b, gy))
-        res.append({"case": case_id(case), "kernels": sorted(kernels), "errs": check_against_fp64(x, w, b, gy)})
-    print("FMA_CHILD " + json.dumps(res))
-
-
-@pytest.mark.gpu
-def test_fma_backward_at_tensor_core_shapes():
-    env = dict(os.environ, PB_CONV_MMA="0")
-    code = "import sys; sys.path[:0] = [%r, %r]; import test_gpu_conv; test_gpu_conv.fma_child_main()" % (HERE, ROOT)
-    p = subprocess.run([sys.executable, "-c", code], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True,
-                       timeout=300, env=env)
-    assert p.returncode == 0, p.stdout[-3000:]
-    line, = [l for l in p.stdout.splitlines() if l.startswith("FMA_CHILD ")]
-    res = json.loads(line[len("FMA_CHILD "):])
-    assert len(res) == len(FMA_CHILD_CASES)
-    for r in res:
-        print("conv rel_err PB_CONV_MMA=0 %s: fwd %.2e dW %.2e db %.2e" % ((r["case"],) + tuple(r["errs"])))
-        assert r["kernels"] == ["fma"], r
-        assert r["errs"][0] < FWD_BAR and max(r["errs"][1:]) < GRAD_BAR, r
 
 
 @pytest.mark.gpu

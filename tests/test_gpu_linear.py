@@ -4,8 +4,7 @@ bwd_weight), against float64 math at every kernel, split factor and pipeline dep
 - ``gemm_async_kernel<AK, BK, ROWSUM, STAGES>`` (cp.async tiles, 16-byte aligned operands): STAGES 2 (a split of at
   most 2 chunks of 32 along the inner dimension), STAGES 4 with the whole split in flight, and STAGES 4 with the ring
   wrapping (more than 4 chunks per split),
-- ``gemm_kernel<AK, BK, ROWSUM, FLIGHT, TC>`` (register-staged tiles): unaligned shapes and pointers, and at aligned
-  shapes in child processes under PB_GEMM_ASYNC=0, PB_GEMM_MMA=0 (fp32 FFMA products) and PB_GEMM_FLIGHT=1,
+- ``gemm_kernel<AK, BK, ROWSUM>`` (register-staged tiles): unaligned shapes and pointers, at split factors 1, 2, 4 and 8,
 - split-K factors 1, 2, 4 and 8, including a split that gets no chunks (272 rows = the padded data-parallel batch),
 - the fused epilogue and operand work: bias, ReLU, the ReLU mask as a third operand, the bias gradient (ROWSUM),
   heads as a batch and heads as inner-dimension segments (``sum_heads``).
@@ -18,10 +17,7 @@ the CPU that single-pass TF32 and 3xTF32 without its lo.hi term both exceed it o
 Which kernel runs is mirrored in Python (``plan``, no GPU needed) and checked against the kernel names and grids the
 CUDA profiler records."""
 import json
-import os
 import re
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -30,8 +26,6 @@ import torch
 from helpers import rel_err
 
 DEV = "cuda:0"
-HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 
 BAR = 2e-5
 SMS_B200 = 148
@@ -43,13 +37,13 @@ SENTINEL = 1234.5
 # ------------------------------------------------------------------------------------------------------------------
 TM = TN = 64
 TK = 32
-NS = 4
+NS = 4                       # cp.async stages of a split with more than 2 chunks
 ENTRIES = ("fwd", "bwd_input", "bwd_weight")
 
 
-def pick_splits(tiles, chunks, sms, max_split=8):
+def pick_splits(tiles, chunks, sms):
     s = 1
-    while s < max_split and tiles * (s * 2) <= 2 * sms and chunks // (s * 2) >= 2:
+    while s < 8 and tiles * (s * 2) <= 2 * sms and chunks // (s * 2) >= 2:
         s *= 2
     return s
 
@@ -74,23 +68,16 @@ def gemm_args(entry, case, masked=False):
     return N, J, M, 1, K, async_eligible(x_ok and mask_ok, N, J, (M * N, xhs), False, False, N, J, M)
 
 
-def plan(entry, case, sms=SMS_B200, env=None, masked=False):
-    """What launch_gemm launches for `entry` on `case` with the PB_GEMM_* switches in `env`: kernel ('async2',
-    'async4', 'reg', 'reg_flight', 'ffma', 'ffma_flight'), split factor, chunks per split, grid and label."""
-    env = {} if env is None else env
+def plan(entry, case, sms=SMS_B200, masked=False):
+    """What launch_gemm launches for `entry` on `case`: kernel ('async2', 'async4', 'reg'), split factor, chunks per
+    split, grid and label."""
     gM, gN, gK, n_seg, batch, aligned = gemm_args(entry, case, masked)
     m_tiles, n_tiles = -(-gM // TM), -(-gN // TN)
     cps = -(-gK // TK)
     chunks = n_seg * cps
     splits = pick_splits(m_tiles * n_tiles * batch, chunks, sms)
     per = -(-chunks // splits)
-    tc = not env.get("PB_GEMM_MMA", "").startswith("0")
-    use_async = not env.get("PB_GEMM_ASYNC", "").startswith("0")
-    flight = env.get("PB_GEMM_FLIGHT", "").startswith("1") and 3 <= per <= NS
-    if tc and use_async and aligned:
-        kernel = "async2" if per <= 2 else "async4"
-    else:
-        kernel = ("reg" if tc else "ffma") + ("_flight" if flight else "")
+    kernel = ("async2" if per <= 2 else "async4") if aligned else "reg"
     ranges = [(s * per, min(chunks, s * per + per)) for s in range(splits)]
     return {"kernel": kernel, "splits": splits, "per": per, "chunks": chunks, "cps": cps, "n_seg": n_seg,
             "ranges": ranges, "grid": [n_tiles, m_tiles * batch, splits],
@@ -121,16 +108,12 @@ TABLE = [
 VARIANTS = {"bias-relu-mask-db": (True, 1, True, True), "plain": (False, 0, False, False),
             "bias-db": (True, 0, False, True), "relu-mask": (False, 1, True, False)}
 
-SWITCHES = {"async0": {"PB_GEMM_ASYNC": "0"}, "async0-flight": {"PB_GEMM_ASYNC": "0", "PB_GEMM_FLIGHT": "1"},
-            "mma0": {"PB_GEMM_MMA": "0"}, "mma0-flight": {"PB_GEMM_MMA": "0", "PB_GEMM_FLIGHT": "1"}}
-
-
 def case_id(case):
     K, M, N, J, shared, off = case
     return "K%d-M%d-N%d-J%d-%s%s" % (K, M, N, J, "shared" if shared else "perhead", "-" + off if off else "")
 
 
-def coverage(table, sms=SMS_B200, env=None):
+def coverage(table, sms=SMS_B200):
     """Required dispatch item -> id of the first table case that reaches it."""
     hit = {}
 
@@ -139,15 +122,15 @@ def coverage(table, sms=SMS_B200, env=None):
 
     for case in table:
         for entry in ENTRIES:
-            p = plan(entry, case, sms, env, masked=True)
+            p = plan(entry, case, sms, masked=True)
             k = p["kernel"]
             if k == "async2":
                 mark("%s: async STAGES 2" % entry, case)
             if k == "async4":
                 mark("%s: async STAGES 4, %s" % (entry, "ring wraps" if p["per"] > NS else "<= 4 chunks per split"), case)
             mark("%s: %d splits" % (entry, p["splits"]), case)
-            if k.startswith(("reg", "ffma")):
-                mark("%s kernel, %s" % (k, "splits = 1" if p["splits"] == 1 else "splits > 1"), case)
+            if k == "reg":
+                mark("reg kernel, %d splits" % p["splits"], case)
             if any(a >= b for a, b in p["ranges"]):
                 mark("a split with zero chunks", case)
             if entry == "bwd_input" and p["n_seg"] > 1 and any(
@@ -161,7 +144,8 @@ def coverage(table, sms=SMS_B200, env=None):
 REQUIRED = ([e + ": " + s for e in ENTRIES for s in ("async STAGES 2", "async STAGES 4, <= 4 chunks per split",
                                                       "async STAGES 4, ring wraps")]
             + [e + ": %d splits" % s for e in ENTRIES for s in (1, 2, 4, 8)]
-            + ["reg kernel, splits = 1", "reg kernel, splits > 1", "a split with zero chunks",
+            + ["reg kernel, %d splits" % s for s in (1, 2, 4, 8)]
+            + ["a split with zero chunks",
                "bwd_input sum_heads: segments cross a split boundary",
                "bwd_weight with db on async", "bwd_weight with db on register-staged"])
 
@@ -293,16 +277,13 @@ def launched_gemms(fn, trace_path):
         if not m:
             continue
         targs = [a.strip() for a in m.group(2).split(",")]
-        if m.group(1) == "gemm_async_kernel":
-            kernel = "async%s" % targs[3]
-        else:
-            kernel = ("reg" if targs[4] == "true" else "ffma") + ("_flight" if targs[3] == "true" else "")
+        kernel = "async%s" % targs[3] if m.group(1) == "gemm_async_kernel" else "reg"
         assert "grid" in e.get("args", {}), "the profiler trace records no grid for %s" % e["name"]
         got.append({"kernel": kernel, "rowsum": targs[2] == "true", "grid": list(e["args"]["grid"])})
     return got
 
 
-def witness_table(trace_path, env):
+def witness_table(trace_path):
     """Run every table case once (bias, ReLU, mask, db) under the profiler; returns (launched, expected)."""
     sms = torch.cuda.get_device_properties(0).multi_processor_count
     inputs = [make_inputs(case) for case in TABLE]
@@ -316,7 +297,7 @@ def witness_table(trace_path, env):
     want = []
     for case in TABLE:
         for entry in ENTRIES:
-            p = plan(entry, case, sms, env, masked=True)
+            p = plan(entry, case, sms, masked=True)
             want.append({"kernel": p["kernel"], "rowsum": entry == "bwd_weight", "grid": p["grid"]})
     return got, want
 
@@ -349,18 +330,6 @@ def test_mirror_table_covers_every_dispatch_path():
     assert x_off[0] == "reg" and x_off[1].startswith("async") and x_off[2] == "reg"
     mask_off = [plan(e, TABLE[15], masked=True)["kernel"] for e in ENTRIES]
     assert mask_off[0].startswith("async") and mask_off[1] == "reg" and mask_off[2] == "reg"
-
-
-def test_mirror_switches_reach_their_kernels():
-    """Each PB_GEMM_* child runs its kernel on aligned shapes; the in-flight variants need splits of 3-4 chunks."""
-    want = {"async0": "reg", "async0-flight": "reg_flight", "mma0": "ffma", "mma0-flight": "ffma_flight"}
-    for name, env in SWITCHES.items():
-        kernels = {plan(e, c, env=env, masked=True)["kernel"] for c in TABLE for e in ENTRIES}
-        assert not any(k.startswith("async") for k in kernels), name
-        assert want[name] in kernels, (name, kernels)
-        aligned = [c for c in TABLE if all(gemm_args(e, c, True)[5] for e in ENTRIES)]
-        assert {plan("fwd", c, env=env)["kernel"] for c in aligned} >= {want[name]}, name
-    assert {plan(e, c, env=SWITCHES["async0-flight"])["kernel"] for c in TABLE for e in ENTRIES} == {"reg", "reg_flight"}
 
 
 def _tf32(a):
@@ -410,54 +379,11 @@ def test_linear_entries_match_fp64(case, variant):
 
 
 @pytest.mark.gpu
-def test_profiler_sees_the_mirrored_kernels(tmp_path):
+def test_profiler_sees_the_mirrored_gemm_kernels(tmp_path):
     """Kernel, pipeline depth, ROWSUM and grid (gridDim.z = split factor) of every launch over the table equal the
     mirror's plan at this GPU's SM count."""
-    got, want = witness_table(tmp_path / "linear.pt.trace.json", {})
+    got, want = witness_table(tmp_path / "linear.pt.trace.json")
     assert len(got) == len(want)
     for i, (g, w) in enumerate(zip(got, want)):
         assert g == w, (case_id(TABLE[i // 3]), ENTRIES[i % 3], g, w)
 
-
-def switch_child_main():
-    """Body of a PB_GEMM_* child (the switches are read once per process): the kernels the profiler sees over the
-    table, and every case and variant against fp64."""
-    env = {k: v for k, v in os.environ.items() if k.startswith("PB_GEMM_")}
-    import tempfile
-    with tempfile.TemporaryDirectory() as d:
-        got, want = witness_table(os.path.join(d, "linear.pt.trace.json"), env)
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    errs = []
-    for case in TABLE:
-        for variant in VARIANTS:
-            e = check_case(case, variant)
-            errs.append({"case": case_id(case), "variant": variant,
-                         "errs": {"%s[%s]" % (k, plan(entry_of(k), case, sms, env, VARIANTS[variant][2])["kernel"]): v
-                                  for k, v in e.items()}})
-    print("LINEAR_CHILD " + json.dumps({"got": got, "want": want, "errs": errs}))
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("switch", list(SWITCHES))
-def test_switches_match_fp64_in_a_child(switch):
-    env = dict(os.environ, **SWITCHES[switch])
-    for k in ("PB_GEMM_ASYNC", "PB_GEMM_MMA", "PB_GEMM_FLIGHT", "PB_GEMM_SPLITS", "PB_GEMM_MAX_SPLIT"):
-        if k not in SWITCHES[switch]:
-            env.pop(k, None)
-    code = ("import sys; sys.path[:0] = [%r, %r]; import test_gpu_linear; test_gpu_linear.switch_child_main()"
-            % (HERE, ROOT))
-    p = subprocess.run([sys.executable, "-c", code], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True,
-                       timeout=500, env=env)
-    assert p.returncode == 0, p.stdout[-3000:]
-    line, = [l for l in p.stdout.splitlines() if l.startswith("LINEAR_CHILD ")]
-    res = json.loads(line[len("LINEAR_CHILD "):])
-    assert len(res["got"]) == len(res["want"]) == 3 * len(TABLE)
-    for i, (g, w) in enumerate(zip(res["got"], res["want"])):
-        assert g == w, (switch, case_id(TABLE[i // 3]), ENTRIES[i % 3], g, w)
-    worst = {}
-    for r in res["errs"]:
-        for k, v in r["errs"].items():
-            assert v < BAR, (switch, r)
-            worst[k] = max(worst.get(k, 0.0), v)
-    assert len(res["errs"]) == len(TABLE) * len(VARIANTS)
-    print("linear rel_err %s worst: %s" % (switch, ", ".join("%s %.2e" % kv for kv in sorted(worst.items()))))
